@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the CPU port of the reference's sampler, same metric and config
+    python bench.py ... --dump-outputs DIR    # also write the sampler state after the last timed step (one process)
 
 A "step" is one full sweep ([theta +] z with the count rebuild, [exchange], Phi draw) over the corpus.
 Default workload: BASELINE.json configs[3] -- the WHOLE PubMed-shaped corpus (8.2 M documents, ~738 M tokens,
@@ -72,6 +73,34 @@ def profile_record(workload):
     if os.path.exists(p):
         return json.load(open(p)).get(workload)
     return None
+
+
+DUMP_Z = 4 << 20           # topic indicators kept (float32: 16 MiB)
+DUMP_CELLS = 2 << 20       # cells of the n_wk rows (float64: 16 MiB) and of the same Phi^T rows (float32: 8 MiB)
+
+
+def dump_outputs(s, out_dir):
+    """What a caller of sample() receives after the last timed sweep, as DIR/<name>.npy: the topic indicators z,
+    the type-topic counts n_wk and Phi^T (the same rows of both, [rows][K]), the topic totals n_k and the model
+    log-likelihood.  Arrays larger than the caps above are a sample drawn from SEED, the same one for the same
+    corpus shape, so two builds run with the same arguments can be compared output for output.  theta is left out:
+    it is D x K (33.6 GB on the default workload), the library exports it only whole, and z is drawn from it."""
+    rng = np.random.default_rng(SEED)
+
+    def pick(n, cap):
+        return np.arange(n) if n <= cap else np.sort(rng.choice(n, cap, replace=False))
+
+    z = s.get_z_flat()
+    z = z[pick(len(z), DUMP_Z)]
+    rows = pick(s.numTypes, max(1, DUMP_CELLS // s.numTopics))
+    n_wk = s.getTypeTopicMatrix()[rows]
+    phiT = s.getPhi().T[rows]
+    out = {"z": z.astype(np.float32), "n_wk_rows": n_wk.astype(np.float64), "phiT_rows": phiT.astype(np.float32),
+           "n_k": s.getTopicTotals().astype(np.float64),
+           "log_likelihood": np.array([s.modelLogLikelihood()], np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_config(name, wl, scaling):
@@ -243,11 +272,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="N=1: skip the NIPS-/Enron-/Wikipedia-shaped side measurements")
     ap.add_argument("--cpu-sample-tokens", type=int, default=3_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the state of the last one as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours in one process")
     wl = dict(WORKLOADS[args.workload])
     if args.docs:
         wl["D"] = args.docs
@@ -279,7 +312,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def measure(name, wl, scaling, steps, warmup, with_e2e, with_clocks, with_props=True):
+    def measure(name, wl, scaling, steps, warmup, with_e2e, with_clocks, with_props=True, dump_dir=None):
         """One workload on this process group: device-resident sweeps, then the end-to-end loop."""
         if scaling == "strong":
             d0, d1 = wl["D"] * rank // world, wl["D"] * (rank + 1) // world      # this rank's documents of the fixed corpus
@@ -310,6 +343,7 @@ def main():
 
         # ---- device-resident: warm-up, then exactly K sweeps in one library call ---------------
         s.sample(warmup, chunk=0)
+        it0 = s.getCurrentIteration()
         clocks = ClockSampler()
         barrier()
         if rank == 0 and with_clocks:
@@ -319,7 +353,11 @@ def main():
         barrier()
         wall_ms = (time.perf_counter() - w0) * 1e3
         call_ms, zk_ms, zk_launches, launches = s.getLastCallStats()
+        if s.getCurrentIteration() - it0 != steps:
+            raise RuntimeError(f"{name}: the timed call ran {s.getCurrentIteration() - it0} sweeps, not {steps}")
         ck = clocks.stop(set(range(world))) if (rank == 0 and with_clocks) else None
+        if dump_dir:
+            dump_outputs(s, dump_dir)
         need_more = 1.0 if (rank == 0 and with_clocks and (ck.get("samples") or 0) < 3) else 0.0
         wall_ms = all_max(wall_ms)
         if all_max(need_more) > 0:
@@ -432,7 +470,8 @@ def main():
         return res, off, tokens
 
     config = make_config(args.workload, wl, scaling)
-    res, off, tokens = measure(args.workload, wl, scaling, args.steps, args.warmup, True, True)
+    res, off, tokens = measure(args.workload, wl, scaling, args.steps, args.warmup, True, True,
+                               dump_dir=args.dump_outputs)
 
     # ---- roofline of the dominant kernel (z-step; GGS: with the fused theta draw) ---------------------
     peak, peak_src = peaks()

@@ -610,12 +610,17 @@ template <int NT> static cudaError_t launch_theta_t(const ThetaArgs &a, int sm_c
 cudaError_t launch_theta(const ThetaArgs &a, int sm_count, cudaStream_t st)
 {
     if (a.n_docs <= 0) return cudaSuccess;
-    switch (a.dm.NT) {
-    case 1: return launch_theta_t<1>(a, sm_count, st);
-    case 2: return launch_theta_t<2>(a, sm_count, st);
-    case 4: return launch_theta_t<4>(a, sm_count, st);
-    case 8: if (a.dm.K <= 1024) return launch_theta_t<8>(a, sm_count, st);
-    default: break;
+    // theta_kernel<NT> writes rows in the register path's layout (Ks = 128 * NT, permuted columns); the sparse scheme
+    // keeps its rows in natural topic order with Ks = round_up(K, 32) and takes the general kernel at every K
+    const int NT = a.dm.NT, lg = NT == 1 ? 2 : NT == 2 ? 3 : NT == 4 ? 4 : 5;
+    if (a.dm.K <= 1024 && a.dm.Ks == NT * TILE && a.dm.lg == lg) {
+        switch (NT) {
+        case 1: return launch_theta_t<1>(a, sm_count, st);
+        case 2: return launch_theta_t<2>(a, sm_count, st);
+        case 4: return launch_theta_t<4>(a, sm_count, st);
+        case 8: return launch_theta_t<8>(a, sm_count, st);
+        default: break;
+        }
     }
     return launch_theta_big(a, sm_count, st);
 }

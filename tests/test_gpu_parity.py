@@ -126,7 +126,12 @@ def test_whole_sweeps_bit_exact_cats(oracle, cats, golden, scheme, osch):
     s.close()
 
 
-@pytest.mark.parametrize("scheme,osch,K", [("gpu_ggs", 0, 100), ("gpu_pcgs", 1, 400), ("gpu_ggs", 0, 1000)])
+# K boundaries of the register path: 1 and 2 topics, full tiles (128, 512: no padding), 513 (the first K with 8 tiles;
+# GGS switches to its 8-tile launch shape), 1024 (the largest K there: the clamp to K - 1 falls in a full lane)
+@pytest.mark.parametrize("scheme,osch,K", [("gpu_ggs", 0, 100), ("gpu_pcgs", 1, 400), ("gpu_ggs", 0, 1000),
+                                           ("gpu_ggs", 0, 1), ("gpu_ggs", 0, 2), ("gpu_ggs", 0, 128), ("gpu_ggs", 0, 512),
+                                           ("gpu_ggs", 0, 513), ("gpu_ggs", 0, 1024), ("gpu_pcgs", 1, 256),
+                                           ("gpu_pcgs", 1, 513), ("gpu_pcgs", 1, 1024)])
 def test_whole_sweeps_bit_exact_synthetic(oracle, scheme, osch, K):
     import ldagroupedgibbssampler_b200 as L
     V = 1200
@@ -236,9 +241,11 @@ def test_diagnostic_files(oracle, tmp_path):
 
 
 @pytest.mark.parametrize("scheme,osch,K", [("gpu_ggs", 0, 1025), ("gpu_pcgs", 1, 1500), ("gpu_ggs", 0, 2600),
-                                           ("gpu_pcgs", 1, 2049)])
+                                           ("gpu_pcgs", 1, 2049), ("gpu_ggs", 0, 2048), ("gpu_pcgs", 1, 2048),
+                                           ("gpu_ggs", 0, 27000), ("gpu_pcgs", 1, 18000)])
 def test_large_k_dense_path_bit_exact(oracle, scheme, osch, K):
-    """K > 1024: Phi^T row staged in shared memory, tile totals in groups of 8 tiles with a carry."""
+    """K > 1024: Phi^T row staged in shared memory, tile totals in groups of 8 tiles with a carry.  K = 2048 is whole
+    groups of 8 tiles (no partial group for the carry); 27 000 (GGS) and 18 000 (PCGS) are the largest K that fit."""
     off, tokens = make_corpus(40, 300, 30, seed=K, empty_every=9)
     V, alpha, beta, seed = 300, 50.0 / K, 0.01, 5
     s = _sampler(scheme, off, tokens, V, K, alpha, beta, seed)
@@ -256,9 +263,11 @@ def test_large_k_dense_path_bit_exact(oracle, scheme, osch, K):
     s.close()
 
 
-@pytest.mark.parametrize("K,V,D,mean_len", [(20, 303, 23, 300), (300, 800, 120, 60), (1500, 400, 60, 40), (4000, 300, 50, 150)])
+@pytest.mark.parametrize("K,V,D,mean_len", [(20, 303, 23, 300), (300, 800, 120, 60), (1500, 400, 60, 40), (4000, 300, 50, 150),
+                                            (1, 120, 30, 40), (5, 200, 40, 50)])
 def test_sparse_pcgs_bit_exact(oracle, K, V, D, mean_len):
-    """gpu_spalias: alias tables and sparse z-step bit-exact against the oracle, whole sweeps included."""
+    """gpu_spalias: alias tables and sparse z-step bit-exact against the oracle, whole sweeps included; the diagnostic
+    theta (rows in natural topic order here, Ks = round_up(K, 32)) and the log-posterior too."""
     off, tokens = make_corpus(D, V, mean_len, seed=K + 2, empty_every=11)
     alpha, beta, seed = 50.0 / K, 0.01, 17
     s = _sampler("gpu_spalias", off, tokens, V, K, alpha, beta, seed)
@@ -277,6 +286,12 @@ def test_sparse_pcgs_bit_exact(oracle, K, V, D, mean_len):
     assert np.array_equal(s.getPhi().T.astype(np.float32), st["phiT"])
     want_ll = oracle.log_likelihood(off, st["z"], K, V, st["n_wk"], st["n_k"], np.full(K, alpha), beta)
     assert abs(s.modelLogLikelihood() - want_ll) <= 1e-9 * abs(want_ll)
+    lp = s.computeLogPosterior()
+    th = oracle.theta_contract(off, st["z"], K, np.full(K, alpha), seed, s.getCurrentIteration())
+    assert np.array_equal(s.getTheta().astype(np.float32), th)
+    want_lp = oracle.log_posterior(off, tokens, st["z"], K, V, th.astype(np.float64), st["phiT"].astype(np.float64),
+                                   np.full(K, alpha), beta)
+    assert abs(lp - want_lp) <= 1e-9 * abs(want_lp)
     s.close()
 
 

@@ -245,6 +245,9 @@ def test_polya_urn_scheme_bit_exact(oracle, K, V, D, mean_len):
     got0 = s.getPhi().T.astype(np.float32)
     assert np.array_equal(got0, phi0)                    # initial Phi: the urn too (UPL:450 -> loopOverTopics override)
     assert (got0 == 0).mean() > 0.5                      # sparse rows
+    if K <= 300:
+        # word types of the corpus whose Phi column is all zero: their tokens take the tot = 0 fallback (DESIGN.md 4.6)
+        assert not got0[np.unique(tokens)].any(axis=1).all()
     s.sample(3)
     st = oracle.sweeps("contract", oracle.POLYAURN, off, tokens, z0, V, K, np.full(K, alpha), beta, seed, 1, 3, phi0)
     assert np.array_equal(s.get_z_flat(), st["z"])

@@ -220,39 +220,39 @@ __device__ __forceinline__ void theta_draw_doc(int *cg, unsigned short *plist, c
 
     // ---- phase 1; the cells it leaves open are appended to the pending list as they are found
     //      (ballot + popc, all lanes) and the list is drained whenever another 32 might not fit
-    //      TH_W cells of the lane go through the attempt side by side (gamma_attempt_squeeze_w: independent
-    //      dependency chains in one basic block; the values are those of the scalar attempt)
-#ifndef TH_W_DEF
-#define TH_W_DEF 2
-#endif
-    constexpr int TH_W = TH_W_DEF;
+    //      two cells of the lane (q, q + 1: adjacent columns) go through the attempt side by side in packed FP32
+    //      (gamma_attempt_squeeze2; the values are those of the scalar attempt)
 #pragma unroll 1
-    for (int q = 0; q < NT * 4; q += TH_W) {
-        int p[TH_W];
-        bool valid[TH_W], zero[TH_W], done[TH_W];
-        float dd[TH_W], cc[TH_W], ii[TH_W], gv[TH_W];
-        uint4 rnd[TH_W];
+    for (int q = 0; q < NT * 4; q += 2) {
+        int p[2];
+        bool valid[2], zero[2], done[2];
+        uint4 rnd[2];
 #pragma unroll
-        for (int w = 0; w < TH_W; ++w) {
+        for (int w = 0; w < 2; ++w) {
             p[w] = ((q + w) >> 2) * TILE + lane * 4 + ((q + w) & 3);
             const int k = lane * (4 * NT) + q + w;
             valid[w] = k < K;
             zero[w] = valid[w] && cg[p[w]] == 0;
-            dd[w] = tb.d0[p[w]]; cc[w] = tb.c0[p[w]]; ii[w] = tb.i0[p[w]];
             const unsigned long long cell = cell0 + (unsigned long long)k;
             rnd[w] = philox4x32_10((uint32_t)cell, (uint32_t)(cell >> 32), sweep, STREAM_THETA << 24, rk);
         }
-        gamma_attempt_squeeze_w<TH_W>(dd, cc, ii, rnd, done, gv);
+        // q is even, so the two cells are one aligned float2 of each table
+        const float2 dd = *reinterpret_cast<const float2 *>(tb.d0 + p[0]);
+        const float2 cc = *reinterpret_cast<const float2 *>(tb.c0 + p[0]);
+        const float2 ii = *reinterpret_cast<const float2 *>(tb.i0 + p[0]);
+        float2 gv;
+        gamma_attempt_squeeze2(dd, cc, ii, rnd[0], rnd[1], done[0], done[1], gv);
+        const float g2[2] = {gv.x, gv.y};
 #pragma unroll
-        for (int w = 0; w < TH_W; ++w) {
+        for (int w = 0; w < 2; ++w) {
             const bool settled = zero[w] && done[w];
-            if (settled) cg[p[w]] = __float_as_int(gv[w]);
+            if (settled) cg[p[w]] = __float_as_int(g2[w]);
             const bool open = valid[w] && !settled;
             const unsigned open_mask = __ballot_sync(FULL, open);
             if (open) plist[npend + __popc(open_mask & lt_mask)] = (unsigned short)p[w];
             npend += __popc(open_mask);
         }
-        if (npend > TH_PLIST - 32 * TH_W) drain();
+        if (npend > TH_PLIST - 64) drain();
     }
     // ---- phase 2
     if (npend > 0) drain();

@@ -2,9 +2,11 @@
 // the C ABI declared in include/ldagpu.h.
 //
 // One sweep (reference order: topics/UncollapsedParallelLDA.java:645-693):
-//   [GGS] theta_kernel        theta_d ~ Dir(n_d + alpha)                 (GGS:60-72)
-//   z_kernel                  z_i | theta/n_d, Phi                        (GGS:79-130, UPL:1491-1543)
-//   counts_kernel             n_wk, n_k from z                            (UPL:1107-1221 net effect)
+//   [GGS] theta_kernel        theta_d ~ Dir(n_d + alpha) for the documents the z-step does not draw itself:
+//                             those longer than one work item (all of them above the register path's K)  (GGS:60-72)
+//   z_kernel                  [GGS] theta_d of a whole-document work item, then z_i | theta/n_d, Phi; n_wk
+//                             accumulated from the new z                  (GGS:79-130, UPL:1491-1543, 1107-1221)
+//   topic_totals_kernel       n_k from n_wk
 //   [G>1] reduce-scatter n_wk by vocabulary slice, all-reduce n_k         (stand-in for the shared
 //                                                                         AtomicInteger[K][V], UPL:102)
 //   phi_draw / segments       Gamma(beta + n_wk) for the rank's slice     (GGS:182-192, PCGS:91-101)
@@ -29,6 +31,7 @@
 #include <numeric>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/ldagpu.h"
@@ -174,8 +177,10 @@ struct ldagpu_handle_s {
 
     // single-process multi-GPU (ldagpu_create_multi): this handle only coordinates; the shards hold the state
     std::vector<ldagpu_handle> shards;
-    std::vector<int64_t> shard_doc0, shard_tok0;   // [G+1] first document / token of every shard
+    std::vector<int64_t> shard_doc0, shard_tok0;   // [parts + 1] first document / token of every part, in this handle's order
     bool multi() const { return !shards.empty(); }
+    // what an entry point fans out to, in shard order: the shards of a group, else the handle itself (a group of one)
+    std::vector<ldagpu_handle> parts() { return multi() ? shards : std::vector<ldagpu_handle>{this}; }
 
     std::atomic<int> abort_flag{0};
     std::string err;
@@ -210,8 +215,22 @@ struct ldagpu_handle_s {
 #define NEED(h)                                  \
     if (!(h)) return 1;                          \
     CK(h, cudaSetDevice((h)->device))
+// one part's share of a call: on the part's device; a failure is reported on the caller's handle
+#define MC(P, c, call)                               \
+    do {                                             \
+        cudaSetDevice((c)->device);                  \
+        if (call) return part_fail(P, c);            \
+    } while (0)
 
 namespace {
+
+using Parts = std::vector<ldagpu_handle>;
+
+int part_fail(ldagpu_handle P, ldagpu_handle c)
+{
+    P->err = c->err;
+    return 1;
+}
 
 int ensure_events(ldagpu_handle h, size_t n)
 {
@@ -327,37 +346,51 @@ int rendezvous(ldagpu_handle h, int *abort_any = nullptr)
 // for another shard's signal must only be enqueued after the kernel that gives the signal: a launch can block the
 // host until the device drains (first use of a kernel under lazy module loading, a larger local-memory pool), and a
 // device that waits for work the blocked host has not enqueued yet would never drain.  So the exchange and the Phi
-// draw are cut into stages -- every waiter in a later stage than the signals it waits for -- and the multi-GPU layer
-// runs stage by stage over all shards.  stage < 0 runs all stages (one shard per caller: nothing to order).
-enum { EXCH_STAGES = 3, PHI_STAGES = 3 };
+// draw are cut into stages -- every waiter in a later stage than the signals it waits for -- and every operation that
+// exchanges runs stage by stage over all parts (run_stages); a single GPU is a group of one.  The NCCL collectives and a
+// single GPU have nothing to order: they do all their work in the first stage of the exchange and of the Phi draw.
+enum Stage {
+    ST_LOCAL,       // [theta +] z-step, topic totals, push n_k parts + "my partial counts are complete"
+    ST_REDUCE,      // reduce the rank's vocabulary rows over all ranks' counts (waits for ST_LOCAL of all), signal the barrier
+    ST_BARRIER,     // wait for the barrier: nobody touches its partial counts again before every rank has read them
+    ST_DRAW,        // Phi draw (+ the peers' counts when fused) + segment sums stored to every rank + "segments in place"
+    ST_NORMALISE,   // normalise (waits for every rank's segments) + rows stored to every rank + "rows in place"
+    ST_LAND,        // wait until every rank's rows have landed here; [sparse scheme] rebuild the alias tables
+    N_STAGES
+};
+
+// every stage on every part before the next stage on any part
+template <typename F> int run_stages(ldagpu_handle h, const Parts &parts, F &&stage_of_part)
+{
+    for (int st = 0; st < N_STAGES; ++st)
+        for (size_t g = 0; g < parts.size(); ++g) MC(h, parts[g], stage_of_part(g, (Stage)st));
+    return 0;
+}
 
 // defer_reduce (peer-memory mode): only announce the partial counts; the Phi draw that follows sums them.
-//   stage 0  push n_k parts + "my partial counts are complete"
-//   stage 1  reduce the rank's vocabulary rows over all ranks' counts (waits for stage 0 of all), signal the barrier
-//   stage 2  wait for the barrier: nobody touches its partial counts again before every rank has read them
-int step_counts_exchange(ldagpu_handle h, bool defer_reduce, int stage = -1)
+int step_counts_exchange(ldagpu_handle h, bool defer_reduce, Stage stage)
 {
     if (h->world == 1) return 0;
     if (h->p2p) {
-        if (stage < 0 || stage == 0) {
+        if (stage == ST_LOCAL) {
             h->counts_epoch = ++h->ep[P2P_FLAG_COUNTS];
             CK(h, launch_p2p_push_topic_totals(h->pt, h->n_k.p, h->dm.Ks, h->counts_epoch, h->stream));
             h->last_launches += 1;
         }
         if (defer_reduce) return 0;
-        if (stage < 0 || stage == 1) {
+        if (stage == ST_REDUCE) {
             CK(h, launch_p2p_reduce_counts(h->pt, h->dm, h->n_k.p, h->row0, h->row1, h->counts_epoch, h->sm_count, h->stream));
             h->bar_epoch = ++h->ep[P2P_FLAG_BAR];
             CK(h, launch_p2p_signal(h->pt, P2P_FLAG_BAR, h->bar_epoch, h->stream));
             h->last_launches += 2;
         }
-        if (stage < 0 || stage == 2) {
+        if (stage == ST_BARRIER) {
             CK(h, launch_p2p_wait(h->pt, P2P_FLAG_BAR, h->bar_epoch, h->stream));
             h->last_launches += 1;
         }
         return 0;
     }
-    if (stage > 0) return 0;
+    if (stage != ST_LOCAL) return 0;
     const size_t slice = (size_t)(h->dm.Vp / h->world) * h->dm.Ks;
     NK(h, g_nccl.ReduceScatter(h->n_wk.p, h->n_wk.p + (size_t)h->rank * slice, slice, ncclInt32, ncclSum, h->comm, h->stream));
     NK(h, g_nccl.AllReduce(h->n_k.p, h->n_k.p, (size_t)h->dm.Ks, ncclInt32, ncclSum, h->comm, h->stream));
@@ -376,15 +409,11 @@ int phi_mean_buffer(ldagpu_handle h, bool accumulate_mean, double **mean)
     return 0;
 }
 
-// peer-memory mode:
-//   stage 0  draw (summing the peers' partial counts when fused_reduce: waits for their "counts complete"), segment
-//            sums stored to every rank + "segments of rank r are in place"
-//   stage 1  normalise (waits for every rank's segments) + store the rows to every rank + "rows of rank r are in place"
-//   stage 2  wait until every rank's rows have landed here; [sparse scheme] rebuild the alias tables
-int step_phi_p2p(ldagpu_handle h, bool accumulate_mean, cudaEvent_t *ev, bool fused_reduce, int stage)
+// peer-memory mode: the fused draw (fused_reduce) sums the peers' partial counts, waiting for their "counts complete"
+int step_phi_p2p(ldagpu_handle h, bool accumulate_mean, cudaEvent_t *ev, bool fused_reduce, Stage stage)
 {
     const uint32_t lo = (uint32_t)h->seed, hi = (uint32_t)(h->seed >> 32);
-    if (stage < 0 || stage == 0) {
+    if (stage == ST_DRAW) {
         CK(h, launch_phi_draw_p2p(h->pt, fused_reduce, h->counts_epoch, h->dm, h->n_wk.p, h->n_k.p, h->beta, h->phiT.p,
                                   h->partial.p, h->row0, h->row1, lo, hi, (uint32_t)h->iteration, h->poisson_L, h->stream));
         h->seg_epoch = ++h->ep[P2P_FLAG_SEG];
@@ -392,7 +421,7 @@ int step_phi_p2p(ldagpu_handle h, bool accumulate_mean, cudaEvent_t *ev, bool fu
         h->last_launches += 2;
         if (ev) { CK(h, cudaEventRecord(ev[0], h->stream)); CK(h, cudaEventRecord(ev[1], h->stream)); }
     }
-    if (stage < 0 || stage == 1) {
+    if (stage == ST_NORMALISE) {
         double *mean = nullptr;
         if (phi_mean_buffer(h, accumulate_mean, &mean)) return 1;
         h->phi_epoch = ++h->ep[P2P_FLAG_PHI];
@@ -401,7 +430,7 @@ int step_phi_p2p(ldagpu_handle h, bool accumulate_mean, cudaEvent_t *ev, bool fu
         h->last_launches += 1;
         if (ev) CK(h, cudaEventRecord(ev[2], h->stream));
     }
-    if (stage < 0 || stage == 2) {
+    if (stage == ST_LAND) {
         CK(h, launch_p2p_wait(h->pt, P2P_FLAG_PHI, h->phi_epoch, h->stream));
         h->last_launches += 1;
         if (step_alias(h)) return 1;
@@ -411,10 +440,10 @@ int step_phi_p2p(ldagpu_handle h, bool accumulate_mean, cudaEvent_t *ev, bool fu
 }
 
 // ev != nullptr: record events after draw+segments, segment all-gather, normalise, Phi all-gather
-int step_phi(ldagpu_handle h, bool accumulate_mean, cudaEvent_t *ev, bool fused_reduce = false, int stage = -1)
+int step_phi(ldagpu_handle h, bool accumulate_mean, cudaEvent_t *ev, bool fused_reduce, Stage stage)
 {
     if (h->p2p) return step_phi_p2p(h, accumulate_mean, ev, fused_reduce, stage);
-    if (stage > 0) return 0;
+    if (stage != ST_DRAW) return 0;
     const uint32_t lo = (uint32_t)h->seed, hi = (uint32_t)(h->seed >> 32);
     CK(h, launch_phi_draw(h->dm, h->n_wk.p, h->beta, h->phiT.p, h->partial.p, h->row0, h->row1, lo, hi,
                           (uint32_t)h->iteration, h->poisson_L, h->stream));
@@ -463,8 +492,32 @@ int sync_check(ldagpu_handle h)
     return 0;
 }
 
+int sync_all(ldagpu_handle h, const Parts &parts)
+{
+    for (ldagpu_handle c : parts) MC(h, c, sync_check(c));
+    return 0;
+}
+
+int ensure_z16(ldagpu_handle h)
+{
+    if (!h->z16.p) CK(h, h->z16.alloc((size_t)std::max<int64_t>(h->dm.N, 1) + 8));
+    return 0;
+}
+
+// z[o, o + cnt) to z_out[o, ...) on `stream`, or narrowed on the device to z16_out[o, ...) when that is given
+int copy_z_out(ldagpu_handle h, int32_t *z_out, uint16_t *z16_out, int64_t o, int64_t cnt, cudaStream_t stream)
+{
+    if (z16_out) {
+        CK(h, launch_pack16(h->z.p + o, h->z16.p + o, cnt, h->sm_count, stream));
+        CK(h, cudaMemcpyAsync(z16_out + o, h->z16.p + o, sizeof(uint16_t) * (size_t)cnt, cudaMemcpyDeviceToHost, stream));
+    } else {
+        CK(h, cudaMemcpyAsync(z_out + o, h->z.p + o, sizeof(int32_t) * (size_t)cnt, cudaMemcpyDeviceToHost, stream));
+    }
+    return 0;
+}
+
 // ---- a call of n sweeps in three pieces, so that one caller thread can drive several shards (ldagpu_create_multi):
-// sweeps_prepare, then sweep_enqueue once per sweep (asynchronous), then sweeps_finish (synchronise, timers).
+// sweeps_prepare, then sweep_enqueue once per sweep and stage (asynchronous), then sweeps_finish (synchronise, timers).
 // z_out / z16_out != nullptr: the topic indicators of the last sweep are copied to the host on the copy stream as
 // soon as its z-step has finished, under the count exchange and the Phi draw (the Java shim copies z back into
 // the documents' LabelSequences after every sample() call, INTEGRATION.md section 2)
@@ -479,21 +532,18 @@ int sweeps_prepare(ldagpu_handle h, SweepCall &c)
 {
     h->last_zk_ms = 0; h->last_call_ms = 0; h->last_zk_launches = 0; h->last_launches = 0;
     c.ran = 0; c.z_copied = false;
+    if (c.z16_out && ensure_z16(h)) return 1;
     if (c.n <= 0) return 0;
     return ensure_events(h, (size_t)c.n * EV_PER_SWEEP);
 }
 
-// stage < 0: the whole sweep; otherwise one of SWEEP_STAGES stages (see "Stages" above):
-//   0  [theta] z + counts, topic totals, announce the counts     1, 2  stand-alone count reduce + barrier (z-only sweeps)
-//   3, 4, 5  the three stages of the Phi draw
-enum { SWEEP_STAGES = 1 + (EXCH_STAGES - 1) + PHI_STAGES };
-
-int sweep_enqueue(ldagpu_handle h, SweepCall &c, int stage = -1)
+// one stage of the next sweep (see "Stages" above); ST_REDUCE and ST_BARRIER only run in z-only sweeps, where no fused
+// Phi draw sums the counts
+int sweep_enqueue(ldagpu_handle h, SweepCall &c, Stage stage)
 {
     const int32_t s = c.ran;
-    const bool all = stage < 0;
     cudaEvent_t *ev = h->events.data() + (size_t)s * EV_PER_SWEEP;
-    if (all || stage == 0) {
+    if (stage == ST_LOCAL) {
         h->iteration += 1;
         CK(h, cudaEventRecord(ev[0], h->stream));
         // the count rebuild is fused into the z kernel: zero n_wk first (Phi, not n_wk, feeds the z-step)
@@ -512,14 +562,8 @@ int sweep_enqueue(ldagpu_handle h, SweepCall &c, int stage = -1)
                 if (step_z(h, true, fuse_theta, (int)p)) return 1;
                 CK(h, cudaEventRecord(h->copy_events[1 + p], h->stream));
                 CK(h, cudaStreamWaitEvent(h->copy_stream, h->copy_events[1 + p], 0));
-                const int64_t o = zp.tok0, cnt = zp.tok1 - zp.tok0;
-                if (c.z16_out) {
-                    CK(h, launch_pack16(h->z.p + o, h->z16.p + o, cnt, h->sm_count, h->copy_stream));
-                    CK(h, cudaMemcpyAsync(c.z16_out + o, h->z16.p + o, sizeof(uint16_t) * (size_t)cnt, cudaMemcpyDeviceToHost, h->copy_stream));
-                    h->last_launches += 1;
-                } else {
-                    CK(h, cudaMemcpyAsync(c.z_out + o, h->z.p + o, sizeof(int32_t) * (size_t)cnt, cudaMemcpyDeviceToHost, h->copy_stream));
-                }
+                if (copy_z_out(h, c.z_out, c.z16_out, zp.tok0, zp.tok1 - zp.tok0, h->copy_stream)) return 1;
+                h->last_launches += c.z16_out ? 1 : 0;
             }
             c.z_copied = true;
         } else if (step_z(h, true, fuse_theta)) return 1;
@@ -527,44 +571,33 @@ int sweep_enqueue(ldagpu_handle h, SweepCall &c, int stage = -1)
         if (!stream_out && (c.z_out || c.z16_out) && s == c.n - 1 && h->dm.N) {
             CK(h, cudaEventRecord(h->copy_events[0], h->stream));
             CK(h, cudaStreamWaitEvent(h->copy_stream, h->copy_events[0], 0));
-            if (c.z16_out) {   // narrow on the device (copy stream, under the Phi draw), half the PCIe bytes
-                CK(h, launch_pack16(h->z.p, h->z16.p, h->dm.N, h->sm_count, h->copy_stream));
-                CK(h, cudaMemcpyAsync(c.z16_out, h->z16.p, sizeof(uint16_t) * (size_t)h->dm.N, cudaMemcpyDeviceToHost, h->copy_stream));
-                h->last_launches += 1;
-            } else {
-                CK(h, cudaMemcpyAsync(c.z_out, h->z.p, sizeof(int32_t) * (size_t)h->dm.N, cudaMemcpyDeviceToHost, h->copy_stream));
-            }
+            // 16-bit transport: narrowed on the device (copy stream, under the Phi draw), half the PCIe bytes
+            if (copy_z_out(h, c.z_out, c.z16_out, 0, h->dm.N, h->copy_stream)) return 1;
+            h->last_launches += c.z16_out ? 1 : 0;
             c.z_copied = true;
         }
         CK(h, launch_topic_totals(h->dm, h->n_wk.p, h->n_k.p, h->stream));
         h->last_launches += 1;
         CK(h, cudaEventRecord(ev[3], h->stream));
-        if (step_counts_exchange(h, c.with_phi, all ? -1 : 0)) return 1;
     }
-    if (!all && (stage == 1 || stage == 2) && step_counts_exchange(h, c.with_phi, stage)) return 1;
-    if (all || stage == 2) CK(h, cudaEventRecord(ev[4], h->stream));
+    if (step_counts_exchange(h, c.with_phi, stage)) return 1;
+    if (stage == ST_BARRIER) CK(h, cudaEventRecord(ev[4], h->stream));
     if (c.with_phi) {
         const bool acc = mean_this_iteration(h);
-        if (all) { if (step_phi(h, acc, ev + 5, true)) return 1; }
-        else if (stage >= 3 && step_phi(h, acc, ev + 5, true, stage - 3)) return 1;
-        if ((all || stage == SWEEP_STAGES - 1) && acc) h->n_sampled_phi += 1;   // GGS:168-170
-    } else if (all || stage == SWEEP_STAGES - 1) {
+        if (step_phi(h, acc, ev + 5, true, stage)) return 1;
+        if (stage == ST_LAND && acc) h->n_sampled_phi += 1;   // GGS:168-170
+    } else if (stage == ST_LAND) {
         for (int i = 5; i < EV_PER_SWEEP; ++i) CK(h, cudaEventRecord(ev[i], h->stream));
     }
-    if (all || stage == SWEEP_STAGES - 1) c.ran += 1;
+    if (stage == ST_LAND) c.ran += 1;
     return 0;
 }
 
 int sweeps_finish(ldagpu_handle h, SweepCall &c)
 {
     const int32_t ran = c.ran;
-    if (!c.z_copied && h->dm.N) {   // aborted before the last sweep: plain copy of the current z
-        if (c.z_out) CK(h, cudaMemcpyAsync(c.z_out, h->z.p, sizeof(int32_t) * (size_t)h->dm.N, cudaMemcpyDeviceToHost, h->stream));
-        if (c.z16_out) {
-            CK(h, launch_pack16(h->z.p, h->z16.p, h->dm.N, h->sm_count, h->stream));
-            CK(h, cudaMemcpyAsync(c.z16_out, h->z16.p, sizeof(uint16_t) * (size_t)h->dm.N, cudaMemcpyDeviceToHost, h->stream));
-        }
-    }
+    // aborted before the last sweep: plain copy of the current z
+    if (!c.z_copied && h->dm.N && (c.z_out || c.z16_out) && copy_z_out(h, c.z_out, c.z16_out, 0, h->dm.N, h->stream)) return 1;
     if (sync_check(h)) return 1;
     if (c.z_copied) CK(h, cudaStreamSynchronize(h->copy_stream));
     for (int32_t s = 0; s < ran; ++s) {
@@ -591,24 +624,57 @@ int sweeps_finish(ldagpu_handle h, SweepCall &c)
     return 0;
 }
 
-int run_sweeps(ldagpu_handle h, int32_t n, bool with_phi, int32_t *done, int32_t *z_out = nullptr, uint16_t *z16_out = nullptr)
+// n sweeps on every part: sweep s is enqueued on every part before sweep s + 1 on any (a shard's kernels wait, on the
+// device, for the other shards' kernels of the same sweep).  z_out / z16_out are in corpus order.
+int run_sweeps(ldagpu_handle h, int32_t n, bool with_phi, int32_t *done, int32_t *z_out, uint16_t *z16_out)
 {
     if (done) *done = 0;
-    SweepCall c;
-    c.n = n; c.with_phi = with_phi; c.z_out = z_out; c.z16_out = z16_out;
-    if (sweeps_prepare(h, c)) return 1;
-    if (n <= 0) return 0;
-    // sharded (one process per GPU): every rank must run the same number of sweeps, or the others would wait for
-    // this one in the exchange -- the ranks agree on the abort flag here, once per call, and a call is short
-    // (the host side caps the sweeps per call); a single GPU looks at its flag before every sweep (UPL:645)
-    int stop = 0;
-    if (rendezvous(h, &stop)) return 1;
-    for (int32_t s = 0; s < n && !stop; ++s) {
-        if (h->world == 1 && h->abort_flag.load(std::memory_order_relaxed)) break;
-        if (sweep_enqueue(h, c)) return 1;
+    const Parts parts = h->parts();
+    std::vector<SweepCall> calls(parts.size());
+    for (size_t g = 0; g < parts.size(); ++g) {
+        SweepCall &c = calls[g];
+        c.n = n; c.with_phi = with_phi;
+        c.z_out = z_out ? z_out + h->shard_tok0[g] : nullptr;
+        c.z16_out = z16_out ? z16_out + h->shard_tok0[g] : nullptr;
+        MC(h, parts[g], sweeps_prepare(parts[g], c));
     }
-    if (sweeps_finish(h, c)) return 1;
-    if (done) *done = c.ran;
+    if (n > 0) {
+        // one process per GPU: every rank must run the same number of sweeps, or the others would wait for this one in
+        // the exchange -- the ranks agree on the abort flag in the rendezvous, once per call, and a call is short (the
+        // host side caps the sweeps per call); otherwise the flag is looked at before every sweep and stops all shards
+        // at the same one (UPL:645)
+        int stop = 0;
+        for (ldagpu_handle c : parts) {
+            int s = 0;
+            MC(h, c, rendezvous(c, &s));
+            stop |= s;
+        }
+        // fault injection for the tests of the bounded waits: LDAGPU_FAULT_STALL_SHARD=g leaves the Phi stages of shard g
+        // of a group out, as if its process had died -- the other shards must report a timeout instead of hanging
+        static const int stall_env = getenv("LDAGPU_FAULT_STALL_SHARD") ? atoi(getenv("LDAGPU_FAULT_STALL_SHARD")) : -1;
+        const int stall = h->multi() ? stall_env : -1;
+        for (int32_t s = 0; s < n && !stop; ++s) {
+            if (!h->comm && parts[0]->abort_flag.load(std::memory_order_relaxed)) break;
+            if (run_stages(h, parts, [&](size_t g, Stage st) {
+                    if ((int)g != stall || st < ST_DRAW) return sweep_enqueue(parts[g], calls[g], st);
+                    if (st == ST_LAND) calls[g].ran += 1;
+                    return 0;
+                }))
+                return 1;
+        }
+        for (size_t g = 0; g < parts.size(); ++g) MC(h, parts[g], sweeps_finish(parts[g], calls[g]));
+    }
+    // the call's statistics: the slowest part sets the time, launches add up
+    double call_ms = 0, zk_ms = 0;
+    int64_t zk_launches = 0, launches = 0;
+    for (ldagpu_handle c : parts) {
+        call_ms = std::max(call_ms, c->last_call_ms);
+        zk_ms = std::max(zk_ms, c->last_zk_ms);
+        zk_launches = std::max(zk_launches, c->last_zk_launches);
+        launches += c->last_launches;
+    }
+    h->last_call_ms = call_ms; h->last_zk_ms = zk_ms; h->last_zk_launches = zk_launches; h->last_launches = launches;
+    if (done) *done = calls[0].ran;
     return 0;
 }
 
@@ -695,17 +761,44 @@ void close_peer_exchange(ldagpu_handle h)
     h->p2p = false;
 }
 
-int setup_peer_exchange(ldagpu_handle h)
+// rank `rank` of `world` owns the vocabulary rows [row0, row1) and the Phi segments [seg0, seg1)
+void set_rank(ldagpu_handle h, int rank, int world)
 {
-    const char *mode = getenv("LDAGPU_EXCHANGE");
-    const bool want = !(mode && std::strcmp(mode, "nccl") == 0);
-    const int G = h->world;
+    h->rank = rank;
+    h->world = world;
+    const int32_t rows = h->dm.Vp / world;
+    h->row0 = rank * rows;
+    h->row1 = h->row0 + rows;
+    h->seg0 = rank * (PHI_SEGMENTS / world);
+    h->seg1 = h->seg0 + PHI_SEGMENTS / world;
+}
+
+// what the peer-memory exchange needs besides the peers' pointers: the zeroed n_k parts and flag buffers and the
+// PeerTable's own fields
+int init_peer_table(ldagpu_handle h)
+{
     CK(h, h->nk_parts.alloc((size_t)P2P_MAX * h->dm.Ks));
     CK(h, h->p2p_flags.alloc((size_t)P2P_FLAG_KINDS * P2P_MAX));
     CK(h, h->p2p_local.alloc((size_t)P2P_FLAG_KINDS + 4));
     CK(h, cudaMemset(h->nk_parts.p, 0, sizeof(int32_t) * h->nk_parts.n));
     CK(h, cudaMemset(h->p2p_flags.p, 0, sizeof(uint32_t) * h->p2p_flags.n));
     CK(h, cudaMemset(h->p2p_local.p, 0, sizeof(uint32_t) * h->p2p_local.n));
+    PeerTable &pt = h->pt;
+    pt = PeerTable{};
+    pt.rank = h->rank; pt.world = h->world;
+    pt.done_ctr = h->p2p_local.p;
+    pt.error = reinterpret_cast<int *>(h->p2p_local.p + P2P_FLAG_KINDS);
+    const char *to = getenv("LDAGPU_P2P_TIMEOUT_MS");
+    pt.timeout_ns = (unsigned long long)(to ? std::max(1L, atol(to)) : 60000L) * 1000000ull;
+    return 0;
+}
+
+int setup_peer_exchange(ldagpu_handle h)
+{
+    const char *mode = getenv("LDAGPU_EXCHANGE");
+    const bool want = !(mode && std::strcmp(mode, "nccl") == 0);
+    const int G = h->world;
+    if (init_peer_table(h)) return 1;
 
     int ok = want && G <= P2P_MAX ? 1 : 0;
     if (!want) h->p2p_note = "LDAGPU_EXCHANGE=nccl";
@@ -729,12 +822,6 @@ int setup_peer_exchange(ldagpu_handle h)
     blobs.release();
 
     PeerTable &pt = h->pt;
-    pt = PeerTable{};
-    pt.rank = h->rank; pt.world = G;
-    pt.done_ctr = h->p2p_local.p;
-    pt.error = reinterpret_cast<int *>(h->p2p_local.p + P2P_FLAG_KINDS);
-    const char *to = getenv("LDAGPU_P2P_TIMEOUT_MS");
-    pt.timeout_ns = (unsigned long long)(to ? std::max(1L, atol(to)) : 60000L) * 1000000ull;
     if (ok) {
         for (int r = 0; r < G && ok; ++r) {
             if (r == h->rank) {
@@ -789,28 +876,82 @@ double lgamma_stirling_host(double z)
     return r;
 }
 
+// alpha (validated by the caller) into the handle: the host copy and its sum (sequential, as MSL:139-143), the float and
+// double device copies and the lgS(alpha_k) table
+int upload_alpha(ldagpu_handle h, const double *alpha)
+{
+    const int K = h->dm.K;
+    h->alpha.assign(alpha, alpha + K);
+    h->alpha_sum = 0.0;
+    for (int k = 0; k < K; ++k) h->alpha_sum += alpha[k];
+    std::vector<float> af((size_t)h->dm.Ks, 0.0f);
+    std::vector<double> ad((size_t)h->dm.Ks, 0.0);
+    for (int k = 0; k < K; ++k) { af[(size_t)k] = (float)alpha[k]; ad[(size_t)k] = alpha[k]; }
+    CK(h, cudaMemcpyAsync(h->alpha_f.p, af.data(), sizeof(float) * af.size(), cudaMemcpyHostToDevice, h->stream));
+    CK(h, cudaMemcpyAsync(h->alpha_d.p, ad.data(), sizeof(double) * ad.size(), cudaMemcpyHostToDevice, h->stream));
+    CK(h, launch_lgs_table(K, h->alpha_d.p, h->lgs_alpha.p, h->stream));
+    return 0;
+}
+
+// An accessor that converts between the device layout and the host's [K][V] / [D][K] layout: the conversion kernel
+// (`launch`, given the scratch buffer) writes or reads `cells` values in host layout in a scratch buffer, which is
+// copied to `out` after it or from `in` before it.
+template <typename T, typename F>
+int via_scratch(ldagpu_handle h, DevBuf<T> &scratch, size_t cells, std::common_type_t<T> *out, const std::common_type_t<T> *in,
+                F &&launch)
+{
+    CK(h, scratch.alloc(cells));
+    if (in) CK(h, cudaMemcpyAsync(scratch.p, in, sizeof(T) * cells, cudaMemcpyHostToDevice, h->stream));
+    if (launch(scratch.p)) return 1;
+    if (out) CK(h, cudaMemcpyAsync(out, scratch.p, sizeof(T) * cells, cudaMemcpyDeviceToHost, h->stream));
+    int rc = sync_check(h);
+    scratch.release();
+    return rc;
+}
+
+// Every rank, and every shard of a group, holds the global values of its own vocabulary rows only (n_wk after the
+// exchange, the Phi-mean sums): collect all rows on parts[0], which exports them.  Ranks all-gather them with NCCL,
+// the shards of a group copy theirs to shard 0 over peer access.
+template <typename T>
+int gather_rows(ldagpu_handle h, const Parts &parts, DevBuf<T> ldagpu_handle_s::*buf, ncclDataType_t type)
+{
+    if (h->world > 1 && h->comm) {
+        const size_t slice = (size_t)(h->dm.Vp / h->world) * h->dm.Ks;
+        T *p = (h->*buf).p;
+        NK(h, g_nccl.AllGather(p + (size_t)h->rank * slice, p, slice, type, h->comm, h->stream));
+        return 0;
+    }
+    ldagpu_handle c0 = parts[0];
+    for (size_t g = 1; g < parts.size(); ++g) {
+        ldagpu_handle c = parts[g];
+        if (!(c->*buf).p || !(c0->*buf).p) continue;
+        const size_t o = (size_t)c->row0 * c->dm.Ks, cnt = (size_t)(c->row1 - c->row0) * c->dm.Ks;
+        cudaSetDevice(c->device);
+        CK(h, cudaMemcpyPeerAsync((c0->*buf).p + o, c0->device, (c->*buf).p + o, c->device, sizeof(T) * cnt, c->stream));
+        CK(h, cudaStreamSynchronize(c->stream));
+    }
+    return 0;
+}
+
+// counts from the resident z on every part, exchanged; redraw_phi: then Phi from them (UPL:450, 1842)
+int refresh_counts_and_phi(ldagpu_handle h, bool redraw_phi)
+{
+    const Parts parts = h->parts();
+    if (run_stages(h, parts, [&](size_t g, Stage st) {
+            ldagpu_handle c = parts[g];
+            if (st == ST_LOCAL && (rendezvous(c) || step_counts_local(c))) return 1;
+            return step_counts_exchange(c, redraw_phi, st) || (redraw_phi && step_phi(c, false, nullptr, true, st)) ? 1 : 0;
+        }))
+        return 1;
+    return sync_all(h, parts);
+}
+
 }  // namespace
 
 // =============================================================================================
 // C ABI
 // =============================================================================================
 extern "C" {
-
-// single-process multi-GPU layer (end of this file)
-static int multi_destroy(ldagpu_handle P);
-static int multi_init_z(ldagpu_handle P, int32_t seed);
-static int multi_set_z(ldagpu_handle P, const void *z, bool is16, int32_t redraw_phi);
-static int multi_get_z(ldagpu_handle P, void *z, bool is16);
-static int multi_run_sweeps(ldagpu_handle P, int32_t n, bool with_phi, int32_t *done, int32_t *z_out, uint16_t *z16_out);
-static int multi_step(ldagpu_handle P, int what);
-static int multi_get_type_topic_counts(ldagpu_handle P, int32_t *out);
-static int multi_get_doc_topic_counts(ldagpu_handle P, int32_t *out);
-static int multi_set_phi(ldagpu_handle P, const double *phi);
-static int multi_get_phi_mean(ldagpu_handle P, double *phi_mean, int32_t *n_sampled);
-static int multi_theta(ldagpu_handle P, double *theta_out, const double *theta_in);
-static int multi_log_likelihood(ldagpu_handle P, double *ll);
-static int multi_log_posterior(ldagpu_handle P, double *lp);
-enum { MSTEP_THETA = 0, MSTEP_Z = 1, MSTEP_COUNTS = 2, MSTEP_PHI = 3 };
 
 const char *ldagpu_version(void) { return "libldagpu 0.4 (sm_100a; GGS with fused theta, PCGS, sparse PCGS; peer-memory exchange; single-process multi-GPU)"; }
 
@@ -852,9 +993,6 @@ int ldagpu_create(int32_t K, int32_t V, int64_t D, const int64_t *doc_offsets, c
     h->scheme = scheme;
     h->beta = beta;
     h->seed = seed;
-    h->alpha.assign(alpha, alpha + K);
-    h->alpha_sum = 0.0;
-    for (int k = 0; k < K; ++k) h->alpha_sum += alpha[k];   // sequential, as MSL:139-143
     Dims &dm = h->dm;
     dm.K = K; dm.Ks = (int32_t)round_up(K, 32); dm.NT = (K + TILE - 1) / TILE; dm.lg = 2;
     if (scheme != LDAGPU_SCHEME_SPALIAS && K <= MAX_REG_TILES * TILE) {
@@ -867,7 +1005,9 @@ int ldagpu_create(int32_t K, int32_t V, int64_t D, const int64_t *doc_offsets, c
     dm.V = V; dm.Vp = (int32_t)round_up(V, PHI_ROW_BLOCK * PHI_SEGMENTS);
     dm.D = D; dm.N = doc_offsets[D]; dm.doc_base = doc_base; dm.token_base = token_base;
     h->D_global = D;
-    h->row0 = 0; h->row1 = dm.Vp; h->seg0 = 0; h->seg1 = PHI_SEGMENTS;
+    set_rank(h, 0, 1);
+    h->shard_doc0 = {0, D};
+    h->shard_tok0 = {0, dm.N};
     h->h_doc_off.assign(doc_offsets, doc_offsets + D + 1);
 
     auto body = [&]() -> int {
@@ -931,12 +1071,7 @@ int ldagpu_create(int32_t K, int32_t V, int64_t D, const int64_t *doc_offsets, c
         CK(h, cudaMemset(h->n_k.p, 0, sizeof(int32_t) * h->n_k.n));
         CK(h, cudaMemset(h->partial.p, 0, sizeof(double) * h->partial.n));
         CK(h, cudaMemset(h->seg.p, 0, sizeof(double) * h->seg.n));
-        std::vector<float> af((size_t)dm.Ks, 0.0f);
-        std::vector<double> ad((size_t)dm.Ks, 0.0);
-        for (int k = 0; k < K; ++k) { af[k] = (float)alpha[k]; ad[k] = alpha[k]; }
-        CK(h, cudaMemcpy(h->alpha_f.p, af.data(), sizeof(float) * af.size(), cudaMemcpyHostToDevice));
-        CK(h, cudaMemcpy(h->alpha_d.p, ad.data(), sizeof(double) * ad.size(), cudaMemcpyHostToDevice));
-        CK(h, launch_lgs_table(K, h->alpha_d.p, h->lgs_alpha.p, h->stream));
+        if (upload_alpha(h, alpha)) return 1;
         // type ids must be inside the alphabet (UPL:360 numTypes = alphabet.size())
         CK(h, launch_validate(dm, h->tokens.p, nullptr, h->bad.p, h->stream));
         int bad = 0;
@@ -955,7 +1090,7 @@ int ldagpu_create(int32_t K, int32_t V, int64_t D, const int64_t *doc_offsets, c
 int ldagpu_destroy(ldagpu_handle h)
 {
     if (!h) return 0;
-    if (h->multi()) return multi_destroy(h);
+    for (ldagpu_handle c : h->shards) ldagpu_destroy(c);   // a group's own buffers are all empty
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
     for (void *p : h->ipc_opened) cudaIpcCloseMemHandle(p);
@@ -999,13 +1134,7 @@ int ldagpu_comm_init(ldagpu_handle h, int32_t rank, int32_t world, const void *i
     ncclUniqueId id;
     std::memcpy(&id, id128, sizeof id);
     NK(h, g_nccl.CommInitRank(&h->comm, world, id, rank));
-    h->rank = rank;
-    h->world = world;
-    const int32_t rows = h->dm.Vp / world;
-    h->row0 = rank * rows;
-    h->row1 = h->row0 + rows;
-    h->seg0 = rank * (PHI_SEGMENTS / world);
-    h->seg1 = h->seg0 + PHI_SEGMENTS / world;
+    set_rank(h, rank, world);
     // global document count for the D * lgS(alphaSum) term of the log-likelihood
     DevBuf<long long> tmp;
     CK(h, tmp.alloc(1));
@@ -1027,25 +1156,22 @@ int ldagpu_get_exchange_mode(ldagpu_handle h, int32_t *mode)
     return 0;
 }
 
-static int refresh_counts_and_phi(ldagpu_handle h, bool redraw_phi)
-{
-    if (rendezvous(h)) return 1;
-    if (step_counts_local(h) || step_counts_exchange(h, redraw_phi)) return 1;
-    if (redraw_phi && step_phi(h, false, nullptr, true)) return 1;
-    return sync_check(h);
-}
-
 int ldagpu_init_z_java_random(ldagpu_handle h, int32_t seed)
 {
     NEED(h);
-    if (h->multi()) return multi_init_z(h, seed);
-    // the stream of nextInt(K) is sequential over the whole corpus: skip the draws of the shards before ours
+    // java.util.Random(seed).nextInt(K) is one stream over the whole corpus in document order (UPL:398-406,458-460):
+    // skip the draws of the ranks before this one, then every part takes its slice
+    const Parts parts = h->parts();
     JavaRandom r((int64_t)seed);
-    for (int64_t i = 0; i < h->dm.token_base; ++i) (void)r.nextInt(h->dm.K);
-    std::vector<int32_t> z((size_t)h->dm.N);
-    for (int64_t i = 0; i < h->dm.N; ++i) z[(size_t)i] = r.nextInt(h->dm.K);
-    if (h->dm.N) CK(h, cudaMemcpyAsync(h->z.p, z.data(), sizeof(int32_t) * z.size(), cudaMemcpyHostToDevice, h->stream));
-    CK(h, cudaStreamSynchronize(h->stream));
+    for (int64_t i = 0; i < parts[0]->dm.token_base; ++i) (void)r.nextInt(h->dm.K);
+    std::vector<int32_t> z;
+    for (ldagpu_handle c : parts) {
+        z.resize((size_t)c->dm.N);
+        for (int64_t i = 0; i < c->dm.N; ++i) z[(size_t)i] = r.nextInt(c->dm.K);
+        CK(h, cudaSetDevice(c->device));
+        if (c->dm.N) CK(h, cudaMemcpyAsync(c->z.p, z.data(), sizeof(int32_t) * z.size(), cudaMemcpyHostToDevice, c->stream));
+        CK(h, cudaStreamSynchronize(c->stream));
+    }
     return refresh_counts_and_phi(h, true);   // initialSamplePhi, UPL:450
 }
 
@@ -1060,14 +1186,11 @@ int ldagpu_init_z_java_random(ldagpu_handle h, int32_t seed)
 static int set_z_upload(ldagpu_handle h, const void *z, bool is16)
 {
     const int64_t N = h->dm.N;
-    if (!z && N) return h->fail("null z");
-    if (is16 && h->dm.K > 65536) return h->fail("16-bit topic indicators need K <= 65536");
-    const size_t N1 = (size_t)std::max<int64_t>(N, 1);
     if (!h->z_stage.p) {
-        CK(h, h->z_stage.alloc(N1 + 4));
+        CK(h, h->z_stage.alloc((size_t)std::max<int64_t>(N, 1) + 4));
         CK(h, cudaMemsetAsync(h->z_stage.p, 0, sizeof(int32_t) * h->z_stage.n, h->stream));
     }
-    if (is16 && !h->z16.p) CK(h, h->z16.alloc(N1 + 8));
+    if (is16 && ensure_z16(h)) return 1;
     CK(h, cudaMemsetAsync(h->n_wk.p, 0, sizeof(int32_t) * h->n_wk.n, h->stream));
     CK(h, cudaMemsetAsync(h->bad.p, 0, sizeof(int), h->stream));
     CK(h, cudaEventRecord(h->copy_events[0], h->stream));
@@ -1105,12 +1228,10 @@ static int set_z_read_flag(ldagpu_handle h, int *bad)
 
 // bad == 0: the staged indicators become the resident ones; otherwise the previous state is kept -- the counts are
 // rebuilt from the untouched z and exchanged like any rebuild (Phi was never touched).  Enqueues only.
-// stage < 0: everything; else stage 0 = local part + announce, 1..2 = count reduce + barrier, 3..5 = Phi draw
-static int set_z_commit(ldagpu_handle h, int bad, int32_t redraw_phi, int stage = -1)
+static int set_z_commit(ldagpu_handle h, int bad, int32_t redraw_phi, Stage stage)
 {
-    const bool all = stage < 0;
     const bool defer = !bad && redraw_phi != 0;
-    if (all || stage == 0) {
+    if (stage == ST_LOCAL) {
         if (rendezvous(h)) return 1;
         if (bad) {
             if (step_counts_local(h)) return 1;
@@ -1119,53 +1240,74 @@ static int set_z_commit(ldagpu_handle h, int bad, int32_t redraw_phi, int stage 
             CK(h, launch_topic_totals(h->dm, h->n_wk.p, h->n_k.p, h->stream));
             h->last_launches += 1;
         }
-        if (step_counts_exchange(h, defer, all ? -1 : 0)) return 1;
     }
-    if (!all && (stage == 1 || stage == 2) && step_counts_exchange(h, defer, stage)) return 1;
-    if (defer) {   // UPL:1842
-        if (all) { if (step_phi(h, false, nullptr, true)) return 1; }
-        else if (stage >= 3 && step_phi(h, false, nullptr, true, stage - 3)) return 1;
-    }
-    return 0;
+    if (step_counts_exchange(h, defer, stage)) return 1;
+    return defer && step_phi(h, false, nullptr, true, stage) ? 1 : 0;   // UPL:1842
 }
 
-static int set_z_fail(ldagpu_handle h, bool sharded)
+// z in corpus order
+static int set_z(ldagpu_handle h, const void *z, bool is16, int32_t redraw_phi)
 {
-    return h->fail("topic indicator out of range [0, %d)%s; the previous indicators stay in place", h->dm.K,   // UPL:475-481 throws
-                   sharded ? " (on this or another shard)" : "");
-}
-
-static int set_z_impl(ldagpu_handle h, const void *z, bool is16, int32_t redraw_phi)
-{
+    if (!z && h->dm.N) return h->fail("null z");
+    if (is16 && h->dm.K > 65536) return h->fail("16-bit topic indicators need K <= 65536");
+    const size_t esz = is16 ? sizeof(uint16_t) : sizeof(int32_t);
+    const Parts parts = h->parts();
+    for (size_t g = 0; g < parts.size(); ++g)
+        MC(h, parts[g], set_z_upload(parts[g], static_cast<const char *>(z) + (size_t)h->shard_tok0[g] * esz, is16));
     int bad = 0;
-    if (set_z_upload(h, z, is16) || set_z_read_flag(h, &bad) || set_z_commit(h, bad, redraw_phi) || sync_check(h)) return 1;
-    return bad ? set_z_fail(h, h->world > 1) : 0;
+    for (ldagpu_handle c : parts) {
+        int b = 0;
+        MC(h, c, set_z_read_flag(c, &b));
+        bad |= b;
+    }
+    if (run_stages(h, parts, [&](size_t g, Stage st) { return set_z_commit(parts[g], bad, redraw_phi, st); })) return 1;
+    if (sync_all(h, parts)) return 1;
+    return bad ? h->fail("topic indicator out of range [0, %d)%s; the previous indicators stay in place", h->dm.K,   // UPL:475-481 throws
+                         h->world > 1 ? " (on this or another shard)" : "")
+               : 0;
 }
 
 int ldagpu_set_z(ldagpu_handle h, const int32_t *z, int32_t redraw_phi)
 {
     NEED(h);
-    if (h->multi()) return multi_set_z(h, z, false, redraw_phi);
-    return set_z_impl(h, z, false, redraw_phi);
+    return set_z(h, z, false, redraw_phi);
 }
 
 int ldagpu_set_z16(ldagpu_handle h, const uint16_t *z, int32_t redraw_phi)
 {
     NEED(h);
-    if (h->multi()) return multi_set_z(h, z, true, redraw_phi);
-    return set_z_impl(h, z, true, redraw_phi);
+    return set_z(h, z, true, redraw_phi);
+}
+
+// the resident z of one part to the host; z16: narrowed on the device
+static int get_z_one(ldagpu_handle h, int32_t *z, uint16_t *z16)
+{
+    if (h->dm.N && ((z16 && ensure_z16(h)) || copy_z_out(h, z, z16, 0, h->dm.N, h->stream))) return 1;
+    return sync_check(h);
+}
+
+// z in corpus order
+static int get_z(ldagpu_handle h, int32_t *z, uint16_t *z16)
+{
+    const Parts parts = h->parts();
+    for (size_t g = 0; g < parts.size(); ++g) {
+        const int64_t t0 = h->shard_tok0[g];
+        MC(h, parts[g], get_z_one(parts[g], z ? z + t0 : nullptr, z16 ? z16 + t0 : nullptr));
+    }
+    return 0;
 }
 
 int ldagpu_get_z16(ldagpu_handle h, uint16_t *z)
 {
     NEED(h);
-    if (h->multi()) return multi_get_z(h, z, true);
     if (h->dm.K > 65536) return h->fail("16-bit topic indicators need K <= 65536");
-    if (!h->dm.N) return 0;
-    if (!h->z16.p) CK(h, h->z16.alloc((size_t)h->dm.N + 8));
-    CK(h, launch_pack16(h->z.p, h->z16.p, h->dm.N, h->sm_count, h->stream));
-    CK(h, cudaMemcpyAsync(z, h->z16.p, sizeof(uint16_t) * (size_t)h->dm.N, cudaMemcpyDeviceToHost, h->stream));
-    return sync_check(h);
+    return get_z(h, nullptr, z);
+}
+
+int ldagpu_get_z(ldagpu_handle h, int32_t *z)
+{
+    NEED(h);
+    return get_z(h, z, nullptr);
 }
 
 int ldagpu_sweep_get_z16(ldagpu_handle h, int32_t n, int32_t *done, uint16_t *z)
@@ -1173,8 +1315,6 @@ int ldagpu_sweep_get_z16(ldagpu_handle h, int32_t n, int32_t *done, uint16_t *z)
     NEED(h);
     if (!z && h->dm.N) return h->fail("null z");
     if (h->dm.K > 65536) return h->fail("16-bit topic indicators need K <= 65536");
-    if (h->multi()) return multi_run_sweeps(h, n, true, done, nullptr, z);
-    if (h->dm.N && !h->z16.p) CK(h, h->z16.alloc((size_t)h->dm.N + 8));
     return run_sweeps(h, n, true, done, nullptr, z);
 }
 
@@ -1182,155 +1322,141 @@ int ldagpu_sweep_get_z(ldagpu_handle h, int32_t n, int32_t *done, int32_t *z)
 {
     NEED(h);
     if (!z && h->dm.N) return h->fail("null z");
-    if (h->multi()) return multi_run_sweeps(h, n, true, done, z, nullptr);
-    return run_sweeps(h, n, true, done, z);
-}
-
-int ldagpu_get_z(ldagpu_handle h, int32_t *z)
-{
-    NEED(h);
-    if (h->multi()) return multi_get_z(h, z, false);
-    if (h->dm.N) CK(h, cudaMemcpyAsync(z, h->z.p, sizeof(int32_t) * (size_t)h->dm.N, cudaMemcpyDeviceToHost, h->stream));
-    return sync_check(h);
+    return run_sweeps(h, n, true, done, z, nullptr);
 }
 
 int ldagpu_sweep(ldagpu_handle h, int32_t n, int32_t *done)
 {
     NEED(h);
-    if (h->multi()) return multi_run_sweeps(h, n, true, done, nullptr, nullptr);
-    return run_sweeps(h, n, true, done);
+    return run_sweeps(h, n, true, done, nullptr, nullptr);
 }
 
 int ldagpu_sample_z_given_phi(ldagpu_handle h, int32_t n, int32_t *done)
 {
     NEED(h);
-    if (h->multi()) return multi_run_sweeps(h, n, false, done, nullptr, nullptr);
-    return run_sweeps(h, n, false, done);
+    return run_sweeps(h, n, false, done, nullptr, nullptr);
 }
 
+// Settings live on the parts: the setters write every part, the getters read parts[0].
 int ldagpu_next_iteration(ldagpu_handle h)
 {
     NEED(h);
-    h->iteration += 1;
-    for (ldagpu_handle c : h->shards) c->iteration = h->iteration;
+    for (ldagpu_handle c : h->parts()) c->iteration += 1;
     return 0;
 }
-int ldagpu_get_iteration(ldagpu_handle h, int32_t *it) { if (!h || !it) return 1; *it = h->iteration; return 0; }
+int ldagpu_get_iteration(ldagpu_handle h, int32_t *it) { if (!h || !it) return 1; *it = h->parts()[0]->iteration; return 0; }
 int ldagpu_set_iteration(ldagpu_handle h, int32_t it)
 {
     if (!h) return 1;
-    h->iteration = it;
-    for (ldagpu_handle c : h->shards) c->iteration = it;
+    for (ldagpu_handle c : h->parts()) c->iteration = it;
     return 0;
 }
 
 int ldagpu_sample_theta(ldagpu_handle h)
 {
     NEED(h);
-    if (h->multi()) return multi_step(h, MSTEP_THETA);
-    if (step_theta(h)) return 1;
-    return sync_check(h);
+    const Parts parts = h->parts();
+    for (ldagpu_handle c : parts) MC(h, c, step_theta(c));
+    return sync_all(h, parts);
 }
 int ldagpu_sample_z(ldagpu_handle h)
 {
     NEED(h);
-    if (h->multi()) return multi_step(h, MSTEP_Z);
-    if (step_z(h)) return 1;
-    return sync_check(h);
+    const Parts parts = h->parts();
+    for (ldagpu_handle c : parts) MC(h, c, step_z(c));
+    return sync_all(h, parts);
 }
 int ldagpu_rebuild_counts(ldagpu_handle h)
 {
     NEED(h);
-    if (h->multi()) return multi_step(h, MSTEP_COUNTS);
     return refresh_counts_and_phi(h, false);
 }
 int ldagpu_sample_phi(ldagpu_handle h)
 {
     NEED(h);
-    if (h->multi()) return multi_step(h, MSTEP_PHI);
-    bool acc = mean_this_iteration(h);
-    if (rendezvous(h)) return 1;
-    if (step_phi(h, acc, nullptr)) return 1;
-    if (acc) h->n_sampled_phi += 1;
-    return sync_check(h);
+    const Parts parts = h->parts();
+    if (run_stages(h, parts, [&](size_t g, Stage st) {
+            ldagpu_handle c = parts[g];
+            if (st == ST_LOCAL && rendezvous(c)) return 1;
+            return step_phi(c, mean_this_iteration(c), nullptr, false, st);
+        }))
+        return 1;
+    for (ldagpu_handle c : parts)
+        if (mean_this_iteration(c)) c->n_sampled_phi += 1;
+    return sync_all(h, parts);
 }
 
 int ldagpu_get_type_topic_counts(ldagpu_handle h, int32_t *out)
 {
     NEED(h);
-    if (h->multi()) return multi_get_type_topic_counts(h, out);
-    const size_t cells = (size_t)h->dm.V * h->dm.K;
-    if (h->world > 1 && h->comm) {
-        // every rank holds the global counts of its vocabulary slice only: gather the slices
-        const size_t slice = (size_t)(h->dm.Vp / h->world) * h->dm.Ks;
-        NK(h, g_nccl.AllGather(h->n_wk.p + (size_t)h->rank * slice, h->n_wk.p, slice, ncclInt32, h->comm, h->stream));
-    }
-    CK(h, h->scratch_i32.alloc(cells));
-    CK(h, launch_export_counts(h->dm, h->n_wk.p, h->scratch_i32.p, h->stream));
-    CK(h, cudaMemcpyAsync(out, h->scratch_i32.p, sizeof(int32_t) * cells, cudaMemcpyDeviceToHost, h->stream));
-    int rc = sync_check(h);
-    h->scratch_i32.release();
-    return rc;
+    const Parts parts = h->parts();
+    if (gather_rows(h, parts, &ldagpu_handle_s::n_wk, ncclInt32)) return 1;
+    ldagpu_handle c = parts[0];
+    MC(h, c, via_scratch(c, c->scratch_i32, (size_t)c->dm.V * c->dm.K, out, nullptr,
+                         [&](int32_t *s) { CK(c, launch_export_counts(c->dm, c->n_wk.p, s, c->stream)); return 0; }));
+    return 0;
 }
 
 int ldagpu_get_topic_totals(ldagpu_handle h, int32_t *n_k)
 {
     NEED(h);
-    if (h->multi()) return ldagpu_get_topic_totals(h->shards[0], n_k) ? (h->err = h->shards[0]->err, 1) : 0;
-    CK(h, cudaMemcpyAsync(n_k, h->n_k.p, sizeof(int32_t) * (size_t)h->dm.K, cudaMemcpyDeviceToHost, h->stream));
-    return sync_check(h);
+    ldagpu_handle c = h->parts()[0];
+    CK(h, cudaSetDevice(c->device));
+    CK(h, cudaMemcpyAsync(n_k, c->n_k.p, sizeof(int32_t) * (size_t)c->dm.K, cudaMemcpyDeviceToHost, c->stream));
+    MC(h, c, sync_check(c));
+    return 0;
 }
 
+// per document, in corpus order
 int ldagpu_get_doc_topic_counts(ldagpu_handle h, int32_t *n_dk)
 {
     NEED(h);
-    if (h->multi()) return multi_get_doc_topic_counts(h, n_dk);
-    const size_t cells = (size_t)h->dm.D * h->dm.K;
-    if (cells == 0) return 0;
-    CK(h, h->scratch_i32.alloc(cells));
-    CK(h, launch_doc_topic_counts(h->dm, h->doc_off.p, h->z.p, h->scratch_i32.p, h->stream));
-    CK(h, cudaMemcpyAsync(n_dk, h->scratch_i32.p, sizeof(int32_t) * cells, cudaMemcpyDeviceToHost, h->stream));
-    int rc = sync_check(h);
-    h->scratch_i32.release();
-    return rc;
+    const Parts parts = h->parts();
+    for (size_t g = 0; g < parts.size(); ++g) {
+        ldagpu_handle c = parts[g];
+        const size_t cells = (size_t)c->dm.D * c->dm.K;
+        if (cells == 0) continue;
+        MC(h, c, via_scratch(c, c->scratch_i32, cells, n_dk + (size_t)h->shard_doc0[g] * h->dm.K, nullptr,
+                             [&](int32_t *s) { CK(c, launch_doc_topic_counts(c->dm, c->doc_off.p, c->z.p, s, c->stream)); return 0; }));
+    }
+    return 0;
 }
 
 int ldagpu_get_phi(ldagpu_handle h, double *phi)
 {
     NEED(h);
-    if (h->multi()) return ldagpu_get_phi(h->shards[0], phi) ? (h->err = h->shards[0]->err, 1) : 0;   // replicated
-    const size_t cells = (size_t)h->dm.V * h->dm.K;
-    CK(h, h->scratch_f64.alloc(cells));
-    CK(h, launch_export_phi(h->dm, h->phiT.p, h->scratch_f64.p, h->stream));
-    CK(h, cudaMemcpyAsync(phi, h->scratch_f64.p, sizeof(double) * cells, cudaMemcpyDeviceToHost, h->stream));
-    int rc = sync_check(h);
-    h->scratch_f64.release();
-    return rc;
+    ldagpu_handle c = h->parts()[0];   // Phi is replicated
+    MC(h, c, via_scratch(c, c->scratch_f64, (size_t)c->dm.V * c->dm.K, phi, nullptr,
+                         [&](double *s) { CK(c, launch_export_phi(c->dm, c->phiT.p, s, c->stream)); return 0; }));
+    return 0;
 }
 
-int ldagpu_set_phi(ldagpu_handle h, const double *phi)
+static int set_phi_one(ldagpu_handle h, const double *phi)
 {
-    NEED(h);
-    if (h->multi()) return multi_set_phi(h, phi);
-    const size_t cells = (size_t)h->dm.V * h->dm.K;
-    CK(h, h->scratch_f64.alloc(cells));
-    CK(h, cudaMemcpyAsync(h->scratch_f64.p, phi, sizeof(double) * cells, cudaMemcpyHostToDevice, h->stream));
-    CK(h, launch_import_phi(h->dm, h->scratch_f64.p, h->phiT.p, h->stream));
-    if (step_alias(h)) return 1;
-    int rc = sync_check(h);
-    h->scratch_f64.release();
+    int rc = via_scratch(h, h->scratch_f64, (size_t)h->dm.V * h->dm.K, nullptr, phi, [&](double *s) {
+        CK(h, launch_import_phi(h->dm, s, h->phiT.p, h->stream));
+        return step_alias(h);
+    });
     // UPL:1897-1903: setPhi resets the running mean
     if (h->phi_mean.p) CK(h, cudaMemset(h->phi_mean.p, 0, sizeof(double) * h->phi_mean.n));
     h->n_sampled_phi = 0;
     return rc;
 }
 
+int ldagpu_set_phi(ldagpu_handle h, const double *phi)
+{
+    NEED(h);
+    for (ldagpu_handle c : h->parts()) MC(h, c, set_phi_one(c, phi));
+    return 0;
+}
+
 int ldagpu_set_phi_mean_schedule(ldagpu_handle h, int32_t burn_in, int32_t thin)
 {
     if (!h) return 1;
-    h->mean_burn_in = burn_in;
-    h->mean_thin = thin < 1 ? 1 : thin;
-    for (ldagpu_handle c : h->shards) { c->mean_burn_in = h->mean_burn_in; c->mean_thin = h->mean_thin; }
+    for (ldagpu_handle c : h->parts()) {
+        c->mean_burn_in = burn_in;
+        c->mean_thin = thin < 1 ? 1 : thin;
+    }
     return 0;
 }
 
@@ -1340,62 +1466,58 @@ int ldagpu_set_phi_sampler(ldagpu_handle h, int32_t sampler, int32_t alias_poiss
     if (sampler != LDAGPU_PHI_GAMMA && sampler != LDAGPU_PHI_POLYA_URN) return h->fail("unknown Phi sampler");
     if (sampler == LDAGPU_PHI_POLYA_URN && (alias_poisson_threshold < 1 || alias_poisson_threshold > (1 << 20)))
         return h->fail("alias_poisson_threshold must be in [1, 2^20]");
-    h->poisson_L = sampler == LDAGPU_PHI_POLYA_URN ? alias_poisson_threshold : 0;
-    for (ldagpu_handle c : h->shards) c->poisson_L = h->poisson_L;
+    for (ldagpu_handle c : h->parts()) c->poisson_L = sampler == LDAGPU_PHI_POLYA_URN ? alias_poisson_threshold : 0;
     return 0;
 }
 
 int ldagpu_get_phi_mean(ldagpu_handle h, double *phi_mean, int32_t *n_sampled)
 {
     NEED(h);
-    if (h->multi()) return multi_get_phi_mean(h, phi_mean, n_sampled);
-    if (n_sampled) *n_sampled = h->n_sampled_phi;
-    if (h->n_sampled_phi == 0 || !h->phi_mean.p) return 0;   // UPL:1955-1958 returns null
-    if (h->world > 1 && h->comm) {
-        const size_t slice = (size_t)(h->dm.Vp / h->world) * h->dm.Ks;
-        NK(h, g_nccl.AllGather(h->phi_mean.p + (size_t)h->rank * slice, h->phi_mean.p, slice, ncclDouble, h->comm, h->stream));
+    const Parts parts = h->parts();
+    ldagpu_handle c = parts[0];
+    if (n_sampled) *n_sampled = c->n_sampled_phi;
+    if (c->n_sampled_phi == 0 || !c->phi_mean.p) return 0;   // UPL:1955-1958 returns null
+    if (gather_rows(h, parts, &ldagpu_handle_s::phi_mean, ncclDouble)) return 1;
+    MC(h, c, via_scratch(c, c->scratch_f64, (size_t)c->dm.V * c->dm.K, phi_mean, nullptr, [&](double *s) {
+           CK(c, launch_export_mean(c->dm, c->phi_mean.p, 1.0 / (double)c->n_sampled_phi, s, c->stream));
+           return 0;
+       }));
+    return 0;
+}
+
+// theta_out != nullptr: export theta, else import theta_in; both per document, in corpus order
+static int theta_io(ldagpu_handle h, double *theta_out, const double *theta_in)
+{
+    const Parts parts = h->parts();
+    for (size_t g = 0; g < parts.size(); ++g) {
+        ldagpu_handle c = parts[g];
+        MC(h, c, ensure_theta(c));
+        const size_t cells = (size_t)c->dm.D * c->dm.K, o = (size_t)h->shard_doc0[g] * h->dm.K;
+        if (cells == 0) continue;
+        MC(h, c, via_scratch(c, c->scratch_f64, cells, theta_out ? theta_out + o : nullptr, theta_in ? theta_in + o : nullptr,
+                             [&](double *s) {
+                                 CK(c, theta_out ? launch_export_theta(c->dm, c->theta.p, s, c->stream)
+                                                 : launch_import_theta(c->dm, s, c->theta.p, c->stream));
+                                 return 0;
+                             }));
     }
-    const size_t cells = (size_t)h->dm.V * h->dm.K;
-    CK(h, h->scratch_f64.alloc(cells));
-    CK(h, launch_export_mean(h->dm, h->phi_mean.p, 1.0 / (double)h->n_sampled_phi, h->scratch_f64.p, h->stream));
-    CK(h, cudaMemcpyAsync(phi_mean, h->scratch_f64.p, sizeof(double) * cells, cudaMemcpyDeviceToHost, h->stream));
-    int rc = sync_check(h);
-    h->scratch_f64.release();
-    return rc;
+    return 0;
 }
 
 int ldagpu_get_theta(ldagpu_handle h, double *theta)
 {
     NEED(h);
-    if (h->multi()) return multi_theta(h, theta, nullptr);
-    if (ensure_theta(h)) return 1;
-    const size_t cells = (size_t)h->dm.D * h->dm.K;
-    if (cells == 0) return 0;
-    CK(h, h->scratch_f64.alloc(cells));
-    CK(h, launch_export_theta(h->dm, h->theta.p, h->scratch_f64.p, h->stream));
-    CK(h, cudaMemcpyAsync(theta, h->scratch_f64.p, sizeof(double) * cells, cudaMemcpyDeviceToHost, h->stream));
-    int rc = sync_check(h);
-    h->scratch_f64.release();
-    return rc;
+    return theta_io(h, theta, nullptr);
 }
 
 int ldagpu_set_theta(ldagpu_handle h, const double *theta)
 {
     NEED(h);
-    if (h->multi()) return multi_theta(h, nullptr, theta);
-    if (ensure_theta(h)) return 1;
-    const size_t cells = (size_t)h->dm.D * h->dm.K;
-    if (cells == 0) return 0;
-    CK(h, h->scratch_f64.alloc(cells));
-    CK(h, cudaMemcpyAsync(h->scratch_f64.p, theta, sizeof(double) * cells, cudaMemcpyHostToDevice, h->stream));
-    CK(h, launch_import_theta(h->dm, h->scratch_f64.p, h->theta.p, h->stream));
-    int rc = sync_check(h);
-    h->scratch_f64.release();
-    return rc;
+    return theta_io(h, nullptr, theta);
 }
 
-// this shard's three partial sums of the log-likelihood into red_out[0..2] (enqueue only): document part, type part
-// over the shard's vocabulary rows, and the number of non-zero cells there
+// this part's three partial sums of the log-likelihood into red_out[0..2] (enqueue only): document part, type part
+// over the part's vocabulary rows, and the number of non-zero cells there
 static int ll_partials(ldagpu_handle h)
 {
     CK(h, launch_ll_doc(h->dm, h->doc_off.p, h->z.p, h->alpha_d.p, h->lgs_alpha.p, h->alpha_sum, h->red.p, N_PARTIALS, h->sm_count,
@@ -1430,30 +1552,41 @@ static int lp_partials(ldagpu_handle h)
     return 0;
 }
 
+// the three partial sums of every part, combined: an NCCL all-reduce between the ranks, a host sum in fixed shard order
+// (reproducible) over the shards of a group.  nk != nullptr: also n_k, from parts[0]
+static int sum_partials(ldagpu_handle h, bool ll, double part[3], std::vector<int32_t> *nk)
+{
+    const Parts parts = h->parts();
+    for (ldagpu_handle c : parts) MC(h, c, ll ? ll_partials(c) : lp_partials(c));
+    if (h->world > 1 && h->comm) NK(h, g_nccl.AllReduce(h->red_out.p, h->red_out.p, 3, ncclDouble, ncclSum, h->comm, h->stream));
+    part[0] = part[1] = part[2] = 0.0;
+    for (ldagpu_handle c : parts) {
+        double q[3];
+        CK(h, cudaSetDevice(c->device));
+        CK(h, cudaMemcpyAsync(q, c->red_out.p, sizeof q, cudaMemcpyDeviceToHost, c->stream));
+        if (nk && c == parts[0])
+            CK(h, cudaMemcpyAsync(nk->data(), c->n_k.p, sizeof(int32_t) * nk->size(), cudaMemcpyDeviceToHost, c->stream));
+        MC(h, c, sync_check(c));
+        part[0] += q[0]; part[1] += q[1]; part[2] += q[2];
+    }
+    return 0;
+}
+
 int ldagpu_log_likelihood(ldagpu_handle h, double *ll)
 {
     NEED(h);
-    if (h->multi()) return multi_log_likelihood(h, ll);
-    if (ll_partials(h)) return 1;
-    if (h->world > 1) NK(h, g_nccl.AllReduce(h->red_out.p, h->red_out.p, 3, ncclDouble, ncclSum, h->comm, h->stream));
     double part[3];
     std::vector<int32_t> nk((size_t)h->dm.K);
-    CK(h, cudaMemcpyAsync(part, h->red_out.p, sizeof part, cudaMemcpyDeviceToHost, h->stream));
-    CK(h, cudaMemcpyAsync(nk.data(), h->n_k.p, sizeof(int32_t) * nk.size(), cudaMemcpyDeviceToHost, h->stream));
-    if (sync_check(h)) return 1;
-    *ll = ll_finish(h, part, nk);
+    if (sum_partials(h, true, part, &nk)) return 1;
+    *ll = ll_finish(h->parts()[0], part, nk);
     return 0;
 }
 
 int ldagpu_log_posterior(ldagpu_handle h, double *lp)
 {
     NEED(h);
-    if (h->multi()) return multi_log_posterior(h, lp);
-    if (lp_partials(h)) return 1;
-    if (h->world > 1) NK(h, g_nccl.AllReduce(h->red_out.p, h->red_out.p, 3, ncclDouble, ncclSum, h->comm, h->stream));
     double part[3];
-    CK(h, cudaMemcpyAsync(part, h->red_out.p, sizeof part, cudaMemcpyDeviceToHost, h->stream));
-    if (sync_check(h)) return 1;
+    if (sum_partials(h, false, part, nullptr)) return 1;
     *lp = part[0] + part[1] + part[2];
     return 0;
 }
@@ -1461,26 +1594,29 @@ int ldagpu_log_posterior(ldagpu_handle h, double *lp)
 int ldagpu_abort(ldagpu_handle h)
 {
     if (!h) return 1;
-    h->abort_flag.store(1);
-    for (ldagpu_handle c : h->shards) c->abort_flag.store(1);
+    for (ldagpu_handle c : h->parts()) c->abort_flag.store(1);
     return 0;
 }
-int ldagpu_get_abort(ldagpu_handle h, int32_t *aborted) { if (!h || !aborted) return 1; *aborted = h->abort_flag.load(); return 0; }
+int ldagpu_get_abort(ldagpu_handle h, int32_t *aborted)
+{
+    if (!h || !aborted) return 1;
+    *aborted = h->parts()[0]->abort_flag.load();
+    return 0;
+}
 
+// the slowest part sets the pace of every phase
 int ldagpu_get_timers(ldagpu_handle h, double *z_ms, double *counts_ms, double *phi_ms, double *comm_ms)
 {
     if (!h) return 1;
-    if (h->multi()) {   // the slowest shard sets the pace of every phase
-        h->t_z = h->t_counts = h->t_phi = h->t_comm = 0;
-        for (ldagpu_handle c : h->shards) {
-            h->t_z = std::max(h->t_z, c->t_z); h->t_counts = std::max(h->t_counts, c->t_counts);
-            h->t_phi = std::max(h->t_phi, c->t_phi); h->t_comm = std::max(h->t_comm, c->t_comm);
-        }
+    double t[4] = {0, 0, 0, 0};
+    for (ldagpu_handle c : h->parts()) {
+        t[0] = std::max(t[0], c->t_z); t[1] = std::max(t[1], c->t_counts);
+        t[2] = std::max(t[2], c->t_phi); t[3] = std::max(t[3], c->t_comm);
     }
-    if (z_ms) *z_ms = h->t_z;
-    if (counts_ms) *counts_ms = h->t_counts;
-    if (phi_ms) *phi_ms = h->t_phi;
-    if (comm_ms) *comm_ms = h->t_comm;
+    if (z_ms) *z_ms = t[0];
+    if (counts_ms) *counts_ms = t[1];
+    if (phi_ms) *phi_ms = t[2];
+    if (comm_ms) *comm_ms = t[3];
     return 0;
 }
 
@@ -1498,59 +1634,27 @@ int ldagpu_get_last_call_stats(ldagpu_handle h, double *call_ms, double *z_kerne
 // =============================================================================================
 // Single-process multi-GPU: ldagpu_create_multi.
 // The reference drives everything from ONE coordinator thread of one JVM (tui/ParallelLDA.java:173-202,
-// UPL:552-943); so does this layer: the handle it returns owns one shard handle per GPU and every entry point
-// enqueues its work on all shards before it waits for any of them.  The exchange is the peer-memory one
+// UPL:552-943); so does this layer: the handle it returns owns one shard handle per GPU, and every entry point fans
+// out over them (ldagpu_handle_s::parts) and enqueues its work on all shards before it waits for any of them.  The exchange is the peer-memory one
 // (kernels_p2p.cu, kernels_phi.cu) over direct peer pointers (cudaDeviceEnablePeerAccess) -- no IPC, no NCCL,
 // the same fused Phi kernels.  Results are those of the one-process-per-GPU path and of a single GPU, bit for
 // bit: counters are keyed by global indices and the integer sums are order independent.
 // =============================================================================================
-static int multi_fail(ldagpu_handle P, ldagpu_handle c)
-{
-    P->err = c->err;
-    return 1;
-}
-#define MC(P, c, call)                               \
-    do {                                             \
-        cudaSetDevice((c)->device);                  \
-        if (call) return multi_fail(P, c);           \
-    } while (0)
-
-static int multi_sync_all(ldagpu_handle P)
-{
-    for (ldagpu_handle c : P->shards) MC(P, c, sync_check(c));
-    return 0;
-}
-
 static int multi_link_shards(ldagpu_handle P)
 {
     const int G = (int)P->shards.size();
-    const char *to = getenv("LDAGPU_P2P_TIMEOUT_MS");
     for (int g = 0; g < G; ++g) {
         ldagpu_handle c = P->shards[(size_t)g];
         cudaSetDevice(c->device);
-        c->rank = g; c->world = G; c->comm = nullptr; c->D_global = P->dm.D;
-        const int32_t rows = c->dm.Vp / G;
-        c->row0 = g * rows; c->row1 = c->row0 + rows;
-        c->seg0 = g * (PHI_SEGMENTS / G); c->seg1 = c->seg0 + PHI_SEGMENTS / G;
-        CK(c, c->nk_parts.alloc((size_t)P2P_MAX * c->dm.Ks));
-        CK(c, c->p2p_flags.alloc((size_t)P2P_FLAG_KINDS * P2P_MAX));
-        CK(c, c->p2p_local.alloc((size_t)P2P_FLAG_KINDS + 4));
-        CK(c, cudaMemset(c->nk_parts.p, 0, sizeof(int32_t) * c->nk_parts.n));
-        CK(c, cudaMemset(c->p2p_flags.p, 0, sizeof(uint32_t) * c->p2p_flags.n));
-        CK(c, cudaMemset(c->p2p_local.p, 0, sizeof(uint32_t) * c->p2p_local.n));
+        c->comm = nullptr; c->D_global = P->dm.D;
+        set_rank(c, g, G);
+        if (init_peer_table(c)) return 1;
     }
-    for (int g = 0; g < G; ++g) {
-        ldagpu_handle c = P->shards[(size_t)g];
-        PeerTable &pt = c->pt;
-        pt = PeerTable{};
-        pt.rank = g; pt.world = G;
-        pt.done_ctr = c->p2p_local.p;
-        pt.error = reinterpret_cast<int *>(c->p2p_local.p + P2P_FLAG_KINDS);
-        pt.timeout_ns = (unsigned long long)(to ? std::max(1L, atol(to)) : 60000L) * 1000000ull;
+    for (ldagpu_handle c : P->shards) {
         for (int r = 0; r < G; ++r) {
             ldagpu_handle o = P->shards[(size_t)r];
-            pt.n_wk[r] = o->n_wk.p; pt.phiT[r] = o->phiT.p; pt.seg[r] = o->seg.p;
-            pt.nk_parts[r] = o->nk_parts.p; pt.flags[r] = o->p2p_flags.p;
+            c->pt.n_wk[r] = o->n_wk.p; c->pt.phiT[r] = o->phiT.p; c->pt.seg[r] = o->seg.p;
+            c->pt.nk_parts[r] = o->nk_parts.p; c->pt.flags[r] = o->p2p_flags.p;
         }
         c->p2p = true;
         c->p2p_note = "single process, direct peer pointers";
@@ -1615,7 +1719,7 @@ int ldagpu_create_multi(int32_t K, int32_t V, int64_t D, const int64_t *doc_offs
         ldagpu_handle c = nullptr;
         if (ldagpu_create(K, V, d1 - d0, loc.data(), tokens ? tokens + t0 : nullptr, alpha, beta, seed, scheme, dev[(size_t)g],
                           d0, t0, &c)) {
-            multi_destroy(P);
+            ldagpu_destroy(P);
             return 1;   // g_create_error holds the shard's message
         }
         P->shards.push_back(c);
@@ -1623,7 +1727,7 @@ int ldagpu_create_multi(int32_t K, int32_t V, int64_t D, const int64_t *doc_offs
     if (multi_link_shards(P)) {
         for (ldagpu_handle c : P->shards)
             if (!c->err.empty()) g_create_error = c->err;
-        multi_destroy(P);
+        ldagpu_destroy(P);
         return 1;
     }
     *out = P;
@@ -1633,231 +1737,8 @@ int ldagpu_create_multi(int32_t K, int32_t V, int64_t D, const int64_t *doc_offs
 int ldagpu_get_shards(ldagpu_handle h, int32_t *n_shards, int64_t *first_docs /*[n+1] or null*/)
 {
     if (!h || !n_shards) return 1;
-    *n_shards = h->multi() ? (int32_t)h->shards.size() : 1;
-    if (first_docs) {
-        if (h->multi()) for (size_t g = 0; g < h->shard_doc0.size(); ++g) first_docs[g] = h->shard_doc0[g];
-        else { first_docs[0] = 0; first_docs[1] = h->dm.D; }
-    }
-    return 0;
-}
-
-static int multi_destroy(ldagpu_handle P)
-{
-    for (ldagpu_handle c : P->shards) {
-        c->p2p = false;     // peer pointers are plain device pointers of the other shards: nothing to unmap
-        ldagpu_destroy(c);
-    }
-    P->shards.clear();
-    delete P;
-    return 0;
-}
-
-// initial z = java.util.Random(seed).nextInt(K) over the WHOLE corpus in document order (UPL:398-406,458-460): one
-// pass, each shard takes its slice; then counts, exchange and the initial Phi on all shards
-static int multi_init_z(ldagpu_handle P, int32_t seed)
-{
-    JavaRandom r((int64_t)seed);
-    std::vector<int32_t> z;
-    for (ldagpu_handle c : P->shards) {
-        z.resize((size_t)c->dm.N);
-        for (int64_t i = 0; i < c->dm.N; ++i) z[(size_t)i] = r.nextInt(c->dm.K);
-        cudaSetDevice(c->device);
-        if (c->dm.N) {
-            CK(P, cudaMemcpyAsync(c->z.p, z.data(), sizeof(int32_t) * z.size(), cudaMemcpyHostToDevice, c->stream));
-            CK(P, cudaStreamSynchronize(c->stream));
-        }
-    }
-    for (ldagpu_handle c : P->shards) MC(P, c, step_counts_local(c) || step_counts_exchange(c, true, 0));
-    for (int st = 0; st < PHI_STAGES; ++st)
-        for (ldagpu_handle c : P->shards) MC(P, c, step_phi(c, false, nullptr, true, st));   // UPL:450
-    return multi_sync_all(P);
-}
-
-static int multi_set_z(ldagpu_handle P, const void *z, bool is16, int32_t redraw_phi)
-{
-    if (!z && P->dm.N) return P->fail("null z");
-    const size_t esz = is16 ? sizeof(uint16_t) : sizeof(int32_t);
-    const int G = (int)P->shards.size();
-    for (int g = 0; g < G; ++g)
-        MC(P, P->shards[(size_t)g], set_z_upload(P->shards[(size_t)g], static_cast<const char *>(z) + (size_t)P->shard_tok0[(size_t)g] * esz, is16));
-    int any = 0;
-    for (ldagpu_handle c : P->shards) {
-        int bad = 0;
-        MC(P, c, set_z_read_flag(c, &bad));
-        any |= bad;
-    }
-    for (int st = 0; st < SWEEP_STAGES; ++st)
-        for (ldagpu_handle c : P->shards) MC(P, c, set_z_commit(c, any, redraw_phi, st));
-    if (multi_sync_all(P)) return 1;
-    return any ? set_z_fail(P, true) : 0;
-}
-
-static int multi_get_z(ldagpu_handle P, void *z, bool is16)
-{
-    const int G = (int)P->shards.size();
-    for (int g = 0; g < G; ++g) {
-        ldagpu_handle c = P->shards[(size_t)g];
-        const int64_t t0 = P->shard_tok0[(size_t)g];
-        if (is16) MC(P, c, ldagpu_get_z16(c, static_cast<uint16_t *>(z) + t0));
-        else MC(P, c, ldagpu_get_z(c, static_cast<int32_t *>(z) + t0));
-    }
-    return 0;
-}
-
-// n sweeps on all shards: sweep s is enqueued on every shard before sweep s + 1 on any (a shard's kernels wait, on
-// the device, for the other shards' kernels of the same sweep); the abort flag is looked at before every sweep
-// and stops all shards at the same one (UPL:645)
-static int multi_run_sweeps(ldagpu_handle P, int32_t n, bool with_phi, int32_t *done, int32_t *z_out, uint16_t *z16_out)
-{
-    if (done) *done = 0;
-    const int G = (int)P->shards.size();
-    std::vector<SweepCall> calls((size_t)G);
-    for (int g = 0; g < G; ++g) {
-        ldagpu_handle c = P->shards[(size_t)g];
-        SweepCall &sc = calls[(size_t)g];
-        sc.n = n; sc.with_phi = with_phi;
-        sc.z_out = z_out ? z_out + P->shard_tok0[(size_t)g] : nullptr;
-        sc.z16_out = z16_out ? z16_out + P->shard_tok0[(size_t)g] : nullptr;
-        cudaSetDevice(c->device);
-        if (sc.z16_out && c->dm.N && !c->z16.p) CK(P, c->z16.alloc((size_t)c->dm.N + 8));
-        MC(P, c, sweeps_prepare(c, sc));
-    }
-    P->last_call_ms = 0; P->last_zk_ms = 0; P->last_zk_launches = 0; P->last_launches = 0;
-    if (n <= 0) return 0;
-    int32_t ran = 0;
-    for (int32_t s = 0; s < n; ++s) {
-        if (P->abort_flag.load(std::memory_order_relaxed)) break;
-        // fault injection for the tests of the bounded waits: LDAGPU_FAULT_STALL_SHARD=g leaves shard g's Phi stages
-        // out, as if its process had died -- the other shards must report a timeout instead of hanging
-        static const int stall = getenv("LDAGPU_FAULT_STALL_SHARD") ? atoi(getenv("LDAGPU_FAULT_STALL_SHARD")) : -1;
-        for (int st = 0; st < SWEEP_STAGES; ++st)
-            for (int g = 0; g < G; ++g) {
-                if (g == stall && st >= 3) { if (st == SWEEP_STAGES - 1) calls[(size_t)g].ran += 1; continue; }
-                MC(P, P->shards[(size_t)g], sweep_enqueue(P->shards[(size_t)g], calls[(size_t)g], st));
-            }
-        ++ran;
-    }
-    for (int g = 0; g < G; ++g) {
-        // a stopped call still owes the caller its z: sweeps_finish copies it when the last sweep did not
-        if (ran < n) calls[(size_t)g].z_copied = false;
-        MC(P, P->shards[(size_t)g], sweeps_finish(P->shards[(size_t)g], calls[(size_t)g]));
-    }
-    P->iteration = P->shards[0]->iteration;
-    for (ldagpu_handle c : P->shards) {
-        P->last_call_ms = std::max(P->last_call_ms, c->last_call_ms);
-        P->last_zk_ms = std::max(P->last_zk_ms, c->last_zk_ms);
-        P->last_zk_launches = std::max(P->last_zk_launches, c->last_zk_launches);
-        P->last_launches += c->last_launches;
-    }
-    if (done) *done = ran;
-    return 0;
-}
-
-static int multi_step(ldagpu_handle P, int what)
-{
-    if (what == MSTEP_THETA) for (ldagpu_handle c : P->shards) MC(P, c, step_theta(c));
-    if (what == MSTEP_Z) for (ldagpu_handle c : P->shards) MC(P, c, step_z(c));
-    if (what == MSTEP_COUNTS) {
-        for (ldagpu_handle c : P->shards) MC(P, c, step_counts_local(c) || step_counts_exchange(c, false, 0));
-        for (int st = 1; st < EXCH_STAGES; ++st)
-            for (ldagpu_handle c : P->shards) MC(P, c, step_counts_exchange(c, false, st));
-    }
-    if (what == MSTEP_PHI) {
-        for (int st = 0; st < PHI_STAGES; ++st)
-            for (ldagpu_handle c : P->shards) MC(P, c, step_phi(c, mean_this_iteration(c), nullptr, false, st));
-        for (ldagpu_handle c : P->shards)
-            if (mean_this_iteration(c)) c->n_sampled_phi += 1;
-    }
-    return multi_sync_all(P);
-}
-
-// every shard holds the global counts (and the Phi-mean sums) of its vocabulary rows only: collect the slices on
-// shard 0 (peer copies) and export from there
-static int multi_gather_rows(ldagpu_handle P, bool mean)
-{
-    ldagpu_handle c0 = P->shards[0];
-    for (size_t g = 1; g < P->shards.size(); ++g) {
-        ldagpu_handle c = P->shards[g];
-        const size_t o = (size_t)c->row0 * c->dm.Ks, cnt = (size_t)(c->row1 - c->row0) * c->dm.Ks;
-        cudaSetDevice(c->device);
-        if (mean) {
-            if (!c->phi_mean.p || !c0->phi_mean.p) continue;
-            CK(P, cudaMemcpyPeerAsync(c0->phi_mean.p + o, c0->device, c->phi_mean.p + o, c->device, sizeof(double) * cnt, c->stream));
-        } else {
-            CK(P, cudaMemcpyPeerAsync(c0->n_wk.p + o, c0->device, c->n_wk.p + o, c->device, sizeof(int32_t) * cnt, c->stream));
-        }
-        CK(P, cudaStreamSynchronize(c->stream));
-    }
-    return 0;
-}
-
-static int multi_get_type_topic_counts(ldagpu_handle P, int32_t *out)
-{
-    if (multi_gather_rows(P, false)) return 1;
-    MC(P, P->shards[0], ldagpu_get_type_topic_counts(P->shards[0], out));
-    return 0;
-}
-
-static int multi_get_doc_topic_counts(ldagpu_handle P, int32_t *out)
-{
-    for (size_t g = 0; g < P->shards.size(); ++g)
-        MC(P, P->shards[g], ldagpu_get_doc_topic_counts(P->shards[g], out + (size_t)P->shard_doc0[g] * P->dm.K));
-    return 0;
-}
-
-static int multi_set_phi(ldagpu_handle P, const double *phi)
-{
-    for (ldagpu_handle c : P->shards) MC(P, c, ldagpu_set_phi(c, phi));
-    return 0;
-}
-
-static int multi_get_phi_mean(ldagpu_handle P, double *phi_mean, int32_t *n_sampled)
-{
-    if (multi_gather_rows(P, true)) return 1;
-    MC(P, P->shards[0], ldagpu_get_phi_mean(P->shards[0], phi_mean, n_sampled));
-    return 0;
-}
-
-static int multi_theta(ldagpu_handle P, double *theta_out, const double *theta_in)
-{
-    for (size_t g = 0; g < P->shards.size(); ++g) {
-        const size_t o = (size_t)P->shard_doc0[g] * P->dm.K;
-        if (theta_out) MC(P, P->shards[g], ldagpu_get_theta(P->shards[g], theta_out + o));
-        else MC(P, P->shards[g], ldagpu_set_theta(P->shards[g], theta_in + o));
-    }
-    return 0;
-}
-
-static int multi_sum_partials(ldagpu_handle P, bool ll, double part[3])
-{
-    for (ldagpu_handle c : P->shards) MC(P, c, ll ? ll_partials(c) : lp_partials(c));
-    part[0] = part[1] = part[2] = 0.0;
-    for (ldagpu_handle c : P->shards) {   // fixed shard order: the sum is reproducible
-        double q[3];
-        cudaSetDevice(c->device);
-        CK(P, cudaMemcpyAsync(q, c->red_out.p, sizeof q, cudaMemcpyDeviceToHost, c->stream));
-        MC(P, c, sync_check(c));
-        part[0] += q[0]; part[1] += q[1]; part[2] += q[2];
-    }
-    return 0;
-}
-
-static int multi_log_likelihood(ldagpu_handle P, double *ll)
-{
-    double part[3];
-    if (multi_sum_partials(P, true, part)) return 1;
-    ldagpu_handle c0 = P->shards[0];
-    std::vector<int32_t> nk((size_t)c0->dm.K);
-    MC(P, c0, ldagpu_get_topic_totals(c0, nk.data()));
-    *ll = ll_finish(c0, part, nk);
-    return 0;
-}
-
-static int multi_log_posterior(ldagpu_handle P, double *lp)
-{
-    double part[3];
-    if (multi_sum_partials(P, false, part)) return 1;
-    *lp = part[0] + part[1] + part[2];
+    *n_shards = (int32_t)h->shard_doc0.size() - 1;
+    if (first_docs) std::copy(h->shard_doc0.begin(), h->shard_doc0.end(), first_docs);
     return 0;
 }
 
@@ -1867,18 +1748,9 @@ static int multi_log_posterior(ldagpu_handle P, double *lp)
 // new values back.
 static int set_alpha_one(ldagpu_handle h, const double *alpha)
 {
-    const int K = h->dm.K;
-    for (int k = 0; k < K; ++k)
+    for (int k = 0; k < h->dm.K; ++k)
         if (!(alpha[k] > 0.0)) return h->fail("alpha must be > 0");
-    h->alpha.assign(alpha, alpha + K);
-    h->alpha_sum = 0.0;
-    for (int k = 0; k < K; ++k) h->alpha_sum += alpha[k];
-    std::vector<float> af((size_t)h->dm.Ks, 0.0f);
-    std::vector<double> ad((size_t)h->dm.Ks, 0.0);
-    for (int k = 0; k < K; ++k) { af[(size_t)k] = (float)alpha[k]; ad[(size_t)k] = alpha[k]; }
-    CK(h, cudaMemcpyAsync(h->alpha_f.p, af.data(), sizeof(float) * af.size(), cudaMemcpyHostToDevice, h->stream));
-    CK(h, cudaMemcpyAsync(h->alpha_d.p, ad.data(), sizeof(double) * ad.size(), cudaMemcpyHostToDevice, h->stream));
-    CK(h, launch_lgs_table(K, h->alpha_d.p, h->lgs_alpha.p, h->stream));
+    if (upload_alpha(h, alpha)) return 1;
     if (step_alias(h)) return 1;   // the sparse scheme's tables are built over alpha_k * phi_kw
     return sync_check(h);
 }
@@ -1887,19 +1759,15 @@ int ldagpu_set_alpha(ldagpu_handle h, const double *alpha)
 {
     NEED(h);
     if (!alpha) return h->fail("null alpha");
-    if (h->multi()) {
-        for (ldagpu_handle c : h->shards) MC(h, c, set_alpha_one(c, alpha));
-        return 0;
-    }
-    return set_alpha_one(h, alpha);
+    for (ldagpu_handle c : h->parts()) MC(h, c, set_alpha_one(c, alpha));
+    return 0;
 }
 
 int ldagpu_set_beta(ldagpu_handle h, double beta)
 {
     if (!h) return 1;
     if (!(beta > 0.0)) return h->fail("beta must be > 0");
-    h->beta = beta;
-    for (ldagpu_handle c : h->shards) c->beta = beta;
+    for (ldagpu_handle c : h->parts()) c->beta = beta;
     return 0;
 }
 
@@ -1918,7 +1786,7 @@ int ldagpu_get_count_histograms(ldagpu_handle h, int32_t n_doc_bins, int64_t *do
     if ((n_doc_bins > 0 && !doc_topic_hist) || (n_type_bins > 0 && !type_topic_hist)) return h->fail("null histogram");
     const size_t nd = (size_t)std::max(n_doc_bins, 0), nt = (size_t)std::max(n_type_bins, 0);
     std::vector<unsigned long long> acc(nd + nt + 1, 0ull), tmp(nd + nt + 1);
-    std::vector<ldagpu_handle> parts = h->multi() ? h->shards : std::vector<ldagpu_handle>{h};
+    const Parts parts = h->parts();
     for (ldagpu_handle c : parts) {
         DevBuf<unsigned long long> buf;
         cudaSetDevice(c->device);
@@ -1930,7 +1798,7 @@ int ldagpu_get_count_histograms(ldagpu_handle h, int32_t n_doc_bins, int64_t *do
         buf.release();
         for (size_t i = 0; i < nd + nt; ++i) acc[i] += tmp[i];
     }
-    const int64_t D_all = h->multi() ? h->dm.D : h->D_global;
+    const int64_t D_all = parts[0]->D_global;
     if (nd) {
         unsigned long long others = 0;
         for (size_t i = 1; i < nd; ++i) others += acc[i];

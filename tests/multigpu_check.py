@@ -15,6 +15,7 @@ import torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import ldagroupedgibbssampler_b200 as L  # noqa: E402
+from ldagroupedgibbssampler_b200._lib import ptr  # noqa: E402
 from oracle import oracle as O  # noqa: E402
 
 
@@ -63,6 +64,49 @@ def stress(rank, world, local, sweeps):
         print(f"stress: {sweeps} sweeps, world {world}, exchange {mode}:", checks, flush=True)
         ok = all(checks.values())
     return ok
+
+
+def accessors(rank, world, local):
+    """The accessors that gather rows or sums across the ranks -- the Phi mean under a burn-in / thin schedule, both
+    count histograms -- and set_alpha (asymmetric) / set_beta followed by sweeps, against one GPU running the whole
+    corpus in rank 0's process."""
+    K, V = 100, 900
+    off, tokens = L.synth_corpus(400, V, 70.0, seed=8)
+    cfg = L.LDAConfiguration(scheme="gpu_ggs", topics=K, alpha=0.5, beta=0.01, seed=2019, exec_time=0)
+    s = L.GpuLDASampler(cfg, device=local)
+    box = [L.GpuLDASampler.make_comm_id() if rank == 0 else None]
+    dist.broadcast_object_list(box, src=0)
+    s.addInstances(L.InstanceList.from_csr(off, tokens, V), rank=rank, world=world, comm_id=box[0])
+    runs = [s]
+    if rank == 0:
+        ref = L.GpuLDASampler(cfg, device=local)
+        ref.addInstances(L.InstanceList.from_csr(off, tokens, V))
+        runs.append(ref)
+    # the same bin counts on every rank: the histograms are summed over the ranks
+    dh = np.zeros(int(np.diff(off).max()) + 1, np.int64)
+    th = np.zeros(int(np.bincount(tokens, minlength=V).max()) + 1, np.int64)
+    out = []
+    for r in runs:
+        r._ck(r._L.ldagpu_set_phi_mean_schedule(r._h, 2, 2))
+        r.sample(4)
+        r.alpha = np.linspace(0.05, 1.5, K)
+        r._ck(r._L.ldagpu_set_alpha(r._h, ptr(r.alpha)))
+        r._ck(r._L.ldagpu_set_beta(r._h, 0.03))
+        r.sample(3)
+        r._ck(r._L.ldagpu_get_count_histograms(r._h, len(dh), ptr(dh), len(th), ptr(th)))
+        out.append(dict(mean=r.getPhiMeans(), dh=dh.copy(), th=th.copy(), phi=r.getPhi(), n_wk=r.getTypeTopicMatrix(),
+                        z=r.get_z_flat()))
+    zs = [None] * world
+    dist.all_gather_object(zs, out[0]["z"])
+    out[0]["z"] = np.concatenate(zs)
+    s.close()
+    if rank != 0:
+        return True
+    ref.close()
+    got, want = out
+    checks = {k: want[k] is not None and np.array_equal(got[k], want[k]) for k in want}
+    print("accessors, world", world, checks, flush=True)
+    return all(checks.values())
 
 
 def main():
@@ -123,6 +167,7 @@ def main():
             print(scheme, K, s.getExchangeMode(), checks, flush=True)
         ok &= all(checks.values())
         s.close()
+    ok &= accessors(rank, world, local)
     t = torch.tensor([1 if ok else 0], device="cuda")
     dist.all_reduce(t, op=dist.ReduceOp.MIN)
     dist.destroy_process_group()

@@ -20,8 +20,8 @@ from conftest import make_corpus
 
 gpu = pytest.mark.gpu
 
-GGS, PCGS, SPALIAS = 0, 1, 2
-OSCH = {"gpu_ggs": GGS, "gpu_pcgs": PCGS, "gpu_spalias": SPALIAS}
+GGS, PCGS, SPALIAS, POLYAURN = 0, 1, 2, 3
+OSCH = {"gpu_ggs": GGS, "gpu_pcgs": PCGS, "gpu_spalias": SPALIAS, "gpu_polyaurn": POLYAURN}
 
 
 def _sampler(scheme, off, tokens, V, K, alpha, beta, seed, **add):
@@ -60,10 +60,11 @@ def _mixed_lengths(seed):
     return lens
 
 
-def _check_sweeps(oracle, s, scheme, off, tokens, z0, phi0, V, K, alpha, beta, seed, n):
-    """The handle ran n whole sweeps from (z0, phi0): z, counts, Phi (and GGS theta) bit-exact, LL and LP within 1e-9."""
+def _check_sweeps(oracle, s, scheme, off, tokens, z0, phi0, V, K, alpha, beta, seed, n, first_sweep=1):
+    """The handle ran n whole sweeps from (z0, phi0), the first of them numbered first_sweep: z, counts, Phi (and GGS
+    theta) bit-exact, LL and LP within 1e-9."""
     osch = OSCH[scheme]
-    st = oracle.sweeps("contract", osch, off, tokens, z0, V, K, alpha, beta, seed, 1, n, phi0)
+    st = oracle.sweeps("contract", osch, off, tokens, z0, V, K, alpha, beta, seed, first_sweep, n, phi0)
     assert np.array_equal(s.get_z_flat(), st["z"])
     assert np.array_equal(s.getTypeTopicMatrix(), st["n_wk"])
     assert np.array_equal(s.getTopicTotals(), st["n_k"])

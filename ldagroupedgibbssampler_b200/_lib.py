@@ -7,8 +7,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# LDAGPU_LIBRARY overrides the path (kernel-tuning experiments build variants beside the default)
-SO_PATH = os.environ.get("LDAGPU_LIBRARY") or os.path.join(_HERE, "libldagpu.so")
+SO_PATH = os.path.join(_HERE, "libldagpu.so")
 
 # every entry point include/ldagpu.h declares (tests check that the library exports all of them)
 SYMBOLS = [

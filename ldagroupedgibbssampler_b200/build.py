@@ -2,6 +2,9 @@
 
     python -m ldagroupedgibbssampler_b200.build [--force] [--verbose]
 
+There is one build: the kernel configuration (warps, occupancy, register tiles, unrolling) is fixed
+in the sources at its measured values.
+
 Flags that matter:
   -gencode arch=compute_100a,code=sm_100a   B200 only, no fallback architectures
   -fmad=false                               the contract arithmetic must not be contracted into
@@ -34,12 +37,7 @@ def _newer(src: str, dst: str) -> bool:
     return (not os.path.exists(dst)) or os.path.getmtime(src) > os.path.getmtime(dst)
 
 
-def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT) -> str:
-    """defines / out: tuning variants, e.g. build(defines=["Z_MINB_DEF=3"], out=".../libldagpu_m3.so")."""
-    global OBJ
-    if defines:
-        OBJ = os.path.join(HERE, "_obj_" + "_".join(d.replace("=", "") for d in defines))
-        force = True
+def build(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(OBJ, exist_ok=True)
     hdr_paths = [os.path.normpath(os.path.join(CSRC, h)) for h in HEADERS]
     objs = []
@@ -51,8 +49,7 @@ def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT
         stale = force or _newer(sp, op) or any(_newer(h, op) for h in hdr_paths)
         if not stale:
             continue
-        cmd = ([NVCC] + ARCH + NVFLAGS + ["-D" + d for d in defines] + (["-Xptxas", "-v"] if verbose else [])
-               + ["-c", sp, "-o", op])
+        cmd = [NVCC] + ARCH + NVFLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", sp, "-o", op]
         if verbose:
             print(" ".join(cmd), flush=True)
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
@@ -64,13 +61,13 @@ def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT
         failed |= p.returncode != 0
     if failed:
         raise RuntimeError("nvcc failed")
-    if force or procs or not os.path.exists(out):
-        cmd = [NVCC] + ARCH + ["-shared", "-o", out] + objs + ["-Xcompiler", "-pthread", "-ldl"]
+    if force or procs or not os.path.exists(OUT):
+        cmd = [NVCC] + ARCH + ["-shared", "-o", OUT] + objs + ["-Xcompiler", "-pthread", "-ldl"]
         if verbose:
             print(" ".join(cmd), flush=True)
         subprocess.check_call(cmd)
     build_synth(force)
-    return out
+    return OUT
 
 
 def build_synth(force: bool = False) -> str:
@@ -82,7 +79,4 @@ def build_synth(force: bool = False) -> str:
 
 
 if __name__ == "__main__":
-    defs = [a[2:] for a in sys.argv[1:] if a.startswith("-D")]
-    outs = [a.split("=", 1)[1] for a in sys.argv[1:] if a.startswith("--out=")]
-    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv, defines=defs,
-                out=os.path.join(HERE, outs[0]) if outs else OUT))
+    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))

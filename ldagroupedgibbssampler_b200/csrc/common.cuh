@@ -39,6 +39,9 @@ struct Dims {
 // permutation of the bits of k.  Topic indicators (z), alpha and n_k stay in natural topic order; every
 // kernel that indexes a row by topic goes through these two functions.  lg == 2 is the identity
 // (K <= 128, the K > 1024 path and the sparse scheme).
+// NT of the register path for K <= MAX_REG_TILES * TILE, and lg of NT tiles (L = 4 * NT = 1 << lg)
+__host__ __device__ constexpr int reg_tiles(int K) { return K <= 128 ? 1 : K <= 256 ? 2 : K <= 512 ? 4 : 8; }
+__host__ __device__ constexpr int lg_of_tiles(int NT) { return NT == 1 ? 2 : NT == 2 ? 3 : NT == 4 ? 4 : 5; }
 __host__ __device__ __forceinline__ int tpos_lg(int lg, int k)
 {
     return (((k & ((1 << lg) - 1)) >> 2) << 7) | ((k >> lg) << 2) | (k & 3);

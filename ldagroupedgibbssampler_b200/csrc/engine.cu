@@ -548,10 +548,10 @@ int sweep_enqueue(ldagpu_handle h, SweepCall &c, Stage stage)
         CK(h, cudaEventRecord(ev[0], h->stream));
         // the count rebuild is fused into the z kernel: zero n_wk first (Phi, not n_wk, feeds the z-step)
         CK(h, cudaMemsetAsync(h->n_wk.p, 0, sizeof(int32_t) * h->n_wk.n, h->stream));
-        // LDAGPU_FUSE_THETA=0 (tuning knob): theta for all documents up front, as round 1 did
-        static const bool fuse_env = !(getenv("LDAGPU_FUSE_THETA") && atoi(getenv("LDAGPU_FUSE_THETA")) == 0);
-        const bool fuse_theta = h->scheme == LDAGPU_SCHEME_GGS && fuse_env;
-        if (h->scheme == LDAGPU_SCHEME_GGS && step_theta(h, fuse_theta)) return 1;
+        // GGS draws theta inside the z kernel for the documents that are one work item, and in the stand-alone
+        // kernel beforehand for the documents split into several
+        const bool fuse_theta = h->scheme == LDAGPU_SCHEME_GGS;
+        if (fuse_theta && step_theta(h, /*only_long=*/true)) return 1;
         CK(h, cudaEventRecord(ev[1], h->stream));
         const bool stream_out = (c.z_out || c.z16_out) && s == c.n - 1 && h->scheme == LDAGPU_SCHEME_GGS && h->z_parts.size() > 1;
         if (stream_out) {
@@ -998,9 +998,9 @@ int ldagpu_create(int32_t K, int32_t V, int64_t D, const int64_t *doc_offsets, c
     if (scheme != LDAGPU_SCHEME_SPALIAS && K <= MAX_REG_TILES * TILE) {
         // register path of the dense z-step: 1, 2, 4 or 8 tiles, lane l owns 4 * NT consecutive topics and the
         // rows of Phi^T / n_wk / theta are stored in the matching column order (common.cuh: tpos / ttopic)
-        dm.NT = K <= 128 ? 1 : K <= 256 ? 2 : K <= 512 ? 4 : 8;
+        dm.NT = reg_tiles(K);
         dm.Ks = dm.NT * TILE;
-        dm.lg = dm.NT == 1 ? 2 : dm.NT == 2 ? 3 : dm.NT == 4 ? 4 : 5;
+        dm.lg = lg_of_tiles(dm.NT);
     }
     dm.V = V; dm.Vp = (int32_t)round_up(V, PHI_ROW_BLOCK * PHI_SEGMENTS);
     dm.D = D; dm.N = doc_offsets[D]; dm.doc_base = doc_base; dm.token_base = token_base;

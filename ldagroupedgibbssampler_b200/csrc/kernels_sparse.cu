@@ -42,13 +42,9 @@ constexpr unsigned FULL = 0xffffffffu;
 // utilisation, 20.4 ms at K = 10 000).
 // Only the types that occur in this rank's tokens get a table (no token ever reads the others).
 // ---------------------------------------------------------------------------------------
-#ifndef ALIAS_Q
-#define ALIAS_Q 4   // stack entries a lane of the pairing kernel holds ahead in registers (measured 2, 4, 8: 9.5, 9.05, 9.3 ms)
-#endif
-#ifndef ALIAS_TPS
-#define ALIAS_TPS 1024   // scratch slots per SM: one round covers 151 552 types
-#endif
-constexpr int ALIAS_CW = 8;   // warps per CTA of the classify kernel
+constexpr int ALIAS_Q = 4;      // stack entries a lane of the pairing kernel holds ahead in registers (measured 2, 4, 8: 9.5, 9.05, 9.3 ms)
+constexpr int ALIAS_TPS = 1024; // scratch slots per SM: one round covers 151 552 types
+constexpr int ALIAS_CW = 8;     // warps per CTA of the classify kernel
 
 __global__ void __launch_bounds__(ALIAS_CW * 32)
 alias_classify_kernel(Dims dm, const float *__restrict__ alpha, const float *__restrict__ phiT,

@@ -28,22 +28,12 @@
 namespace ldagpu {
 
 constexpr unsigned FULL = 0xffffffffu;
-#ifndef Z_MINB_DEF
-#define Z_MINB_DEF 3
-#endif
-#ifndef Z_WARPS_GGS8
-#define Z_WARPS_GGS8 8
-#endif
-#ifndef Z_TH_REG
-#define Z_TH_REG 3   // theta tiles of the 8-tile GGS kernel kept in registers (the rest in shared memory; measured 1..8, profiles/README.md)
-#endif
 // warps per CTA / CTAs per SM.  GGS at 1024 topics keeps theta (32 registers) and the prefixes (32) live;
 // 24 warps per SM leave 80 registers per thread (profiles/README.md, round 2)
-template <int NT, bool PCGS> __host__ __device__ constexpr int z_warps() { return (NT == 8 && !PCGS) ? Z_WARPS_GGS8 : 8; }
-template <int NT, bool PCGS> __host__ __device__ constexpr int z_minb() { return NT == 8 ? (PCGS ? 2 : Z_MINB_DEF) : 4; }
+constexpr int Z_WARPS = 8;
+template <int NT, bool PCGS> __host__ __device__ constexpr int z_minb() { return NT == 8 ? (PCGS ? 2 : 3) : 4; }
 
-template <int NT> __host__ __device__ constexpr int lg_of() { return NT == 1 ? 2 : NT == 2 ? 3 : NT == 4 ? 4 : 5; }
-template <int NT> __device__ __forceinline__ int pos_of(int k) { return tpos_lg(lg_of<NT>(), k); }
+template <int NT> __device__ __forceinline__ int pos_of(int k) { return tpos_lg(lg_of_tiles(NT), k); }
 
 template <int NT> struct RowScan {
     float p[NT][4];   // lane-local inclusive prefix over the lane's 4*NT consecutive topics (p[NT-1][3] = lane total)
@@ -157,7 +147,7 @@ template <int NT>
 __device__ __forceinline__ void theta_tables_fill(float *d0, float *c0, float *i0, const float *__restrict__ alpha, int K)
 {
     for (int p = threadIdx.x; p < NT * TILE; p += blockDim.x) {
-        const int k = ttopic_lg(lg_of<NT>(), p);
+        const int k = ttopic_lg(lg_of_tiles(NT), p);
         bool b; float dd, cc, ii;
         gamma_setup<float>(k < K ? alpha[k] : 1.0f, b, dd, cc, ii);
         d0[p] = dd; c0[p] = cc; i0[p] = ii;
@@ -170,7 +160,7 @@ __device__ __forceinline__ void theta_draw_doc(int *cg, unsigned short *plist, c
                                                int64_t t0, int64_t t1, int K, unsigned long long cell0,
                                                uint32_t sweep, const PhiloxKeys &rk, int lane)
 {
-    constexpr int LG = lg_of<NT>();
+    constexpr int LG = lg_of_tiles(NT);
     const unsigned lt_mask = (1u << lane) - 1u;
     for (int64_t t = t0 + lane; t < t1; t += 32) atomicAdd(&cg[pos_of<NT>(z[t])], 1);
     __syncwarp();
@@ -294,8 +284,9 @@ __device__ __forceinline__ void theta_draw_doc(int *cg, unsigned short *plist, c
     __syncwarp();
 }
 
+// theta tiles kept in registers: 3 in the 8-tile GGS kernel (the rest in shared memory; measured 1..8, profiles/README.md)
+template <int NT, bool PCGS> __host__ __device__ constexpr int z_th_reg() { return (NT == 8 && !PCGS) ? 3 : NT; }
 // shared-memory footprint, in bytes
-template <int NT, bool PCGS> __host__ __device__ constexpr int z_th_reg() { return (NT == 8 && !PCGS) ? Z_TH_REG : NT; }
 template <int NT, bool PCGS> __host__ __device__ constexpr size_t z_warp_smem()
 {
     // GGS: row slot + one auxiliary area that is the pending list during the theta draw and the home of the theta tiles
@@ -306,17 +297,16 @@ template <int NT, bool PCGS> __host__ __device__ constexpr size_t z_warp_smem()
 }
 template <int NT, bool PCGS> __host__ __device__ constexpr size_t z_cta_smem()
 {
-    return z_warps<NT, PCGS>() * z_warp_smem<NT, PCGS>() + (PCGS ? 1 : 3) * (size_t)NT * TILE * 4 +
-           (size_t)z_warps<NT, PCGS>() * 8;
+    return Z_WARPS * z_warp_smem<NT, PCGS>() + (PCGS ? 1 : 3) * (size_t)NT * TILE * 4 +
+           (size_t)Z_WARPS * 8;
 }
 
 template <int NT, bool PCGS>
-__global__ void __launch_bounds__(z_warps<NT, PCGS>() * 32, z_minb<NT, PCGS>()) z_kernel(ZArgs a)
+__global__ void __launch_bounds__(Z_WARPS * 32, z_minb<NT, PCGS>()) z_kernel(ZArgs a)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     constexpr int ROWF = NT * TILE;
-    constexpr int Z_WARPS = z_warps<NT, PCGS>();
     unsigned char *wbase = smem_raw + (size_t)warp * z_warp_smem<NT, PCGS>();
     float *const slot = reinterpret_cast<float *>(wbase);           // the warp's Phi^T row slot (GGS: also the theta scratch)
     int *cnt = reinterpret_cast<int *>(wbase + (size_t)ROWF * 4);   // PCGS: n_dk by column
@@ -336,7 +326,7 @@ __global__ void __launch_bounds__(z_warps<NT, PCGS>() * 32, z_minb<NT, PCGS>()) 
     if (PCGS) {
         for (int i = lane; i < ROWF / 4; i += 32) reinterpret_cast<int4 *>(cnt)[i] = make_int4(0, 0, 0, 0);
         for (int p = threadIdx.x; p < ROWF; p += blockDim.x) {
-            const int k = ttopic_lg(lg_of<NT>(), p);
+            const int k = ttopic_lg(lg_of_tiles(NT), p);
             alpha_s[p] = k < K ? a.alpha[k] : 0.0f;
         }
     } else if (a.fuse_theta) {
@@ -466,9 +456,7 @@ __global__ void __launch_bounds__(z_warps<NT, PCGS>() * 32, z_minb<NT, PCGS>()) 
                 if (!PCGS) scan_scores<NT, TH_REG>(th, th_sm, ph, rs, lane);
                 // not unrolled: runs average 1.4 tokens here; the compiler's 4x unrolled loop with its remainder
                 // handling cost 3.7 % of the z-step (11.29 -> 10.88 ms on the 400 000-document slice)
-#ifndef Z_TOKEN_UNROLL
 #pragma unroll 1
-#endif
                 for (int tt = b; tt < e; ++tt) {
                     if (PCGS) {
                         // remove the token from the document counts (UncollapsedParallelLDA.java:1494);
@@ -521,7 +509,6 @@ template <int NT, bool PCGS>
 static cudaError_t launch_z_t(const ZArgs &a, int sm_count, cudaStream_t st)
 {
     constexpr size_t smem = z_cta_smem<NT, PCGS>();
-    constexpr int Z_WARPS = z_warps<NT, PCGS>();
     int ctas_per_sm = 1;
     cudaError_t e = kernel_config(reinterpret_cast<const void *>(z_kernel<NT, PCGS>), Z_WARPS * 32, smem, &ctas_per_sm);
     if (e != cudaSuccess) return e;
@@ -536,12 +523,14 @@ static cudaError_t launch_z_t(const ZArgs &a, int sm_count, cudaStream_t st)
 template <bool PCGS> static cudaError_t launch_z_any(const ZArgs &a, int sm_count, cudaStream_t st)
 {
     if (a.n_items == 0) return cudaSuccess;
-    switch (a.dm.NT) {   // the engine sets NT to 1, 2, 4 or 8 for K <= 1024 (row layout, common.cuh)
-    case 1: return launch_z_t<1, PCGS>(a, sm_count, st);
-    case 2: return launch_z_t<2, PCGS>(a, sm_count, st);
-    case 4: return launch_z_t<4, PCGS>(a, sm_count, st);
-    case 8: if (a.dm.K <= 1024) return launch_z_t<8, PCGS>(a, sm_count, st);
-    default: break;
+    if (a.dm.K <= MAX_REG_TILES * TILE) {
+        switch (a.dm.NT) {   // reg_tiles(K) (row layout, common.cuh)
+        case 1: return launch_z_t<1, PCGS>(a, sm_count, st);
+        case 2: return launch_z_t<2, PCGS>(a, sm_count, st);
+        case 4: return launch_z_t<4, PCGS>(a, sm_count, st);
+        case 8: return launch_z_t<8, PCGS>(a, sm_count, st);
+        default: break;
+        }
     }
     return PCGS ? launch_z_pcgs_big(a, sm_count, st) : launch_z_ggs_big(a, sm_count, st);
 }
@@ -612,8 +601,8 @@ cudaError_t launch_theta(const ThetaArgs &a, int sm_count, cudaStream_t st)
     if (a.n_docs <= 0) return cudaSuccess;
     // theta_kernel<NT> writes rows in the register path's layout (Ks = 128 * NT, permuted columns); the sparse scheme
     // keeps its rows in natural topic order with Ks = round_up(K, 32) and takes the general kernel at every K
-    const int NT = a.dm.NT, lg = NT == 1 ? 2 : NT == 2 ? 3 : NT == 4 ? 4 : 5;
-    if (a.dm.K <= 1024 && a.dm.Ks == NT * TILE && a.dm.lg == lg) {
+    const int NT = a.dm.NT;
+    if (a.dm.K <= MAX_REG_TILES * TILE && a.dm.Ks == NT * TILE && a.dm.lg == lg_of_tiles(NT)) {
         switch (NT) {
         case 1: return launch_theta_t<1>(a, sm_count, st);
         case 2: return launch_theta_t<2>(a, sm_count, st);

@@ -290,15 +290,15 @@ __global__ void __launch_bounds__(256) theta_kernel_big(ThetaArgs a)
             if (k < K) {
                 gv = c_gamma<float>(__fadd_rn(__int2float_rn(cg[k]), a.alpha[k]), a.seed_lo, a.seed_hi,
                                     cell0 + (unsigned long long)k, a.sweep, STREAM_THETA);
-                if (K > 1024) acc = __fadd_rn(acc, gv);
+                if (K > MAX_REG_TILES * TILE) acc = __fadd_rn(acc, gv);
             }
             cg[k] = __float_as_int(gv);
         }
         __syncwarp();
-        if (K <= 1024) {
+        if (K <= MAX_REG_TILES * TILE) {
             // the sparse scheme's rows at K <= 1024: the contract sums over the lane's L consecutive topics, L = 4 x the
             // register path's tile count (DESIGN.md 4.3), whatever the row layout
-            const int L = K <= 128 ? 4 : K <= 256 ? 8 : K <= 512 ? 16 : 32;
+            const int L = 4 * reg_tiles(K);
             for (int m = 0; m < L; ++m) {
                 const int k = lane * L + m;
                 if (k < K) acc = __fadd_rn(acc, __int_as_float(cg[k]));

@@ -162,6 +162,24 @@ int ldagpu_log_likelihood(ldagpu_handle h, double *ll);
 /* computeLogPosterior (UPL:1573-1634); GGS uses the sweep's theta (UPL:716-720) */
 int ldagpu_log_posterior(ldagpu_handle h, double *lp);
 
+/*
+ * Held-out evaluation (UPL:604-611,840-844: MarginalProbEstimatorPlain.evaluateLeftToRight, MALLET's left-to-right
+ * estimator without resampling; DESIGN.md 4.8).  K <= 1024 only: a larger K fails with an error naming the limit.
+ * addTestInstances (LGS): upload a test set in CSR form, as for ldagpu_create, with the global index of its first
+ * document / token (doc_base, token_base; 0 unless the caller shards the test set over ranks itself).  The documents stay
+ * resident; a second call replaces them, D_test = 0 removes them.  A type outside [0, V) or malformed offsets fail the
+ * call and leave the previous test set in place.  A create_multi handle takes the whole test set and shards it by
+ * tokens over its GPUs; with one process per GPU every rank passes its own shard.
+ */
+int ldagpu_set_test_documents(ldagpu_handle h, int64_t D_test, const int64_t *doc_offsets, const int32_t *tokens,
+                              int64_t doc_base, int64_t token_base);
+/* getHeldOutLogLikelihood (UPL:604-611,840-844), evaluateLeftToRight: the model is phi_kw = (n_wk + beta) /
+ * (n_k + V beta) from the current counts and alpha; n_particles (R, MALLET's default 10) particles per document.
+ * doc_ll (NULL or double[D_test] of this handle's test documents) receives ln p(w_d), *total the sum over the whole
+ * test set (every rank returns the same total).  Reads the counts only: z, counts, Phi, theta, the iteration and the
+ * training random streams are untouched, and two calls at the same iteration return the same values. */
+int ldagpu_heldout_log_likelihood(ldagpu_handle h, int32_t n_particles, double *doc_ll, double *total);
+
 /* Hooks for the hyper-parameter optimisation (MSL:812-905, called every hyperparam_optim_interval sweeps, UPL:891-894;
  * off by default).  MALLET's fixed-point iteration (Dirichlet.learnParameters / learnSymmetricConcentration) stays on the
  * host; the library supplies the histograms it consumes -- doc_topic_hist[c] = number of (document, topic) pairs with

@@ -71,6 +71,10 @@ public class GpuLDASampler extends ModifiedSimpleLDA implements LDAGibbsSampler,
             ADDRESS, JAVA_INT, ADDRESS, JAVA_INT, ADDRESS));
     private static final MethodHandle SET_ALPHA = fn("ldagpu_set_alpha", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
     private static final MethodHandle SET_BETA = fn("ldagpu_set_beta", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_DOUBLE));
+    private static final MethodHandle SET_TEST_DOCS = fn("ldagpu_set_test_documents", FunctionDescriptor.of(JAVA_INT,
+            ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG));
+    private static final MethodHandle HELDOUT_LL = fn("ldagpu_heldout_log_likelihood", FunctionDescriptor.of(JAVA_INT,
+            ADDRESS, JAVA_INT, ADDRESS, ADDRESS));
 
     private final Arena arena = Arena.ofShared();
     private MemorySegment handle = MemorySegment.NULL;
@@ -360,6 +364,34 @@ public class GpuLDASampler extends ModifiedSimpleLDA implements LDAGibbsSampler,
             for (int k = 0; k < numTopics; k++) MemorySegment.copy(m, JAVA_DOUBLE, (long) k * numTypes * 8, out[k], 0, numTypes);
         } catch (RuntimeException e) { throw e; } catch (Throwable t) { throw new IllegalStateException(t); }
         return out;
+    }
+
+    /** LDAGibbsSampler.addTestInstances: the test set (type ids of the training alphabet) goes to the library once and
+     *  stays resident; the library shards it over the GPUs of this handle.  K <= 1024 only. */
+    @Override
+    public void addTestInstances(InstanceList testSet) {
+        int D = testSet.size();
+        long[] off = new long[D + 1];
+        for (int d = 0; d < D; d++) off[d + 1] = off[d] + ((FeatureSequence) testSet.get(d).getData()).getLength();
+        int[] tokens = new int[(int) off[D]];
+        for (int d = 0; d < D; d++) {
+            FeatureSequence fs = (FeatureSequence) testSet.get(d).getData();
+            System.arraycopy(fs.getFeatures(), 0, tokens, (int) off[d], fs.getLength());
+        }
+        try (Arena a = Arena.ofConfined()) {
+            ck((int) SET_TEST_DOCS.invokeExact(handle, (long) D, a.allocateFrom(JAVA_LONG, off),
+                    a.allocateFrom(JAVA_INT, tokens), 0L, 0L));
+        } catch (RuntimeException e) { throw e; } catch (Throwable t) { throw new IllegalStateException(t); }
+    }
+
+    /** MarginalProbEstimatorPlain.evaluateLeftToRight (UPL:604-611,840-844): MALLET's left-to-right estimator without
+     *  resampling on the current counts, nParticles particles (MALLET's default 10) */
+    public double heldOutLogLikelihood(int nParticles) {
+        try (Arena a = Arena.ofConfined()) {
+            MemorySegment v = a.allocate(JAVA_DOUBLE);
+            ck((int) HELDOUT_LL.invokeExact(handle, nParticles, MemorySegment.NULL, v));
+            return v.get(JAVA_DOUBLE, 0);
+        } catch (RuntimeException e) { throw e; } catch (Throwable t) { throw new IllegalStateException(t); }
     }
 
     @Override

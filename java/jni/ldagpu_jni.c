@@ -30,6 +30,8 @@
  *       static native void   getCountHistograms(long h, long[] docTopicHist, long[] typeTopicHist);   // either may be empty
  *       static native void   setAlpha(long h, double[] alpha);           // optimizeAlpha / optimizeBeta (MSL:812-905)
  *       static native void   setBeta(long h, double beta);
+ *       static native void   setTestDocuments(long h, long[] docOffsets, int[] tokens);   // addTestInstances
+ *       static native double heldOutLogLikelihood(long h, int nParticles);            // evaluateLeftToRight
  *   }
  * Every failure is rethrown as IllegalStateException with ldagpu_last_error's message, which is what the
  * reference's own samplers throw on an invariant break (UncollapsedParallelLDA.java:475-481,1828-1830).
@@ -191,4 +193,25 @@ JNIEXPORT void JNICALL CLS(setBeta)(JNIEnv *env, jclass c, jlong h, jdouble beta
 {
     (void)c;
     if (ldagpu_set_beta((ldagpu_handle)(intptr_t)h, beta)) throw_last(env, (ldagpu_handle)(intptr_t)h);
+}
+
+JNIEXPORT void JNICALL CLS(setTestDocuments)(JNIEnv *env, jclass c, jlong h, jlongArray docOffsets, jintArray tokens)
+{
+    (void)c;
+    const jsize D = (*env)->GetArrayLength(env, docOffsets) - 1;
+    jlong *off = (*env)->GetLongArrayElements(env, docOffsets, NULL);
+    jint *tok = (*env)->GetIntArrayElements(env, tokens, NULL);
+    const int rc = ldagpu_set_test_documents((ldagpu_handle)(intptr_t)h, D > 0 ? D : 0, (const int64_t *)off,
+                                             (const int32_t *)tok, 0, 0);
+    (*env)->ReleaseLongArrayElements(env, docOffsets, off, JNI_ABORT);
+    (*env)->ReleaseIntArrayElements(env, tokens, tok, JNI_ABORT);
+    if (rc) throw_last(env, (ldagpu_handle)(intptr_t)h);
+}
+
+JNIEXPORT jdouble JNICALL CLS(heldOutLogLikelihood)(JNIEnv *env, jclass c, jlong h, jint nParticles)
+{
+    (void)c;
+    double v = 0.0;
+    if (ldagpu_heldout_log_likelihood((ldagpu_handle)(intptr_t)h, nParticles, NULL, &v)) throw_last(env, (ldagpu_handle)(intptr_t)h);
+    return v;
 }

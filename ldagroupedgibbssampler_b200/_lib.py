@@ -21,6 +21,7 @@ SYMBOLS = [
     "ldagpu_log_likelihood", "ldagpu_log_posterior", "ldagpu_abort", "ldagpu_get_abort",
     "ldagpu_get_timers", "ldagpu_get_last_call_stats",
     "ldagpu_set_z16", "ldagpu_get_z16", "ldagpu_sweep_get_z16", "ldagpu_create_multi", "ldagpu_get_shards", "ldagpu_set_phi_sampler", "ldagpu_get_count_histograms", "ldagpu_set_alpha", "ldagpu_set_beta",
+    "ldagpu_set_test_documents", "ldagpu_heldout_log_likelihood",
 ]
 
 
@@ -81,6 +82,8 @@ def load() -> C.CDLL:
     sig("ldagpu_get_count_histograms", C.c_int, vp, i32, vp, i32, vp)
     sig("ldagpu_set_alpha", C.c_int, vp, vp)
     sig("ldagpu_set_beta", C.c_int, vp, f64)
+    sig("ldagpu_set_test_documents", C.c_int, vp, i64, vp, vp, i64, i64)
+    sig("ldagpu_heldout_log_likelihood", C.c_int, vp, i32, vp, pf64)
     sig("ldagpu_get_phi_mean", C.c_int, vp, vp, pi32)
     sig("ldagpu_log_likelihood", C.c_int, vp, pf64)
     sig("ldagpu_log_posterior", C.c_int, vp, pf64)

@@ -22,10 +22,11 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "_obj")
 OUT = os.path.join(HERE, "libldagpu.so")
 
-CU = ["kernels_z.cu", "kernels_z_big.cu", "kernels_sparse.cu", "kernels_phi.cu", "kernels_p2p.cu", "kernels_misc.cu", "engine.cu"]
+CU = ["kernels_z.cu", "kernels_z_big.cu", "kernels_sparse.cu", "kernels_phi.cu", "kernels_p2p.cu", "kernels_misc.cu", "kernels_heldout.cu",
+      "engine.cu"]
 CPP = []
 SYNTH_SRC, SYNTH_OUT = os.path.join(CSRC, "synth.cpp"), os.path.join(HERE, "libldasynth.so")
-HEADERS = ["common.cuh", "contract_math.cuh", os.path.join("..", "..", "include", "ldagpu.h")]
+HEADERS = ["common.cuh", "contract_math.cuh", "warp_draw.cuh", os.path.join("..", "..", "include", "ldagpu.h")]
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]

@@ -198,7 +198,7 @@ def tfidf_ranking(tf: dict, df: dict, n_docs: int, n_types: int) -> List[int]:
 
 def load_dataset(path: str, stoplist=None, keep_numbers: bool = True, alphabet: Optional[Alphabet] = None,
                  rare_threshold: int = 0, keep_connectors: bool = False, tfidf_vocab_size: int = -1,
-                 max_token_buffer: int = 10000) -> InstanceList:
+                 max_token_buffer: int = 10000, frozen_alphabet: bool = False) -> InstanceList:
     """``LDAUtils.loadDataset`` for a ``name<TAB>label<TAB>text`` file (util/LDAUtils.java:136-182):
 
     * ``tfidf_vocab_size > 0``: ``loadInstancesKeep`` (util/LDAUtils.java:353-460) -- a first pass counts, per
@@ -213,8 +213,23 @@ def load_dataset(path: str, stoplist=None, keep_numbers: bool = True, alphabet: 
       (StringList2FeatureSequence).  With a caller-supplied ``alphabet`` both passes share it, as in the
       reference, so pruned words keep their ids.
 
-    Ties of the TF-IDF ranking follow MALLET's IDSorter (higher id first; restated from memory of 2.0.8)."""
+    Ties of the TF-IDF ranking follow MALLET's IDSorter (higher id first; restated from memory of 2.0.8).
+
+    ``frozen_alphabet`` (a test set read with the training alphabet): the alphabet does not grow, words it does not
+    hold are dropped as MALLET's pipes drop them once the alphabet is frozen, and the pruning passes are skipped (they
+    are the training set's)."""
     stop = _read_stoplist(stoplist)
+    if frozen_alphabet:
+        if alphabet is None:
+            raise ValueError("frozen_alphabet needs the training alphabet")
+        il = InstanceList(alphabet=alphabet)
+        for name, label, text in _read_lines(path):
+            ids = [i for i in (alphabet.lookupIndex(tok, add=False)
+                               for tok in tokenize(text, stop, keep_numbers, keep_connectors, max_token_buffer)) if i >= 0]
+            il.docs.append(np.asarray(ids, np.int32))
+            il.names.append(name)
+            il.labels.append(label)
+        return il
     if tfidf_vocab_size > 0 or rare_threshold > 0:
         first = alphabet if alphabet is not None else Alphabet()
         tf, df, n_docs = corpus_statistics(path, stop, keep_numbers, keep_connectors, first, max_token_buffer)

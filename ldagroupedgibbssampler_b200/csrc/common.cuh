@@ -85,6 +85,24 @@ struct ThetaArgs {
     PhiloxKeys rk;
 };
 
+// held-out left-to-right estimator (kernels_heldout.cu), one batch of documents [doc0, doc1) of the local test set
+struct HeldoutArgs {
+    Dims dm;                  // of phihat: K <= 1024, the register path's NT / Ks / lg, V, Vp
+    const int64_t *doc_off;   // [D_test + 1] local test CSR
+    const int32_t *tokens;    // [N_test]
+    const float *phihat;      // [Vp][Ks]
+    const float *alpha;       // [>= K], natural topic order
+    int64_t doc0, doc1;       // the batch
+    int64_t tok0;             // doc_off[doc0]: token t of the batch is column t - tok0 of S
+    int64_t batch_tokens;     // doc_off[doc1] - tok0
+    int32_t R;                // particles
+    float *S;                 // [R][batch_tokens] score totals S_i^r
+    int64_t token_base;       // global index of local test token 0 (Philox counter)
+    uint32_t iteration;
+    PhiloxKeys rk;
+    unsigned long long *work_counter;
+};
+
 // ---------------------------------------------------------------------------------------
 // Peer-memory exchange (kernels_p2p.cu, kernels_phi.cu): one process per GPU; every rank maps the
 // other ranks' buffers with CUDA IPC, and the count exchange / Phi broadcast of a sweep are loads
@@ -216,6 +234,12 @@ cudaError_t launch_lp_theta(const Dims &dm, const int64_t *doc_off, const int32_
                             int n_partials, int sm_count, cudaStream_t st);
 cudaError_t launch_lp_phi(const Dims &dm, const float *phiT, double beta, int32_t row0, int32_t row1,
                           double *partials, int n_partials, cudaStream_t st);
+// held-out log-likelihood (kernels_heldout.cu): phihat in dst's layout from n_wk in src's layout and n_k; the
+// particles' score totals of one batch; the per-document values of that batch into doc_ll[0, doc1 - doc0)
+cudaError_t launch_heldout_phihat(const Dims &src, const Dims &dst, const int32_t *n_wk, const int32_t *n_k, double beta,
+                                  float *phihat, int sm_count, cudaStream_t st);
+cudaError_t launch_heldout_l2r(const HeldoutArgs &a, int sm_count, cudaStream_t st);
+cudaError_t launch_heldout_reduce(const HeldoutArgs &a, double alpha_sum, double *doc_ll, int sm_count, cudaStream_t st);
 // out[j] = sum_i partials[i*stride + j], sequential in i
 cudaError_t launch_sum_partials(const double *partials, int n, int stride, double *out, cudaStream_t st);
 

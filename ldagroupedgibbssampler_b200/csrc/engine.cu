@@ -118,6 +118,9 @@ struct JavaRandom {
 
 constexpr int N_PARTIALS = 592;   // 4 CTAs per SM on a 148-SM part; fixed so sums are reproducible
 constexpr int EV_PER_SWEEP = 9;
+// bound of the held-out score buffer S[R][batch tokens]: a test set whose R * N_test floats do not fit is evaluated in
+// document batches (a single document longer than the bound gets a batch, and a buffer, of its own)
+constexpr int64_t HELDOUT_SCRATCH_BYTES = 1ll << 30;
 
 }  // namespace
 
@@ -151,6 +154,15 @@ struct ldagpu_handle_s {
     int64_t n_items = 0;
     int32_t ggs_chunk = GGS_CHUNK_MAX;
     std::vector<int64_t> h_doc_off;
+
+    // held-out test set (ldagpu_set_test_documents): local CSR on the device and on the host, and the global index of
+    // its first document / token.  A group keeps the shard bounds of its test set in test_doc0 / test_tok0.
+    DevBuf<int64_t> test_doc_off;
+    DevBuf<int32_t> test_tokens;
+    std::vector<int64_t> h_test_doc_off{0}, test_doc0{0, 0}, test_tok0{0, 0};
+    int64_t test_doc_base = 0, test_token_base = 0;
+    DevBuf<float> phihat, ho_scores;   // during an evaluation: phihat [Vp][Ks of the register path], S [R][batch tokens]
+    DevBuf<double> ho_ll;               // during an evaluation: [D_test] per-document values
 
     int32_t mean_burn_in = 0, mean_thin = 1, n_sampled_phi = 0;
     int32_t poisson_L = 0;   // > 0: Phi rows are drawn by the Poisson Polya urn (ldagpu_set_phi_sampler)
@@ -1108,6 +1120,7 @@ int ldagpu_destroy(ldagpu_handle h)
     h->counter.release(); h->bad.release();
     h->alias_table.release(); h->type_norm.release(); h->alias_stack.release(); h->alias_bs.release();
     h->active_types.release(); h->sparse_lists.release();
+    h->test_doc_off.release(); h->test_tokens.release(); h->phihat.release(); h->ho_scores.release(); h->ho_ll.release();
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
     return 0;
@@ -1811,6 +1824,227 @@ int ldagpu_get_count_histograms(ldagpu_handle h, int32_t n_doc_bins, int64_t *do
         acc[nd] = (unsigned long long)h->dm.V * (unsigned long long)h->dm.K - others;   // cells with n_wk = 0
         for (size_t i = 0; i < nt; ++i) type_topic_hist[i] = (int64_t)acc[nd + i];
     }
+    return 0;
+}
+
+// ---- held-out evaluation (MarginalProbEstimatorPlain.evaluateLeftToRight, UPL:604-611,840-844; kernels_heldout.cu)
+// documents [0, D) with offsets `off` sharded by token count into `parts` contiguous ranges (the rule of create_multi)
+static std::vector<int64_t> shard_bounds_by_tokens(const int64_t *off, int64_t D, int parts)
+{
+    std::vector<int64_t> d0((size_t)parts + 1, D);
+    d0[0] = 0;
+    const int64_t N = off[D];
+    for (int g = 1; g < parts; ++g) {
+        const int64_t target = N / parts * g;
+        int64_t d = std::lower_bound(off, off + D + 1, target) - off;
+        d0[(size_t)g] = std::min<int64_t>(std::max<int64_t>(d, d0[(size_t)g - 1]), D);
+    }
+    return d0;
+}
+
+// replace this part's test set by documents [0, D) (offsets from 0); the old one is released only once the new one is on
+// the device
+static int set_test_one(ldagpu_handle c, int64_t D, const int64_t *off, const int32_t *tok, int64_t doc_base, int64_t token_base)
+{
+    DevBuf<int64_t> o;
+    DevBuf<int32_t> t;
+    auto upload = [&]() -> int {
+        if (D == 0) return 0;
+        const int64_t N = off[D];
+        CK(c, o.alloc((size_t)D + 1));
+        CK(c, t.alloc((size_t)std::max<int64_t>(N, 1)));
+        CK(c, cudaMemcpy(o.p, off, sizeof(int64_t) * ((size_t)D + 1), cudaMemcpyHostToDevice));
+        if (N) CK(c, cudaMemcpy(t.p, tok, sizeof(int32_t) * (size_t)N, cudaMemcpyHostToDevice));
+        return 0;
+    };
+    if (upload()) { o.release(); t.release(); return 1; }
+    std::swap(c->test_doc_off, o);
+    std::swap(c->test_tokens, t);
+    o.release();
+    t.release();
+    c->h_test_doc_off.assign(off, off + D + 1);
+    c->test_doc_base = doc_base;
+    c->test_token_base = token_base;
+    return 0;
+}
+
+int ldagpu_set_test_documents(ldagpu_handle h, int64_t D_test, const int64_t *doc_offsets, const int32_t *tokens,
+                              int64_t doc_base, int64_t token_base)
+{
+    NEED(h);
+    const int32_t K = h->dm.K, V = h->dm.V;
+    if (K > MAX_REG_TILES * TILE)
+        return h->fail("held-out evaluation is limited to K <= %d topics (the dense left-to-right estimator); K = %d",
+                       MAX_REG_TILES * TILE, K);
+    if (D_test < 0 || doc_base < 0 || token_base < 0) return h->fail("D_test, doc_base and token_base must be >= 0");
+    static const int64_t zero = 0;
+    if (D_test == 0) doc_offsets = &zero;   // removes the test set
+    if (!doc_offsets) return h->fail("null doc_offsets");
+    if (doc_offsets[0] != 0) return h->fail("test doc_offsets[0] must be 0");
+    for (int64_t d = 0; d < D_test; ++d)
+        if (doc_offsets[d + 1] < doc_offsets[d]) return h->fail("test doc_offsets must be non-decreasing");
+    const int64_t N = doc_offsets[D_test];
+    if (N > 0 && !tokens) return h->fail("null tokens");
+    for (int64_t i = 0; i < N; ++i)
+        if (tokens[i] < 0 || tokens[i] >= V)
+            return h->fail("test token %lld: type id %d out of range [0, %d)", (long long)i, tokens[i], V);
+    const Parts parts = h->parts();
+    const std::vector<int64_t> d0 = shard_bounds_by_tokens(doc_offsets, D_test, (int)parts.size());
+    std::vector<int64_t> t0(d0.size());
+    for (size_t g = 0; g < d0.size(); ++g) t0[g] = doc_offsets[d0[g]];
+    for (size_t g = 0; g < parts.size(); ++g) {
+        ldagpu_handle c = parts[g];
+        std::vector<int64_t> loc((size_t)(d0[g + 1] - d0[g]) + 1);
+        for (int64_t d = d0[g]; d <= d0[g + 1]; ++d) loc[(size_t)(d - d0[g])] = doc_offsets[d] - t0[g];
+        MC(h, c, set_test_one(c, d0[g + 1] - d0[g], loc.data(), tokens ? tokens + t0[g] : nullptr, doc_base + d0[g],
+                              token_base + t0[g]));
+    }
+    h->test_doc0 = d0;
+    h->test_tok0 = t0;
+    h->test_doc_base = doc_base;
+    h->test_token_base = token_base;
+    return 0;
+}
+
+// enqueue this part's evaluation with particles R and phihat (layout hd) in c->phihat: document batches whose S fits
+// HELDOUT_SCRATCH_BYTES, each one the sampling kernel and then the per-document reduction into c->ho_ll
+static int heldout_enqueue(ldagpu_handle c, const Dims &hd, int32_t R)
+{
+    const std::vector<int64_t> &off = c->h_test_doc_off;
+    const int64_t D = (int64_t)off.size() - 1;
+    if (D == 0) return 0;
+    const int64_t cap = std::max<int64_t>(1, HELDOUT_SCRATCH_BYTES / ((int64_t)sizeof(float) * R));
+    std::vector<int64_t> b{0};
+    while (b.back() < D) {
+        int64_t d = b.back() + 1;   // at least one document per batch
+        while (d < D && off[d + 1] - off[b.back()] <= cap) ++d;
+        b.push_back(d);
+    }
+    int64_t most = 0;
+    for (size_t i = 0; i + 1 < b.size(); ++i) most = std::max(most, off[b[i + 1]] - off[b[i]]);
+    CK(c, c->ho_scores.alloc((size_t)std::max<int64_t>(most, 1) * (size_t)R));
+    CK(c, c->ho_ll.alloc((size_t)D));
+    HeldoutArgs a{};
+    a.dm = hd;
+    a.doc_off = c->test_doc_off.p;
+    a.tokens = c->test_tokens.p;
+    a.phihat = c->phihat.p;
+    a.alpha = c->alpha_f.p;
+    a.R = R;
+    a.S = c->ho_scores.p;
+    a.token_base = c->test_token_base;
+    a.iteration = (uint32_t)c->iteration;
+    a.rk = philox_keys((uint32_t)c->seed, (uint32_t)(c->seed >> 32));
+    a.work_counter = c->counter.p;
+    for (size_t i = 0; i + 1 < b.size(); ++i) {
+        a.doc0 = b[i];
+        a.doc1 = b[i + 1];
+        a.tok0 = off[b[i]];
+        a.batch_tokens = off[b[i + 1]] - off[b[i]];
+        CK(c, cudaMemsetAsync(c->counter.p, 0, sizeof(unsigned long long), c->stream));
+        CK(c, launch_heldout_l2r(a, c->sm_count, c->stream));
+        CK(c, launch_heldout_reduce(a, c->alpha_sum, c->ho_ll.p + b[i], c->sm_count, c->stream));
+    }
+    return 0;
+}
+
+static void heldout_release(const Parts &parts)
+{
+    for (ldagpu_handle c : parts) {
+        cudaSetDevice(c->device);
+        c->phihat.release(); c->ho_scores.release(); c->ho_ll.release();
+    }
+}
+
+static int heldout_run(ldagpu_handle h, const Parts &parts, int32_t R, std::vector<double> &ll)
+{
+    // the global counts on parts[0] (a rank: on every rank), phihat from them, copied to the other shards of a group
+    if (gather_rows(h, parts, &ldagpu_handle_s::n_wk, ncclInt32)) return 1;
+    ldagpu_handle c0 = parts[0];
+    Dims hd = c0->dm;
+    hd.NT = reg_tiles(hd.K);
+    hd.Ks = hd.NT * TILE;
+    hd.lg = lg_of_tiles(hd.NT);
+    const size_t cells = (size_t)hd.Vp * hd.Ks;
+    for (ldagpu_handle c : parts) {
+        CK(h, cudaSetDevice(c->device));
+        MC(h, c, [&]() { CK(c, c->phihat.alloc(cells)); return 0; }());
+    }
+    CK(h, cudaSetDevice(c0->device));
+    MC(h, c0, [&]() {
+        CK(c0, launch_heldout_phihat(c0->dm, hd, c0->n_wk.p, c0->n_k.p, c0->beta, c0->phihat.p, c0->sm_count, c0->stream));
+        CK(c0, cudaStreamSynchronize(c0->stream));
+        return 0;
+    }());
+    for (size_t g = 1; g < parts.size(); ++g) {
+        ldagpu_handle c = parts[g];
+        CK(h, cudaSetDevice(c->device));
+        CK(h, cudaMemcpyPeerAsync(c->phihat.p, c->device, c0->phihat.p, c0->device, sizeof(float) * cells, c->stream));
+    }
+    // every part samples its test documents before any is waited for
+    for (ldagpu_handle c : parts) MC(h, c, heldout_enqueue(c, hd, R));
+    for (ldagpu_handle c : parts) {
+        const size_t D = c->h_test_doc_off.size() - 1, o = ll.size();
+        ll.resize(o + D);
+        CK(h, cudaSetDevice(c->device));
+        if (D) CK(h, cudaMemcpyAsync(ll.data() + o, c->ho_ll.p, sizeof(double) * D, cudaMemcpyDeviceToHost, c->stream));
+        MC(h, c, sync_check(c));
+    }
+    return 0;
+}
+
+// one process per GPU: every rank's per-document values to every rank, placed by global test-document index
+static int heldout_allgather(ldagpu_handle h, const std::vector<double> &local, std::vector<double> &global)
+{
+    DevBuf<int64_t> n;
+    DevBuf<double> buf;
+    auto body = [&]() -> int {
+        int64_t end = h->test_doc_base + (int64_t)local.size();
+        CK(h, n.alloc(1));
+        CK(h, cudaMemcpyAsync(n.p, &end, sizeof end, cudaMemcpyHostToDevice, h->stream));
+        NK(h, g_nccl.AllReduce(n.p, n.p, 1, ncclInt64, ncclMax, h->comm, h->stream));
+        CK(h, cudaMemcpyAsync(&end, n.p, sizeof end, cudaMemcpyDeviceToHost, h->stream));
+        CK(h, cudaStreamSynchronize(h->stream));
+        // each cell is written by one rank and zero on the others, so the sum is exact in any order
+        CK(h, buf.alloc((size_t)std::max<int64_t>(end, 1)));
+        CK(h, cudaMemsetAsync(buf.p, 0, sizeof(double) * buf.n, h->stream));
+        if (!local.empty())
+            CK(h, cudaMemcpyAsync(buf.p + h->test_doc_base, local.data(), sizeof(double) * local.size(), cudaMemcpyHostToDevice,
+                                  h->stream));
+        NK(h, g_nccl.AllReduce(buf.p, buf.p, buf.n, ncclDouble, ncclSum, h->comm, h->stream));
+        global.assign((size_t)end, 0.0);
+        if (end) CK(h, cudaMemcpyAsync(global.data(), buf.p, sizeof(double) * (size_t)end, cudaMemcpyDeviceToHost, h->stream));
+        return sync_check(h);
+    };
+    const int rc = body();
+    n.release();
+    buf.release();
+    return rc;
+}
+
+int ldagpu_heldout_log_likelihood(ldagpu_handle h, int32_t n_particles, double *doc_ll, double *total)
+{
+    NEED(h);
+    if (!total) return h->fail("null total");
+    if (h->dm.K > MAX_REG_TILES * TILE)
+        return h->fail("held-out evaluation is limited to K <= %d topics (the dense left-to-right estimator); K = %d",
+                       MAX_REG_TILES * TILE, h->dm.K);
+    if (n_particles < 1 || n_particles >= (1 << 24)) return h->fail("n_particles must be in [1, 2^24)");
+    const Parts parts = h->parts();
+    std::vector<double> ll;
+    const int rc = heldout_run(h, parts, n_particles, ll);
+    heldout_release(parts);
+    if (rc) return 1;
+    if (doc_ll && !ll.empty()) std::copy(ll.begin(), ll.end(), doc_ll);
+    std::vector<double> all;
+    if (h->world > 1 && h->comm) {
+        if (heldout_allgather(h, ll, all)) return 1;
+    } else {
+        all.swap(ll);
+    }
+    double s = 0.0;
+    for (double v : all) s += v;   // global document order
+    *total = s;
     return 0;
 }
 

@@ -47,6 +47,7 @@ class LDAConfiguration:
     phi_mean_thin: int = 1
     exec_time: float = 10.0               # seconds of cumulative sampling time (LDAConfiguration.java:35)
     dataset: Optional[str] = None
+    test_dataset: Optional[str] = None    # held-out documents: getHeldOutLogLikelihood on the topic_interval grid
     stoplist: Optional[str] = None        # file with one stop word per line (ParsedLDAConfiguration.java:298-304)
     rare_threshold: int = 0               # RARE_WORD_THRESHOLD (LDAConfiguration.java:16)
     keep_numbers: bool = False            # ParsedLDAConfiguration.java:307-310
@@ -97,6 +98,22 @@ class LDAConfiguration:
                             rare_threshold=self.rare_threshold, keep_connectors=self.keep_connecting_punctuation,
                             tfidf_vocab_size=self.tfidf_vocab_size, max_token_buffer=self.max_doc_buf_size)
 
+    def loadTestDataset(self, alphabet, dataset_fn: Optional[str] = None, stoplist_dir: Optional[str] = None):
+        """The test set (``test_dataset``) read with the TRAINING alphabet frozen: words the training set does not hold
+        are dropped, as MALLET's pipes drop them once the alphabet is frozen."""
+        from .corpus import load_dataset
+        fn = dataset_fn or self.test_dataset
+        if not fn:
+            raise ValueError("no test_dataset configured")
+        stop = None
+        if self.stoplist:
+            cand = self.stoplist if os.path.isabs(self.stoplist) else os.path.join(
+                stoplist_dir or os.path.dirname(os.path.abspath(fn)), self.stoplist)
+            stop = cand if os.path.exists(cand) else None
+        return load_dataset(fn, stoplist=stop, keep_numbers=self.keep_numbers, alphabet=alphabet,
+                            keep_connectors=self.keep_connecting_punctuation, max_token_buffer=self.max_doc_buf_size,
+                            frozen_alphabet=True)
+
     @staticmethod
     def from_cfg(path: str, subconfig: Optional[str] = None, **overrides) -> "LDAConfiguration":
         """Parse a reference .cfg: global keys, then the [subconfig] section wins
@@ -120,7 +137,8 @@ class LDAConfiguration:
                           ("iterations", int), ("seed", int), ("start_diagnostic", int),
                           ("compute_likelihood", boolean), ("topic_interval", int),
                           ("save_phi_mean", boolean), ("phi_mean_burnin", int), ("phi_mean_thin", int),
-                          ("exec_time", float), ("dataset", str), ("stoplist", str), ("rare_threshold", int),
+                          ("exec_time", float), ("dataset", str), ("test_dataset", str), ("stoplist", str),
+                          ("rare_threshold", int),
                           ("keep_numbers", boolean), ("keep_connecting_punctuation", boolean),
                           ("tfidf_vocab_size", int), ("max_doc_buf_size", int), ("logging_path", str),
                           ("alias_poisson_threshold", int), ("hyperparam_optim_interval", int), ("save_phi", boolean),
@@ -247,6 +265,8 @@ class GpuLDASampler:
         self._doc_off = None
         self._tokens = None
         self.loglikelihood: List[float] = []
+        self.heldout_loglikelihood: List[float] = []
+        self._test_doc_off: Optional[np.ndarray] = None   # this process's test documents (None: no test set)
         self._rank, self._world = 0, 1
         self._doc_base = self._token_base = 0
 
@@ -331,6 +351,8 @@ class GpuLDASampler:
             java_seed = ((self.startSeed + 2 ** 31) % 2 ** 32) - 2 ** 31     # Java int
             self._ck(self._L.ldagpu_init_z_java_random(self._h, java_seed))
         self.loglikelihood = []
+        self.heldout_loglikelihood = []
+        self._test_doc_off = None
 
     @staticmethod
     def make_comm_id() -> bytes:
@@ -340,7 +362,36 @@ class GpuLDASampler:
         return bytes(buf)
 
     def addTestInstances(self, testSet: InstanceList):
-        raise NotImplementedError("held-out evaluation (MarginalProbEstimatorPlain) is outside the GPU path")
+        """LGS addTestInstances: upload the test set (type ids of the training alphabet, e.g. from
+        ``LDAConfiguration.loadTestDataset``).  With world > 1 this rank keeps the token-balanced shard of the test
+        documents that matches its rank, as for the training set; several GPUs of one process shard it themselves.
+        An empty test set removes it.  K <= 1024 only (DESIGN.md 4.8)."""
+        from .corpus import shard_documents_by_tokens, take_shard
+        self._need()
+        off, tokens = testSet.to_csr()
+        doc_base = token_base = 0
+        if self._world > 1:
+            d0, d1 = shard_documents_by_tokens(off, self._world)[self._rank]
+            off, tokens, doc_base, token_base = take_shard(off, tokens, d0, d1)
+        off = np.ascontiguousarray(off, np.int64)
+        tokens = np.ascontiguousarray(tokens, np.int32)
+        D = len(off) - 1 if testSet.size() else 0
+        self._ck(self._L.ldagpu_set_test_documents(self._h, D, ptr(off), ptr(tokens) if len(tokens) else None,
+                                                   doc_base, token_base))
+        self._test_doc_off = off if testSet.size() else None
+        self.heldout_loglikelihood = []
+
+    def heldOutLogLikelihood(self, n_particles: int = 10):
+        """MarginalProbEstimatorPlain.evaluateLeftToRight (UPL:604-611,840-844) on the current counts: MALLET's
+        left-to-right estimator with ``n_particles`` particles (MALLET's default 10) and no resampling.  Returns
+        (total over the whole test set, float64 array of ln p(w_d) for this process's test documents)."""
+        self._need()
+        if self._test_doc_off is None:
+            raise LdaGpuError("addTestInstances has not been called")
+        out = np.zeros(max(len(self._test_doc_off) - 1, 1), np.float64)
+        total = C.c_double(0)
+        self._ck(self._L.ldagpu_heldout_log_likelihood(self._h, int(n_particles), ptr(out), C.byref(total)))
+        return total.value, out[: len(self._test_doc_off) - 1]
 
     SWEEPS_PER_CALL = 10   # the abort flag and the exec_time budget are looked at between library calls
 
@@ -364,19 +415,24 @@ class GpuLDASampler:
             burn = int(cfg.phi_mean_burnin / 100.0 * iterations)          # UPL:206-207
             self._ck(self._L.ldagpu_set_phi_mean_schedule(self._h, burn, cfg.phi_mean_thin))
         self.preSample()
+        # the log-likelihood grid: every topic_interval sweeps when compute_likelihood is set or a test set is present
+        held_out = self._test_doc_off is not None
+        grid = cfg.compute_likelihood or held_out
         if cfg.compute_likelihood:
             self.loglikelihood.append(self.modelLogLikelihood())
+        if held_out:
+            self.heldout_loglikelihood.append(self.heldOutLogLikelihood()[0])
         hooked = any(getattr(type(self), n) is not getattr(GpuLDASampler, n)
                      for n in ("preIteration", "postIteration", "preZ", "postZ", "prePhi", "postPhi"))
         per_call = self.SWEEPS_PER_CALL if chunk is None else chunk
-        step = max(1, cfg.topic_interval) if cfg.compute_likelihood else iterations
+        step = max(1, cfg.topic_interval) if grid else iterations
         if per_call > 0:
             step = min(step, per_call)
         t_start = sum(self.getTimers())
         done_total = 0
         while done_total < iterations and not self.getAbort():
             n = min(step, iterations - done_total)
-            if cfg.compute_likelihood:   # keep the log-likelihood on its topic_interval grid
+            if grid:   # keep the log-likelihood on its topic_interval grid
                 n = min(n, max(1, cfg.topic_interval) - done_total % max(1, cfg.topic_interval))
             if cfg.hyperparam_optim_interval > 1:   # stop where alpha and beta are re-estimated (UPL:891-894)
                 it = self.getCurrentIteration()
@@ -405,6 +461,8 @@ class GpuLDASampler:
             if cfg.compute_likelihood and done == n and done_total % max(1, cfg.topic_interval) == 0:
                 self.loglikelihood.append(self.modelLogLikelihood())
                 self._log_likelihood_to_file(self.loglikelihood[-1])                          # UPL:846-850
+            if held_out and done == n and done_total % max(1, cfg.topic_interval) == 0:
+                self.heldout_loglikelihood.append(self.heldOutLogLikelihood()[0])            # UPL:840-844
             if done < n:
                 break
             if cfg.hyperparam_optim_interval > 1 and self.getCurrentIteration() % cfg.hyperparam_optim_interval == 0:
@@ -561,7 +619,8 @@ class GpuLDASampler:
         return list(self.loglikelihood)
 
     def getHeldOutLogLikelihood(self) -> List[float]:
-        return []
+        """The held-out log-likelihood series of sample() (empty without a test set)."""
+        return list(self.heldout_loglikelihood)
 
     def modelLogLikelihood(self) -> float:
         """UPL:1644-1758."""

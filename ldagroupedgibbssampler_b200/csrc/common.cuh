@@ -42,6 +42,14 @@ struct Dims {
 // NT of the register path for K <= MAX_REG_TILES * TILE, and lg of NT tiles (L = 4 * NT = 1 << lg)
 __host__ __device__ constexpr int reg_tiles(int K) { return K <= 128 ? 1 : K <= 256 ? 2 : K <= 512 ? 4 : 8; }
 __host__ __device__ constexpr int lg_of_tiles(int NT) { return NT == 1 ? 2 : NT == 2 ? 3 : NT == 4 ? 4 : 5; }
+// a row layout turned into the register path's (host code): NT, Ks = 128 * NT and lg from K
+inline Dims reg_path_dims(Dims dm)
+{
+    dm.NT = reg_tiles(dm.K);
+    dm.Ks = dm.NT * TILE;
+    dm.lg = lg_of_tiles(dm.NT);
+    return dm;
+}
 __host__ __device__ __forceinline__ int tpos_lg(int lg, int k)
 {
     return (((k & ((1 << lg) - 1)) >> 2) << 7) | ((k >> lg) << 2) | (k & 3);

@@ -76,9 +76,25 @@ struct NcclApi {
 };
 NcclApi g_nccl;
 
+// Device memory owned by one object, freed when it is destroyed or overwritten.  That must happen with its own device
+// current: the engine never relies on a cudaFree issued from another device.
 template <typename T> struct DevBuf {
     T *p = nullptr;
     size_t n = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    DevBuf(DevBuf &&o) noexcept : p(o.p), n(o.n) { o.p = nullptr; o.n = 0; }
+    DevBuf &operator=(DevBuf &&o) noexcept
+    {
+        if (this != &o) {
+            release();
+            p = o.p; n = o.n;
+            o.p = nullptr; o.n = 0;
+        }
+        return *this;
+    }
+    ~DevBuf() { release(); }
     cudaError_t alloc(size_t count)
     {
         release();
@@ -831,7 +847,6 @@ int setup_peer_exchange(ldagpu_handle h)
     std::vector<IpcBlob> all((size_t)G);
     CK(h, cudaMemcpyAsync(all.data(), blobs.p, sizeof(IpcBlob) * (size_t)G, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    blobs.release();
 
     PeerTable &pt = h->pt;
     if (ok) {
@@ -866,7 +881,6 @@ int setup_peer_exchange(ldagpu_handle h)
     int all_ok = 0;
     CK(h, cudaMemcpyAsync(&all_ok, agree.p, sizeof all_ok, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    agree.release();
     if (!all_ok) {
         if (ok) h->p2p_note = "another rank could not map peer memory";
         close_peer_exchange(h);
@@ -958,6 +972,47 @@ int refresh_counts_and_phi(ldagpu_handle h, bool redraw_phi)
     return sync_all(h, parts);
 }
 
+// what is wrong with the CSR offsets of D documents (appended to the array's name), or nullptr
+const char *csr_offsets_error(const int64_t *off, int64_t D)
+{
+    if (off[0] != 0) return "[0] must be 0";
+    for (int64_t d = 0; d < D; ++d)
+        if (off[d + 1] < off[d]) return " must be non-decreasing";
+    return nullptr;
+}
+
+// The shard rule of a group, for its training set and its test set: documents [0, D) with offsets `off` split by token
+// count into `parts` contiguous ranges; part g holds documents [d0[g], d0[g + 1]) and tokens [t0[g], t0[g + 1])
+void shard_bounds_by_tokens(const int64_t *off, int64_t D, int parts, std::vector<int64_t> &d0, std::vector<int64_t> &t0)
+{
+    d0.assign((size_t)parts + 1, D);
+    d0[0] = 0;
+    const int64_t N = off[D];
+    for (int g = 1; g < parts; ++g) {
+        const int64_t target = N / parts * g;
+        int64_t d = std::lower_bound(off, off + D + 1, target) - off;
+        d0[(size_t)g] = std::min<int64_t>(std::max<int64_t>(d, d0[(size_t)g - 1]), D);
+    }
+    t0.resize(d0.size());
+    for (size_t g = 0; g < d0.size(); ++g) t0[g] = off[d0[g]];
+}
+
+// documents [d0, d1) of `off` as a part's own offsets: off[d0..d1] - off[d0]
+std::vector<int64_t> local_offsets(const int64_t *off, int64_t d0, int64_t d1)
+{
+    std::vector<int64_t> loc((size_t)(d1 - d0) + 1);
+    for (int64_t d = d0; d <= d1; ++d) loc[(size_t)(d - d0)] = off[d] - off[d0];
+    return loc;
+}
+
+// held-out evaluation runs the register path's draw only
+int heldout_refuses_k(ldagpu_handle h)
+{
+    if (h->dm.K <= MAX_REG_TILES * TILE) return 0;
+    return h->fail("held-out evaluation is limited to K <= %d topics (the dense left-to-right estimator); K = %d",
+                   MAX_REG_TILES * TILE, h->dm.K);
+}
+
 }  // namespace
 
 // =============================================================================================
@@ -992,9 +1047,7 @@ int ldagpu_create(int32_t K, int32_t V, int64_t D, const int64_t *doc_offsets, c
     if (!(beta > 0.0)) return bail("beta must be > 0");   // ParallelRandoms.java:61-63
     for (int k = 0; k < K; ++k)
         if (!(alpha[k] > 0.0)) return bail("alpha must be > 0");
-    if (doc_offsets[0] != 0) return bail("doc_offsets[0] must be 0");
-    for (int64_t d = 0; d < D; ++d)
-        if (doc_offsets[d + 1] < doc_offsets[d]) return bail("doc_offsets must be non-decreasing");
+    if (const char *e = csr_offsets_error(doc_offsets, D)) return bail(std::string("doc_offsets") + e);
     int ndev = ldagpu_device_count();
     if (ndev == 0) return bail("no CUDA device: libldagpu has no CPU fallback");
     if (device < 0 || device >= ndev) return bail("device ordinal out of range");
@@ -1010,9 +1063,7 @@ int ldagpu_create(int32_t K, int32_t V, int64_t D, const int64_t *doc_offsets, c
     if (scheme != LDAGPU_SCHEME_SPALIAS && K <= MAX_REG_TILES * TILE) {
         // register path of the dense z-step: 1, 2, 4 or 8 tiles, lane l owns 4 * NT consecutive topics and the
         // rows of Phi^T / n_wk / theta are stored in the matching column order (common.cuh: tpos / ttopic)
-        dm.NT = reg_tiles(K);
-        dm.Ks = dm.NT * TILE;
-        dm.lg = lg_of_tiles(dm.NT);
+        dm = reg_path_dims(dm);
     }
     dm.V = V; dm.Vp = (int32_t)round_up(V, PHI_ROW_BLOCK * PHI_SEGMENTS);
     dm.D = D; dm.N = doc_offsets[D]; dm.doc_base = doc_base; dm.token_base = token_base;
@@ -1108,21 +1159,11 @@ int ldagpu_destroy(ldagpu_handle h)
     for (void *p : h->ipc_opened) cudaIpcCloseMemHandle(p);
     h->ipc_opened.clear();
     if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
-    h->nk_parts.release(); h->p2p_flags.release(); h->p2p_local.release();
     for (cudaEvent_t e : h->events) cudaEventDestroy(e);
     for (cudaEvent_t e : h->copy_events) cudaEventDestroy(e);
     if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
-    h->doc_off.release(); h->item_begin.release(); h->tokens.release(); h->z.release(); h->z_stage.release(); h->z16.release();
-    h->n_wk.release();
-    h->n_k.release(); h->item_doc.release(); h->long_docs.release(); h->scratch_i32.release(); h->phiT.release(); h->theta.release();
-    h->alpha_f.release(); h->alpha_d.release(); h->lgs_alpha.release(); h->partial.release(); h->seg.release(); h->topic_sum.release();
-    h->phi_mean.release(); h->red.release(); h->red_out.release(); h->scratch_f64.release();
-    h->counter.release(); h->bad.release();
-    h->alias_table.release(); h->type_norm.release(); h->alias_stack.release(); h->alias_bs.release();
-    h->active_types.release(); h->sparse_lists.release();
-    h->test_doc_off.release(); h->test_tokens.release(); h->phihat.release(); h->ho_scores.release(); h->ho_ll.release();
     if (h->stream) cudaStreamDestroy(h->stream);
-    delete h;
+    delete h;   // its device buffers, with its device current
     return 0;
 }
 
@@ -1156,7 +1197,6 @@ int ldagpu_comm_init(ldagpu_handle h, int32_t rank, int32_t world, const void *i
     NK(h, g_nccl.AllReduce(tmp.p, tmp.p, 1, ncclInt64, ncclSum, h->comm, h->stream));
     CK(h, cudaMemcpyAsync(&d, tmp.p, sizeof d, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    tmp.release();
     h->D_global = d;
     return setup_peer_exchange(h);
 }
@@ -1710,25 +1750,14 @@ int ldagpu_create_multi(int32_t K, int32_t V, int64_t D, const int64_t *doc_offs
             }
             cudaGetLastError();
         }
-    // documents shard by TOKEN count into contiguous ranges (SURVEY 8e; north_star)
-    const int64_t N = doc_offsets[D];
     ldagpu_handle P = new ldagpu_handle_s();
-    P->dm.K = K; P->dm.V = V; P->dm.D = D; P->dm.N = N; P->dm.Ks = K; P->dm.lg = 2;
+    P->dm.K = K; P->dm.V = V; P->dm.D = D; P->dm.N = doc_offsets[D]; P->dm.Ks = K; P->dm.lg = 2;
     P->scheme = scheme; P->device = dev[0]; P->seed = seed; P->beta = beta; P->world = n_devices;
-    P->shard_doc0.assign((size_t)n_devices + 1, D);
-    P->shard_tok0.assign((size_t)n_devices + 1, N);
-    P->shard_doc0[0] = 0;
-    for (int g = 1; g < n_devices; ++g) {
-        const int64_t target = N / n_devices * g;
-        int64_t d = std::lower_bound(doc_offsets, doc_offsets + D + 1, target) - doc_offsets;
-        d = std::min<int64_t>(std::max<int64_t>(d, P->shard_doc0[(size_t)g - 1]), D);
-        P->shard_doc0[(size_t)g] = d;
-    }
-    for (int g = 0; g <= n_devices; ++g) P->shard_tok0[(size_t)g] = doc_offsets[P->shard_doc0[(size_t)g]];
+    // documents shard by TOKEN count into contiguous ranges (SURVEY 8e; north_star)
+    shard_bounds_by_tokens(doc_offsets, D, n_devices, P->shard_doc0, P->shard_tok0);
     for (int g = 0; g < n_devices; ++g) {
         const int64_t d0 = P->shard_doc0[(size_t)g], d1 = P->shard_doc0[(size_t)g + 1], t0 = P->shard_tok0[(size_t)g];
-        std::vector<int64_t> loc((size_t)(d1 - d0) + 1);
-        for (int64_t d = d0; d <= d1; ++d) loc[(size_t)(d - d0)] = doc_offsets[d] - t0;
+        const std::vector<int64_t> loc = local_offsets(doc_offsets, d0, d1);
         ldagpu_handle c = nullptr;
         if (ldagpu_create(K, V, d1 - d0, loc.data(), tokens ? tokens + t0 : nullptr, alpha, beta, seed, scheme, dev[(size_t)g],
                           d0, t0, &c)) {
@@ -1807,8 +1836,7 @@ int ldagpu_get_count_histograms(ldagpu_handle h, int32_t n_doc_bins, int64_t *do
         if (c->world > 1 && c->comm)
             NK(h, g_nccl.AllReduce(buf.p, buf.p, nd + nt, ncclUint64, ncclSum, c->comm, c->stream));
         CK(h, cudaMemcpyAsync(tmp.data(), buf.p, sizeof(unsigned long long) * (nd + nt), cudaMemcpyDeviceToHost, c->stream));
-        if (sync_check(c)) { h->err = c->err; buf.release(); return 1; }
-        buf.release();
+        if (sync_check(c)) { h->err = c->err; return 1; }
         for (size_t i = 0; i < nd + nt; ++i) acc[i] += tmp[i];
     }
     const int64_t D_all = parts[0]->D_global;
@@ -1828,40 +1856,21 @@ int ldagpu_get_count_histograms(ldagpu_handle h, int32_t n_doc_bins, int64_t *do
 }
 
 // ---- held-out evaluation (MarginalProbEstimatorPlain.evaluateLeftToRight, UPL:604-611,840-844; kernels_heldout.cu)
-// documents [0, D) with offsets `off` sharded by token count into `parts` contiguous ranges (the rule of create_multi)
-static std::vector<int64_t> shard_bounds_by_tokens(const int64_t *off, int64_t D, int parts)
-{
-    std::vector<int64_t> d0((size_t)parts + 1, D);
-    d0[0] = 0;
-    const int64_t N = off[D];
-    for (int g = 1; g < parts; ++g) {
-        const int64_t target = N / parts * g;
-        int64_t d = std::lower_bound(off, off + D + 1, target) - off;
-        d0[(size_t)g] = std::min<int64_t>(std::max<int64_t>(d, d0[(size_t)g - 1]), D);
-    }
-    return d0;
-}
-
 // replace this part's test set by documents [0, D) (offsets from 0); the old one is released only once the new one is on
 // the device
 static int set_test_one(ldagpu_handle c, int64_t D, const int64_t *off, const int32_t *tok, int64_t doc_base, int64_t token_base)
 {
     DevBuf<int64_t> o;
     DevBuf<int32_t> t;
-    auto upload = [&]() -> int {
-        if (D == 0) return 0;
+    if (D > 0) {
         const int64_t N = off[D];
         CK(c, o.alloc((size_t)D + 1));
         CK(c, t.alloc((size_t)std::max<int64_t>(N, 1)));
         CK(c, cudaMemcpy(o.p, off, sizeof(int64_t) * ((size_t)D + 1), cudaMemcpyHostToDevice));
         if (N) CK(c, cudaMemcpy(t.p, tok, sizeof(int32_t) * (size_t)N, cudaMemcpyHostToDevice));
-        return 0;
-    };
-    if (upload()) { o.release(); t.release(); return 1; }
-    std::swap(c->test_doc_off, o);
-    std::swap(c->test_tokens, t);
-    o.release();
-    t.release();
+    }
+    c->test_doc_off = std::move(o);
+    c->test_tokens = std::move(t);
     c->h_test_doc_off.assign(off, off + D + 1);
     c->test_doc_base = doc_base;
     c->test_token_base = token_base;
@@ -1872,30 +1881,24 @@ int ldagpu_set_test_documents(ldagpu_handle h, int64_t D_test, const int64_t *do
                               int64_t doc_base, int64_t token_base)
 {
     NEED(h);
-    const int32_t K = h->dm.K, V = h->dm.V;
-    if (K > MAX_REG_TILES * TILE)
-        return h->fail("held-out evaluation is limited to K <= %d topics (the dense left-to-right estimator); K = %d",
-                       MAX_REG_TILES * TILE, K);
+    if (heldout_refuses_k(h)) return 1;
+    const int32_t V = h->dm.V;
     if (D_test < 0 || doc_base < 0 || token_base < 0) return h->fail("D_test, doc_base and token_base must be >= 0");
     static const int64_t zero = 0;
     if (D_test == 0) doc_offsets = &zero;   // removes the test set
     if (!doc_offsets) return h->fail("null doc_offsets");
-    if (doc_offsets[0] != 0) return h->fail("test doc_offsets[0] must be 0");
-    for (int64_t d = 0; d < D_test; ++d)
-        if (doc_offsets[d + 1] < doc_offsets[d]) return h->fail("test doc_offsets must be non-decreasing");
+    if (const char *e = csr_offsets_error(doc_offsets, D_test)) return h->fail("test doc_offsets%s", e);
     const int64_t N = doc_offsets[D_test];
     if (N > 0 && !tokens) return h->fail("null tokens");
     for (int64_t i = 0; i < N; ++i)
         if (tokens[i] < 0 || tokens[i] >= V)
             return h->fail("test token %lld: type id %d out of range [0, %d)", (long long)i, tokens[i], V);
     const Parts parts = h->parts();
-    const std::vector<int64_t> d0 = shard_bounds_by_tokens(doc_offsets, D_test, (int)parts.size());
-    std::vector<int64_t> t0(d0.size());
-    for (size_t g = 0; g < d0.size(); ++g) t0[g] = doc_offsets[d0[g]];
+    std::vector<int64_t> d0, t0;
+    shard_bounds_by_tokens(doc_offsets, D_test, (int)parts.size(), d0, t0);
     for (size_t g = 0; g < parts.size(); ++g) {
         ldagpu_handle c = parts[g];
-        std::vector<int64_t> loc((size_t)(d0[g + 1] - d0[g]) + 1);
-        for (int64_t d = d0[g]; d <= d0[g + 1]; ++d) loc[(size_t)(d - d0[g])] = doc_offsets[d] - t0[g];
+        const std::vector<int64_t> loc = local_offsets(doc_offsets, d0[g], d0[g + 1]);
         MC(h, c, set_test_one(c, d0[g + 1] - d0[g], loc.data(), tokens ? tokens + t0[g] : nullptr, doc_base + d0[g],
                               token_base + t0[g]));
     }
@@ -1961,10 +1964,7 @@ static int heldout_run(ldagpu_handle h, const Parts &parts, int32_t R, std::vect
     // the global counts on parts[0] (a rank: on every rank), phihat from them, copied to the other shards of a group
     if (gather_rows(h, parts, &ldagpu_handle_s::n_wk, ncclInt32)) return 1;
     ldagpu_handle c0 = parts[0];
-    Dims hd = c0->dm;
-    hd.NT = reg_tiles(hd.K);
-    hd.Ks = hd.NT * TILE;
-    hd.lg = lg_of_tiles(hd.NT);
+    const Dims hd = reg_path_dims(c0->dm);
     const size_t cells = (size_t)hd.Vp * hd.Ks;
     for (ldagpu_handle c : parts) {
         CK(h, cudaSetDevice(c->device));
@@ -1998,37 +1998,29 @@ static int heldout_allgather(ldagpu_handle h, const std::vector<double> &local, 
 {
     DevBuf<int64_t> n;
     DevBuf<double> buf;
-    auto body = [&]() -> int {
-        int64_t end = h->test_doc_base + (int64_t)local.size();
-        CK(h, n.alloc(1));
-        CK(h, cudaMemcpyAsync(n.p, &end, sizeof end, cudaMemcpyHostToDevice, h->stream));
-        NK(h, g_nccl.AllReduce(n.p, n.p, 1, ncclInt64, ncclMax, h->comm, h->stream));
-        CK(h, cudaMemcpyAsync(&end, n.p, sizeof end, cudaMemcpyDeviceToHost, h->stream));
-        CK(h, cudaStreamSynchronize(h->stream));
-        // each cell is written by one rank and zero on the others, so the sum is exact in any order
-        CK(h, buf.alloc((size_t)std::max<int64_t>(end, 1)));
-        CK(h, cudaMemsetAsync(buf.p, 0, sizeof(double) * buf.n, h->stream));
-        if (!local.empty())
-            CK(h, cudaMemcpyAsync(buf.p + h->test_doc_base, local.data(), sizeof(double) * local.size(), cudaMemcpyHostToDevice,
-                                  h->stream));
-        NK(h, g_nccl.AllReduce(buf.p, buf.p, buf.n, ncclDouble, ncclSum, h->comm, h->stream));
-        global.assign((size_t)end, 0.0);
-        if (end) CK(h, cudaMemcpyAsync(global.data(), buf.p, sizeof(double) * (size_t)end, cudaMemcpyDeviceToHost, h->stream));
-        return sync_check(h);
-    };
-    const int rc = body();
-    n.release();
-    buf.release();
-    return rc;
+    int64_t end = h->test_doc_base + (int64_t)local.size();
+    CK(h, n.alloc(1));
+    CK(h, cudaMemcpyAsync(n.p, &end, sizeof end, cudaMemcpyHostToDevice, h->stream));
+    NK(h, g_nccl.AllReduce(n.p, n.p, 1, ncclInt64, ncclMax, h->comm, h->stream));
+    CK(h, cudaMemcpyAsync(&end, n.p, sizeof end, cudaMemcpyDeviceToHost, h->stream));
+    CK(h, cudaStreamSynchronize(h->stream));
+    // each cell is written by one rank and zero on the others, so the sum is exact in any order
+    CK(h, buf.alloc((size_t)std::max<int64_t>(end, 1)));
+    CK(h, cudaMemsetAsync(buf.p, 0, sizeof(double) * buf.n, h->stream));
+    if (!local.empty())
+        CK(h, cudaMemcpyAsync(buf.p + h->test_doc_base, local.data(), sizeof(double) * local.size(), cudaMemcpyHostToDevice,
+                              h->stream));
+    NK(h, g_nccl.AllReduce(buf.p, buf.p, buf.n, ncclDouble, ncclSum, h->comm, h->stream));
+    global.assign((size_t)end, 0.0);
+    if (end) CK(h, cudaMemcpyAsync(global.data(), buf.p, sizeof(double) * (size_t)end, cudaMemcpyDeviceToHost, h->stream));
+    return sync_check(h);
 }
 
 int ldagpu_heldout_log_likelihood(ldagpu_handle h, int32_t n_particles, double *doc_ll, double *total)
 {
     NEED(h);
     if (!total) return h->fail("null total");
-    if (h->dm.K > MAX_REG_TILES * TILE)
-        return h->fail("held-out evaluation is limited to K <= %d topics (the dense left-to-right estimator); K = %d",
-                       MAX_REG_TILES * TILE, h->dm.K);
+    if (heldout_refuses_k(h)) return 1;
     if (n_particles < 1 || n_particles >= (1 << 24)) return h->fail("n_particles must be in [1, 2^24)");
     const Parts parts = h->parts();
     std::vector<double> ll;

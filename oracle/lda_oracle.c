@@ -383,10 +383,11 @@ static int32_t draw_topic_contract_tiles(const float *a, const float *phirow, in
  *   Kogge-Stone inclusive scan of the 32 lane totals (offsets 1, 2, 4, 8, 16): S = scan[31];
  *   u = U*S; lane = first l with scan[l] >= u; r = u - scan[l-1]; element = first m with p_m >= r.
  * Same selection rule as the reference's walk (first k with cumsum_k >= U*sum), natural topic order.
+ * S_out (may be NULL) receives S: the held-out estimator averages it.
  * ------------------------------------------------------------------------------------------ */
 static int lanes_tiles(int32_t K) { return K <= 128 ? 1 : K <= 256 ? 2 : K <= 512 ? 4 : 8; }
 
-static int32_t draw_topic_contract_lanes(const float *a, const float *phirow, int32_t K, float U)
+static int32_t draw_topic_contract_lanes(const float *a, const float *phirow, int32_t K, float U, float *S_out)
 {
     const int L = 4 * lanes_tiles(K);
     float p[32][32], x[32], y[32];
@@ -405,6 +406,7 @@ static int32_t draw_topic_contract_lanes(const float *a, const float *phirow, in
         memcpy(x, y, sizeof x);
     }
     float S = x[31];
+    if (S_out) *S_out = S;
     float u = U * S;
     int ls = 31;
     for (int l = 0; l < 32; ++l)
@@ -421,7 +423,7 @@ static int32_t draw_topic_contract_lanes(const float *a, const float *phirow, in
  * larger K walks it in shared memory tile by tile (tile tree) */
 static int32_t draw_topic_contract(const float *a, const float *phirow, int32_t K, float U, float *scratch)
 {
-    return K <= 1024 ? draw_topic_contract_lanes(a, phirow, K, U)
+    return K <= 1024 ? draw_topic_contract_lanes(a, phirow, K, U, NULL)
                      : draw_topic_contract_tiles(a, phirow, K, U, scratch);
 }
 
@@ -444,6 +446,13 @@ static inline double z_uniform_f64(uint64_t seed, uint64_t token, uint32_t sweep
 {
     /* same 23 bits the contract uses, so faithful and contract walk with the same U */
     return (double)z_uniform_f32(seed, token, sweep);
+}
+/* held-out evaluation: particle r of the test token at `iteration` (DESIGN.md 4.8); both modes use this fp32 value */
+static inline float heldout_uniform_f32(uint64_t seed, uint64_t token, uint32_t iteration, uint32_t r)
+{
+    uint32_t w[4] = {(uint32_t)token, (uint32_t)(token >> 32), iteration, ((uint32_t)ORACLE_STREAM_HELDOUT << 24) | r};
+    philox4x32_10(w, (uint32_t)seed, (uint32_t)(seed >> 32));
+    return ((float)(w[0] >> 9) + 0.5f) * 0x1p-23f;
 }
 
 /* ------------------------------------------------------------------------------------------
@@ -673,6 +682,120 @@ void oracle_z_pcgs_faithful(int64_t D, const int64_t *doc_off, const int32_t *to
         free(cnt);
         free(score);
     }
+}
+
+/* ------------------------------------------------------------------------------------------
+ * Held-out log-likelihood (DESIGN.md 4.8).  MALLET's MarginalProbEstimator.evaluateLeftToRight
+ * without resampling (Wallach et al. 2009), which the reference's MarginalProbEstimatorPlain
+ * restates over plain count arrays (topics/UncollapsedParallelLDA.java:604-611,840-844 call it).
+ * phihat_kw = (n_wk + beta) / (n_k + V beta); per document and particle r, from n_dk = 0:
+ * S_i = sum_k (n_dk + alpha_k) phihat_kw, draw z_i, n_dz += 1;
+ * l_d = sum_i ln((1/R) sum_r S_i^r / (i + alpha_sum)).  K <= 1024 (the lane-contiguous draw).
+ * ------------------------------------------------------------------------------------------ */
+static double alpha_sum_of(const double *alpha, int32_t K)
+{
+    double s = 0.0;
+    for (int k = 0; k < K; ++k) s += alpha[k];
+    return s;
+}
+
+static int64_t longest_doc(int64_t D, const int64_t *doc_off)
+{
+    int64_t m = 0;
+    for (int64_t d = 0; d < D; ++d)
+        if (doc_off[d + 1] - doc_off[d] > m) m = doc_off[d + 1] - doc_off[d];
+    return m > 0 ? m : 1;
+}
+
+/* contract: fp32 phihat (one fp64 division per cell) and scores, the draw's own S summed over the particles in fp64 in
+ * particle order, the contract ln of the fp64 mean */
+double oracle_heldout_l2r_contract(int64_t D, const int64_t *doc_off, const int32_t *tokens, int32_t V, int32_t K,
+                                   const int32_t *n_wk, const int32_t *n_k, const double *alpha, double beta,
+                                   uint64_t seed, uint32_t iteration, int64_t token_base, int32_t R, double *doc_ll)
+{
+    float *ph = (float *)malloc(sizeof(float) * (size_t)V * (size_t)K);
+    const double vbeta = (double)V * beta, alpha_sum = alpha_sum_of(alpha, K);
+    for (int64_t w = 0; w < V; ++w)
+        for (int k = 0; k < K; ++k)
+            ph[w * K + k] = (float)(((double)n_wk[w * K + k] + beta) / ((double)n_k[k] + vbeta));
+    const int64_t max_len = longest_doc(D, doc_off);
+#pragma omp parallel
+    {
+        int32_t *cnt = (int32_t *)malloc(sizeof(int32_t) * (size_t)K);
+        float *a = (float *)malloc(sizeof(float) * (size_t)K);
+        double *acc = (double *)malloc(sizeof(double) * (size_t)max_len);
+#pragma omp for schedule(dynamic, 4)
+        for (int64_t d = 0; d < D; ++d) {
+            const int64_t t0 = doc_off[d], n = doc_off[d + 1] - t0;
+            for (int64_t i = 0; i < n; ++i) acc[i] = 0.0;
+            for (int32_t r = 0; r < R; ++r) {
+                memset(cnt, 0, sizeof(int32_t) * (size_t)K);
+                for (int k = 0; k < K; ++k) a[k] = (float)alpha[k];
+                for (int64_t i = 0; i < n; ++i) {
+                    const float U = heldout_uniform_f32(seed, (uint64_t)(token_base + t0 + i), iteration, (uint32_t)r);
+                    float S = 0.0f;
+                    const int32_t k = draw_topic_contract_lanes(a, ph + (size_t)tokens[t0 + i] * K, K, U, &S);
+                    acc[i] = acc[i] + (double)S;
+                    cnt[k] += 1;
+                    a[k] = (float)cnt[k] + (float)alpha[k];
+                }
+            }
+            double ll = 0.0;
+            for (int64_t i = 0; i < n; ++i) ll = ll + c_ln_f64(acc[i] / ((double)R * ((double)i + alpha_sum)));
+            doc_ll[d] = ll;
+        }
+        free(acc);
+        free(a);
+        free(cnt);
+    }
+    free(ph);
+    double total = 0.0;
+    for (int64_t d = 0; d < D; ++d) total += doc_ll[d];
+    return total;
+}
+
+/* faithful: fp64 phihat and scores, sequential sums over k, the reference's walk, libm log; the same uniforms */
+double oracle_heldout_l2r_faithful(int64_t D, const int64_t *doc_off, const int32_t *tokens, int32_t V, int32_t K,
+                                   const int32_t *n_wk, const int32_t *n_k, const double *alpha, double beta,
+                                   uint64_t seed, uint32_t iteration, int64_t token_base, int32_t R, double *doc_ll)
+{
+    double *ph = (double *)malloc(sizeof(double) * (size_t)V * (size_t)K);
+    const double vbeta = (double)V * beta, alpha_sum = alpha_sum_of(alpha, K);
+    for (int64_t w = 0; w < V; ++w)
+        for (int k = 0; k < K; ++k) ph[w * K + k] = ((double)n_wk[w * K + k] + beta) / ((double)n_k[k] + vbeta);
+    const int64_t max_len = longest_doc(D, doc_off);
+#pragma omp parallel
+    {
+        int32_t *cnt = (int32_t *)malloc(sizeof(int32_t) * (size_t)K);
+        double *score = (double *)malloc(sizeof(double) * (size_t)K);
+        double *prob = (double *)malloc(sizeof(double) * (size_t)max_len);
+#pragma omp for schedule(dynamic, 4)
+        for (int64_t d = 0; d < D; ++d) {
+            const int64_t t0 = doc_off[d], n = doc_off[d + 1] - t0;
+            for (int64_t i = 0; i < n; ++i) prob[i] = 0.0;
+            for (int32_t r = 0; r < R; ++r) {
+                memset(cnt, 0, sizeof(int32_t) * (size_t)K);
+                for (int64_t i = 0; i < n; ++i) {
+                    const double *row = ph + (size_t)tokens[t0 + i] * K;
+                    double sum = 0.0;
+                    for (int k = 0; k < K; ++k) { score[k] = ((double)cnt[k] + alpha[k]) * row[k]; sum += score[k]; }
+                    prob[i] += sum / ((double)i + alpha_sum);
+                    const double U = (double)heldout_uniform_f32(seed, (uint64_t)(token_base + t0 + i), iteration, (uint32_t)r);
+                    cnt[walk_faithful(score, sum, U, K)] += 1;
+                }
+            }
+            double ll = 0.0;
+            for (int64_t i = 0; i < n; ++i) ll += log(prob[i] / (double)R);
+            doc_ll[d] = ll;
+        }
+        free(prob);
+        free(score);
+        free(cnt);
+    }
+    free(ph);
+    double total = 0.0;
+    for (int64_t d = 0; d < D; ++d) total += doc_ll[d];
+    return total;
 }
 
 /* ------------------------------------------------------------------------------------------

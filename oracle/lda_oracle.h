@@ -3,9 +3,9 @@
  *
  * CPU restatement of one Gibbs sweep of the reference's exact-parallel LDA
  * samplers (LDAGroupedGibbsSampler = "GGS", UncollapsedParallelLDA /
- * LDAPartiallyCollapsedGibbsSampler = "PCGS").  Only tests/, __graft_entry__.smoke()
- * and bench.py's cpu_baseline / --impl reference legs may load this library; the
- * product (libldagpu.so) never does.
+ * LDAPartiallyCollapsedGibbsSampler = "PCGS") and the held-out left-to-right estimator.
+ * Only tests/, __graft_entry__.smoke(), bench.py's cpu_baseline / --impl reference legs
+ * and tools/heldout_bench.py may load this library; the product (libldagpu.so) never does.
  *
  * PARITY UNPINNED (against a running reference): the reference is Java 8 + MALLET 2.0.8
  * and there is no JDK in the build container, the reference holds no golden vectors for
@@ -32,7 +32,7 @@ extern "C" {
 #endif
 
 enum { ORACLE_GGS = 0, ORACLE_PCGS = 1 };
-enum { ORACLE_STREAM_Z = 1, ORACLE_STREAM_THETA = 2, ORACLE_STREAM_PHI = 3, ORACLE_STREAM_POISSON = 4 };
+enum { ORACLE_STREAM_Z = 1, ORACLE_STREAM_THETA = 2, ORACLE_STREAM_PHI = 3, ORACLE_STREAM_POISSON = 4, ORACLE_STREAM_HELDOUT = 5 };
 
 void oracle_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
 
@@ -118,6 +118,17 @@ double oracle_log_likelihood_lgamma(int64_t D, const int64_t *doc_off, const int
 double oracle_log_posterior(int64_t D, const int64_t *doc_off, const int32_t *tokens,
                             const int32_t *z, int32_t K, int32_t V, const double *theta,
                             const double *phiT, const double *alpha, double beta);
+
+/* held-out log-likelihood, left-to-right estimator without resampling: MALLET's MarginalProbEstimator.evaluateLeftToRight
+ * (Wallach et al. 2009) as the reference's MarginalProbEstimatorPlain restates it (UncollapsedParallelLDA.java:604-611,
+ * 840-844 call it).  Test set doc_off[D+1] / tokens (token_base = global index of its first token), R particles at
+ * `iteration`, K <= 1024.  doc_ll[D] receives ln p(w_d); returns their sum in document order. */
+double oracle_heldout_l2r_contract(int64_t D, const int64_t *doc_off, const int32_t *tokens, int32_t V, int32_t K,
+                                   const int32_t *n_wk, const int32_t *n_k, const double *alpha, double beta,
+                                   uint64_t seed, uint32_t iteration, int64_t token_base, int32_t R, double *doc_ll);
+double oracle_heldout_l2r_faithful(int64_t D, const int64_t *doc_off, const int32_t *tokens, int32_t V, int32_t K,
+                                   const int32_t *n_wk, const int32_t *n_k, const double *alpha, double beta,
+                                   uint64_t seed, uint32_t iteration, int64_t token_base, int32_t R, double *doc_ll);
 
 /* whole sweeps, contract mode: for it in first_sweep..first_sweep+n-1:
  *   [GGS: theta], z, counts, Phi     (order: UncollapsedParallelLDA.java:645-693)

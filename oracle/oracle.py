@@ -1,7 +1,8 @@
 """ctypes binding of the CPU oracle (oracle/lda_oracle.c) -- TEST INFRASTRUCTURE ONLY.
 
-Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs
-import this module.  The product package (ldagroupedgibbssampler_b200) never does.
+Only tests/, __graft_entry__.smoke(), bench.py's cpu_baseline / --impl reference legs and
+tools/heldout_bench.py's CPU rate import this module.  The product package (ldagroupedgibbssampler_b200)
+never does.
 
 PARITY UNPINNED against a running reference (no JDK here; see lda_oracle.h).
 """
@@ -85,6 +86,9 @@ def lib():
     sig("oracle_log_likelihood", f64, i64, _i64p, _i32p, i32, i32, _i32p, _i32p, _f64p, f64)
     sig("oracle_log_likelihood_lgamma", f64, i64, _i64p, _i32p, i32, i32, _i32p, _i32p, _f64p, f64)
     sig("oracle_log_posterior", f64, i64, _i64p, _i32p, _i32p, i32, i32, _f64p, _f64p, _f64p, f64)
+    for mode in ("contract", "faithful"):
+        sig("oracle_heldout_l2r_" + mode, f64, i64, _i64p, _i32p, i32, i32, _i32p, _i32p, _f64p, f64, u64, u32, i64, i32,
+            _f64p)
     sig("oracle_sweeps_contract", None, C.c_int, i64, i32, i32, _i64p, _i32p, _i32p, _f64p, f64,
         u64, u32, i32, _f32p, vp, _i32p, _i32p)
     sig("oracle_sweeps_faithful", None, C.c_int, i64, i32, i32, _i64p, _i32p, _i32p, _f64p, f64,
@@ -270,6 +274,21 @@ def log_posterior(doc_off, tokens, z, K, V, theta, phiT, alpha, beta):
         np.ascontiguousarray(tokens, np.int32), np.ascontiguousarray(z, np.int32), K, V,
         np.ascontiguousarray(theta, np.float64), np.ascontiguousarray(phiT, np.float64),
         np.ascontiguousarray(alpha, np.float64), beta)
+
+
+def heldout_l2r(mode, doc_off, tokens, n_wk, n_k, alpha, beta, seed, iteration, R=10, token_base=0):
+    """Held-out log-likelihood by the left-to-right estimator of the test set (doc_off, tokens) under the counts
+    n_wk [V][K] / n_k [K]; mode "contract" (bit-exact with the kernels) or "faithful" (fp64, libm).
+    Returns (total, per-document float64 array)."""
+    V, K = n_wk.shape
+    D = len(doc_off) - 1
+    out = np.zeros(max(D, 1), np.float64)
+    tok = np.ascontiguousarray(tokens, np.int32)
+    total = getattr(lib(), "oracle_heldout_l2r_" + mode)(
+        D, np.ascontiguousarray(doc_off, np.int64), tok if len(tok) else np.zeros(1, np.int32), V, K,
+        np.ascontiguousarray(n_wk, np.int32), np.ascontiguousarray(n_k, np.int32), np.ascontiguousarray(alpha, np.float64),
+        float(beta), int(seed) & 0xFFFFFFFFFFFFFFFF, int(iteration), int(token_base), int(R), out)
+    return total, out[:D]
 
 
 def sweeps(mode, scheme, doc_off, tokens, z, V, K, alpha, beta, seed, first_sweep, n_sweeps, phiT):

@@ -1,6 +1,7 @@
 """Run under torchrun on >= 2 GPUs: the sharded library run (NCCL reduce-scatter / all-gather inside
 libldagpu) must give bit-identical z, counts, Phi and (1e-9) log-likelihood to the CPU oracle run on
-the whole corpus -- results do not depend on the number of GPUs (SURVEY 8e "Determinism").
+the whole corpus -- results do not depend on the number of GPUs (SURVEY 8e "Determinism").  The held-out
+evaluation of a test set (DESIGN.md 4.8) must give the oracle's values bit for bit too.
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 \
         --master-port 29511 tests/multigpu_check.py
@@ -17,6 +18,28 @@ sys.path.insert(0, ROOT)
 import ldagroupedgibbssampler_b200 as L  # noqa: E402
 from ldagroupedgibbssampler_b200._lib import ptr  # noqa: E402
 from oracle import oracle as O  # noqa: E402
+
+
+def heldout(s, rank, world, V, K, beta, seed, n_wk, n_k):
+    """Held-out evaluation with one process per GPU: every rank uploads its token-balanced shard of the test set and
+    builds phihat from the all-gathered n_wk; the per-document values are all-gathered, so every rank returns the total
+    of the whole test set.  The concatenated per-document values and every rank's total must equal the oracle's contract
+    mode on the global counts n_wk / n_k bit for bit.  K > 1024 is refused on every rank."""
+    toff, ttok = L.synth_corpus(150, V, 50.0, seed=9, doc_first=400)
+    if K > 1024:
+        try:
+            s.addTestInstances(L.InstanceList.from_csr(toff, ttok, V))
+            return dict(heldout_refused=False)
+        except L.LdaGpuError as e:
+            return dict(heldout_refused="K <= 1024" in str(e))
+    s.addTestInstances(L.InstanceList.from_csr(toff, ttok, V))
+    parts = [None] * world
+    dist.all_gather_object(parts, s.heldOutLogLikelihood(10))
+    if rank != 0:
+        return {}
+    want_t, want_d = O.heldout_l2r("contract", toff, ttok, n_wk, n_k, s.alpha, beta, seed, s.getCurrentIteration(), R=10)
+    return dict(heldout_total=all(p[0] == want_t for p in parts),
+                heldout_doc_ll=np.array_equal(np.concatenate([p[1] for p in parts]), want_d))
 
 
 def stress(rank, world, local, sweeps):
@@ -149,6 +172,8 @@ def main():
         checks = dict(z=np.array_equal(z, st["z"]), n_wk=np.array_equal(n_wk, st["n_wk"]),
                       n_k=np.array_equal(n_k, st["n_k"]), phi=np.array_equal(phi, st["phiT"]),
                       ll=abs(ll - want_ll) <= 1e-9 * abs(want_ll))
+        # the evaluation changes no state, so the checks below are unaffected
+        checks.update(heldout(s, rank, world, V, K, beta, seed, n_wk, n_k))
         # z-only sweep (Phi frozen): stand-alone count exchange, no Phi draw
         s.sampleZGivenPhi(1)
         zs = [None] * world

@@ -3,7 +3,7 @@
 `--gpus` devices from THIS process and compares with the CPU oracle on the whole corpus, bit for bit:
 whole sweeps, a z-only sweep, the step-wise count rebuild + Phi draw, setZIndicators (32- and 16-bit, the
 refused out-of-range case included), theta / document-topic accessors in corpus order, log-likelihood and
-log-posterior, checkpoint/resume.
+log-posterior, checkpoint/resume, and the held-out evaluation of a test set (DESIGN.md 4.8).
 
     python tests/singleproc_multigpu_check.py --gpus 2
 """
@@ -40,6 +40,27 @@ def stalled_shard(gpus):
         return
     print("no error raised")
     sys.exit(1)
+
+
+def heldout(s, V, K, beta, seed):
+    """Held-out evaluation on the group: the test set is sharded by tokens over the shards and phihat is built once and
+    copied to the others.  The per-document values and the total must equal the oracle's contract mode on the device's
+    counts bit for bit -- the values one GPU gives -- and two evaluations at the same iteration must agree.  K > 1024 is
+    refused with an error naming the limit."""
+    toff, ttok = L.synth_corpus(150, V, 50.0, seed=9, doc_first=400)
+    if K > 1024:
+        try:
+            s.addTestInstances(L.InstanceList.from_csr(toff, ttok, V))
+            return dict(heldout_refused=False)
+        except L.LdaGpuError as e:
+            return dict(heldout_refused="K <= 1024" in str(e))
+    s.addTestInstances(L.InstanceList.from_csr(toff, ttok, V))
+    tot, dll = s.heldOutLogLikelihood(10)
+    tot2, dll2 = s.heldOutLogLikelihood(10)
+    want_t, want_d = O.heldout_l2r("contract", toff, ttok, s.getTypeTopicMatrix(), s.getTopicTotals(), s.alpha, beta, seed,
+                                   s.getCurrentIteration(), R=10)
+    return dict(heldout=tot == want_t and np.array_equal(dll, want_d),
+                heldout_repeatable=tot2 == tot and np.array_equal(dll2, dll))
 
 
 def main():
@@ -79,6 +100,8 @@ def main():
             want_lp = O.log_posterior(off, tokens, st["z"], K, V, st["theta"].astype(np.float64),
                                       st["phiT"].astype(np.float64), al, beta)
             checks["lp"] = abs(s.computeLogPosterior() - want_lp) <= 1e-9 * abs(want_lp)
+        # the evaluation changes no state, so the checks below are unaffected
+        checks.update(heldout(s, V, K, beta, seed))
         # z-only sweep (Phi frozen): stand-alone count exchange, no Phi draw
         s.sampleZGivenPhi(1)
         z3 = s.get_z_flat()
@@ -136,6 +159,16 @@ def main():
         print(scheme, K, f"{args.gpus} GPUs, one process:", checks, flush=True)
         ok &= all(bool(v) for v in checks.values())
         s.close()
+    # the sparse scheme keeps n_wk in natural topic order, phihat is in the register path's layout: held-out only
+    K, V = 1000, 700
+    s = L.GpuLDASampler(L.LDAConfiguration(scheme="gpu_spalias", topics=K, alpha=50.0 / K, beta=0.01, seed=2019, exec_time=0),
+                        devices=devices)
+    s.addInstances(L.InstanceList.from_csr(*L.synth_corpus(400, V, 70.0, seed=8), V))
+    s.sample(2)
+    checks = heldout(s, V, K, 0.01, 2019)
+    print("gpu_spalias", K, f"{args.gpus} GPUs, one process:", checks, flush=True)
+    ok &= all(checks.values())
+    s.close()
     if not ok:
         sys.exit(1)
     print("singleproc_multigpu_check ok, gpus =", args.gpus)

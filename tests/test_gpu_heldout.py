@@ -8,7 +8,6 @@ import pytest
 
 import ldagroupedgibbssampler_b200 as L
 from ldagroupedgibbssampler_b200._lib import LdaGpuError, ptr
-import heldout_oracle as H
 from conftest import make_corpus
 
 pytestmark = pytest.mark.gpu
@@ -33,7 +32,7 @@ def _test_set(seed=21, D=120, mean_len=35, V=V, empty_every=6):
 
 def _expect(oracle, s, toff, ttok, R):
     """the contract oracle on the sampler's current counts, alpha, beta and iteration"""
-    return H.heldout_l2r("contract", toff, ttok, s.getTypeTopicMatrix(), s.getTopicTotals(), s.alpha, s.beta,
+    return oracle.heldout_l2r("contract", toff, ttok, s.getTypeTopicMatrix(), s.getTopicTotals(), s.alpha, s.beta,
                               SEED, s.getCurrentIteration(), R=R)
 
 
@@ -122,7 +121,7 @@ def test_faithful_cats(oracle, cats):
     s = _sampler("gpu_pcgs", 10, off, tokens, V=Vc, alpha=0.1, sweeps=5)
     s.addTestInstances(L.InstanceList.from_csr(off, tokens, Vc))
     total, ll = s.heldOutLogLikelihood(10)
-    tf, f = H.heldout_l2r("faithful", off, tokens, s.getTypeTopicMatrix(), s.getTopicTotals(), s.alpha, s.beta,
+    tf, f = oracle.heldout_l2r("faithful", off, tokens, s.getTypeTopicMatrix(), s.getTopicTotals(), s.alpha, s.beta,
                                SEED, s.getCurrentIteration(), R=10)
     rel = np.abs(ll - f) / np.abs(f)
     assert rel.max() <= 1e-2 and (rel > 1e-6).mean() <= 0.03

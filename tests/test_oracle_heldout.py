@@ -1,12 +1,11 @@
-"""The CPU restatement of the held-out left-to-right estimator (tests/heldout_oracle.c, DESIGN.md 4.8): its primitives
-against oracle/, closed forms, exact enumeration, and the contract mode against the faithful mode.  CPU only."""
+"""The oracle's held-out left-to-right estimator (oracle_heldout_l2r_*, DESIGN.md 4.8): closed forms, exact enumeration,
+and the contract mode against the faithful mode.  CPU only."""
 import itertools
 import math
 
 import numpy as np
 import pytest
 
-import heldout_oracle as H
 from conftest import make_corpus
 
 BETA = 0.01
@@ -22,47 +21,25 @@ def _phihat(n_wk, n_k, beta):
     return (n_wk.astype(np.float64) + beta) / (n_k.astype(np.float64) + V * beta)
 
 
-def test_primitives_match_the_oracle(oracle):
-    """heldout_oracle.c restates Philox, and the K <= 1024 draw of oracle/lda_oracle.c, and compiles the contract ln of
-    oracle/contract_math.inc itself: all three must be those of the oracle -- Philox on the Random123 known answers and
-    random counters, ln on a range of arguments, the draw's topic on random scores at every row layout (K from 1 to
-    1024, padding topics included)"""
-    zero, ones = [0, 0, 0, 0], [0xFFFFFFFF] * 4
-    pi = [0x243F6A88, 0x85A308D3, 0x13198A2E, 0x03707344]
-    for ctr, key, want in ((zero, [0, 0], [0x6627E8D5, 0xE169C58D, 0xBC57AC4C, 0x9B00DBD8]),
-                           (ones, [0xFFFFFFFF, 0xFFFFFFFF], [0x408F276D, 0x41C83B0E, 0xA20BC7C6, 0x6D5451FD]),
-                           (pi, [0xA4093822, 0x299F31D0], [0xD16CFE09, 0x94FDCCEB, 0x5001E420, 0x24126EA1])):
-        assert list(H.philox(ctr, key)) == want
-    rng = np.random.default_rng(0)
-    for _ in range(200):
-        ctr, key = rng.integers(0, 2 ** 32, 4, dtype=np.uint32), rng.integers(0, 2 ** 32, 2, dtype=np.uint32)
-        assert np.array_equal(H.philox(ctr, key), oracle.philox(ctr, key))
-    for x in np.concatenate([np.geomspace(1e-300, 1e300, 500), rng.uniform(0.0, 2.0, 500), [5e-324, 1.0]]):
-        assert H.c_ln_f64(x) == oracle.lib().oracle_c_ln_f64(x)
-    for K in (1, 3, 31, 100, 128, 129, 256, 257, 400, 512, 513, 1000, 1024):
-        for _ in range(20):
-            a = (rng.integers(0, 5, K) + rng.uniform(0.01, 1.0, K)).astype(np.float32)
-            ph = rng.dirichlet(np.full(K, 0.3)).astype(np.float32)
-            U = np.float32((rng.integers(0, 2 ** 23) + 0.5) * 2.0 ** -23)
-            k, S = H.draw_lanes(a, ph, K, U)
-            assert k == oracle.lib().oracle_draw_topic_contract(a, ph, K, U)
-            assert abs(S - float((a.astype(np.float64) * ph).sum())) <= 1e-5 * S
-
-
-def test_one_token_documents():
-    """A one-token document has no draw to average over: l_d = ln(sum_k alpha_k phihat_kw / alpha_sum) in both modes."""
+def test_one_token_documents(oracle):
+    """A one-token document has no draw to average over: l_d = ln(sum_k alpha_k phihat_kw / alpha_sum) in both modes.
+    In contract mode that sum is the total S of the K <= 1024 draw, which must be the fp64 sum within 1e-5 relative at
+    every row layout (K from 1 to 1024, padding topics included)."""
     rng = np.random.default_rng(1)
-    V, K = 40, 7
-    n_wk, n_k = _counts(rng, V, K)
-    alpha = rng.uniform(0.05, 2.0, K)
+    V = 40
     off = np.arange(V + 1, dtype=np.int64)
     tokens = np.arange(V, dtype=np.int32)
-    ph = _phihat(n_wk, n_k, BETA)
-    closed = np.log((alpha[None, :] * ph).sum(axis=1) / alpha.sum())
-    _, f = H.heldout_l2r("faithful", off, tokens, n_wk, n_k, alpha, BETA, 5, 3, R=4)
-    _, c = H.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 5, 3, R=4)
-    np.testing.assert_allclose(f, closed, rtol=1e-12, atol=0)
-    np.testing.assert_allclose(c, closed, rtol=1e-6, atol=0)   # fp32 phihat and scores
+    for K in (7, 1, 3, 31, 100, 128, 129, 256, 257, 400, 512, 513, 1000, 1024):
+        n_wk, n_k = _counts(rng, V, K)
+        alpha = rng.uniform(0.05, 2.0, K)
+        ph = _phihat(n_wk, n_k, BETA)
+        closed = np.log((alpha[None, :] * ph).sum(axis=1) / alpha.sum())
+        _, f = oracle.heldout_l2r("faithful", off, tokens, n_wk, n_k, alpha, BETA, 5, 3, R=4)
+        _, c = oracle.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 5, 3, R=4)
+        np.testing.assert_allclose(f, closed, rtol=1e-12, atol=0, err_msg=f"K = {K}")
+        if K == 7:
+            np.testing.assert_allclose(c, closed, rtol=1e-6, atol=0)   # fp32 phihat and scores
+        assert np.abs(np.expm1(c - closed)).max() <= 1e-5, K       # S / sum_k alpha_k phihat_kw - 1
 
 
 def _enumerate(ph, alpha, words):
@@ -92,7 +69,7 @@ def _enumerate(ph, alpha, words):
 
 
 @pytest.mark.parametrize("n_tok", [2, 3])
-def test_faithful_against_exact_enumeration(n_tok):
+def test_faithful_against_exact_enumeration(oracle, n_tok):
     """R = 4096 particles against exact enumeration over the topics of the earlier tokens (K = 4).  For two tokens the
     particle mean of p_2 is an unbiased estimate of p(w_2 | w_1); for three tokens the estimate exp(l_d) / p_1 =
     mean(p_2) * mean(p_3) is compared with E[p_2] E[p_3], the value it converges to, and sigma comes from the enumerated
@@ -105,7 +82,7 @@ def test_faithful_against_exact_enumeration(n_tok):
     docs = [rng.integers(0, V, n_tok).astype(np.int32) for _ in range(12)]
     off = np.arange(0, n_tok * len(docs) + 1, n_tok, dtype=np.int64)
     tokens = np.concatenate(docs)
-    _, ll = H.heldout_l2r("faithful", off, tokens, n_wk, n_k, alpha, BETA, 11, 2, R=R)
+    _, ll = oracle.heldout_l2r("faithful", off, tokens, n_wk, n_k, alpha, BETA, 11, 2, R=R)
     for d, words in enumerate(docs):
         p1, cases = _enumerate(ph, alpha, words)
         pr = np.array([c[0] for c in cases])
@@ -151,8 +128,8 @@ def test_contract_against_faithful(oracle, cats, case):
         toff, ttok = make_corpus(400, V, 40, 4, sort_docs=False, empty_every=7)
     alpha = np.full(K, 50.0 / K if K > 10 else 0.1)
     n_wk, n_k = _trained_counts(oracle, off, tokens, V, K, alpha, 7, 5)
-    tc, c = H.heldout_l2r("contract", toff, ttok, n_wk, n_k, alpha, BETA, 7, 5, R=10)
-    tf, f = H.heldout_l2r("faithful", toff, ttok, n_wk, n_k, alpha, BETA, 7, 5, R=10)
+    tc, c = oracle.heldout_l2r("contract", toff, ttok, n_wk, n_k, alpha, BETA, 7, 5, R=10)
+    tf, f = oracle.heldout_l2r("faithful", toff, ttok, n_wk, n_k, alpha, BETA, 7, 5, R=10)
     empty = np.diff(toff) == 0
     assert np.all(c[empty] == 0.0) and np.all(f[empty] == 0.0)
     rel = np.abs(c - f) / np.maximum(np.abs(f), 1e-300)
@@ -162,17 +139,17 @@ def test_contract_against_faithful(oracle, cats, case):
     assert tc == np.cumsum(c)[-1]
 
 
-def test_evaluation_is_reproducible_and_keyed():
+def test_evaluation_is_reproducible_and_keyed(oracle):
     """Same iteration: the same values; another iteration or a shifted token base: other uniforms."""
     rng = np.random.default_rng(3)
     V, K = 50, 20
     n_wk, n_k = _counts(rng, V, K)
     off, tokens = make_corpus(30, V, 20, 5, sort_docs=False)
     alpha = np.full(K, 0.3)
-    a = H.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 4, R=3)
-    b = H.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 4, R=3)
-    c = H.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 5, R=3)
-    d = H.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 4, R=3, token_base=1)
+    a = oracle.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 4, R=3)
+    b = oracle.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 4, R=3)
+    c = oracle.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 5, R=3)
+    d = oracle.heldout_l2r("contract", off, tokens, n_wk, n_k, alpha, BETA, 9, 4, R=3, token_base=1)
     assert np.array_equal(a[1], b[1])
     assert not np.array_equal(a[1], c[1])
     assert not np.array_equal(a[1], d[1])

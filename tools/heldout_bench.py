@@ -8,7 +8,7 @@ length 1267, V = 12 419, K = 100) held out from the other 1350 documents.  The m
 sweeps from the random start (the estimator's cost does not depend on the counts' values).  Per shape: the wall time of
 the synchronous call (median of --repeats, after one warm-up call; it includes the phihat build and the copies back) and
 tokens x particles per second.  For comparison, as bench.py's cpu_baseline does, the rate of the faithful CPU
-restatement (tests/heldout_oracle.c) on the first documents of the split (at most 2 M token-particles, all host
+restatement (oracle/lda_oracle.c) on the first documents of the split (at most 2 M token-particles, all host
 threads).  The card's name and power limit are read in the same run.  Writes nothing."""
 import argparse
 import ctypes as C
@@ -22,10 +22,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
-import heldout_oracle as O  # noqa: E402  (the CPU restatement, tests/heldout_oracle.c)
 import ldagroupedgibbssampler_b200 as L  # noqa: E402
 from ldagroupedgibbssampler_b200.corpus import SHAPES  # noqa: E402
+from oracle import oracle as O  # noqa: E402
 
 
 def card(device):

@@ -294,11 +294,17 @@ __device__ __forceinline__ void list_remove(int *nz, int *cnt, int &nnz, int old
     __syncwarp();
 }
 
-// One token: scores over the list, cumulative sum, prior/likelihood branch.  Returns the new topic and, in
-// `slot`, its list position when the likelihood branch found it (-1 otherwise).
+// One token: scores over the list, cumulative sum, prior/likelihood branch.  u (Philox word 0) picks the branch
+// and the likelihood entry; the alias draw takes its slot from word 1 and its keep-or-alias uniform from word 2, so its
+// resolution does not shrink with the prior's share tn/tot (DESIGN.md 4.6).  Only the two branches that use words 1
+// and 2 compute them: every lane takes them together (u, tn and sum are the same on all lanes) and forms the token's
+// Philox block itself, which keeps the token loop's registers and shuffles to word 0.  (Measured on a B200 at 1000 W,
+// wiki8 z-step: 85.96 ms; fetching words 1 and 2 from the token's lane by shuffle, 86.25 ms; the single-word draw
+// this replaced, 85.19 ms.)  Returns the new topic and, in `slot`, its list position when the likelihood branch found
+// it (-1 otherwise).
 template <bool MULTI>
 __device__ __forceinline__ int sparse_draw(const SparseArgs &sa, const int *nz, const int *cnt, float *cum, int nnz,
-                                           int wt, float u, int lane, int &slot)
+                                           int wt, float u, int64_t t, int lane, int &slot)
 {
     const int K = sa.z.dm.K, Ks = sa.z.dm.Ks;
     const float *ph = sa.z.phiT + (size_t)wt * Ks;
@@ -339,21 +345,19 @@ __device__ __forceinline__ int sparse_draw(const SparseArgs &sa, const int *nz, 
     const float sum = carry;
     const float tot = __fadd_rn(tn, sum);
     slot = -1;
-    if (!(tot > 0.0f)) {
-        // neither the prior nor the document gives this type any mass (its Phi column is all zero over the topics
-        // that matter): the reference draws the topic uniformly (topics/PolyaUrnSpaliasLDA.java:275-277)
-        int i = __float2int_rz(__fmul_rn(u, __int2float_rn(K)));
-        return i > K - 1 ? K - 1 : i;
-    }
-    if (u < __fdiv_rn(tn, tot) || nnz == 0) {
-        // prior part: alias draw (:265-267, OptimizedGentleAliasMethod.java:100-107)
-        const float up = __fadd_rn(u, __fdiv_rn(__fmul_rn(sum, u), tn));
-        const float ups = __fmul_rn(up, __int2float_rn(K));
-        int i = __float2int_rz(ups);
-        if (i > K - 1) i = K - 1;
+    const bool uniform_topic = !(tot > 0.0f);
+    if (uniform_topic || u < __fdiv_rn(tn, tot) || nnz == 0) {
+        const ZArgs &a = sa.z;
+        const unsigned long long gt = (unsigned long long)(a.dm.token_base + t);
+        const uint4 r = philox4x32_10((uint32_t)gt, (uint32_t)(gt >> 32), a.sweep, STREAM_Z << 24, a.seed_lo, a.seed_hi);
+        // the alias slot floor(w1 K / 2^32): every slot is hit by floor(2^32 / K) or ceil(2^32 / K) words
+        const int i = (int)__umulhi(r.y, (unsigned)K);
+        // tot = 0: neither the prior nor the document gives this type any mass (its Phi column is all zero over the
+        // topics that matter): the reference draws the topic uniformly (topics/PolyaUrnSpaliasLDA.java:275-277)
+        if (uniform_topic) return i;
+        // prior part: alias draw (:265-267, OptimizedGentleAliasMethod.java:100-107), keep the slot if uniform23(w2) <= ps
         const int2 entry = __ldg(reinterpret_cast<const int2 *>(sa.table + (size_t)wt * Ks + i));   // {ps, alias}
-        if (__fsub_rn(ups, __int2float_rn(i)) > __int_as_float(entry.x)) i = entry.y;
-        return i;
+        return uniform23(r.z) > __int_as_float(entry.x) ? entry.y : i;
     }
     // likelihood part: first slot with u*tot - tn <= cum (:269-275, findIdx :347-375)
     const float ul = __fsub_rn(__fmul_rn(u, tot), tn);
@@ -413,7 +417,7 @@ __device__ __forceinline__ int64_t sparse_tokens(const SparseArgs &sa, int *nz, 
             const float u = __shfl_sync(FULL, U, tt);
             list_remove<MULTI>(nz, cnt, nnz, old, lane);
             int slot;
-            const int nw = sparse_draw<MULTI>(sa, nz, cnt, cum, nnz, wt, u, lane, slot);
+            const int nw = sparse_draw<MULTI>(sa, nz, cnt, cum, nnz, wt, u, tb + tt, lane, slot);
             if (lane == tt) znew = nw;
             if (slot < 0) slot = list_find<MULTI>(nz, nnz, nw, lane);
             list_add_at(nz, cnt, nnz, nw, slot, lane);

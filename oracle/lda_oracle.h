@@ -157,6 +157,8 @@ void oracle_set_num_threads(int n);
  * reference: topics/SpaliasUncollapsedParallelLDA.java:39-60,124-312, util/OptimizedGentleAliasMethod.java:52-107 */
 void oracle_alias_build_contract(int32_t V, int32_t K, const double *alpha, const float *phiT, float *ps,
                                  int32_t *al, float *type_norm);
+/* the prior part's draw of one token from its Philox words 1 (slot) and 2 (keep-or-alias uniform), one type's table */
+int32_t oracle_alias_sample_contract(const float *ps, const int32_t *al, int32_t K, uint32_t w1, uint32_t w2);
 void oracle_z_spalias_contract(int64_t D, const int64_t *doc_off, const int32_t *tokens, int32_t *z,
                                int32_t K, const float *phiT, const float *ps, const int32_t *al,
                                const float *type_norm, uint64_t seed, uint32_t sweep, int64_t token_base);

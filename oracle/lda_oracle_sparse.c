@@ -12,7 +12,9 @@
  *
  * Two modes as in lda_oracle.c: "faithful" (double, the Java statements as written) and "contract"
  * (the fixed fp32/fp64 operation order of the CUDA kernels, DESIGN.md 4.6; bit-exact with the GPU).
- * Both use the injected Philox stream (stream 1 = z, counter = global token index).
+ * Both use the injected Philox stream (stream 1 = z, counter = global token index): word 0 of a token's block for the
+ * branch and the likelihood part, words 1 and 2 for the alias draw, where the reference reuses its one uniform
+ * (same distribution, DESIGN.md 4.6).
  */
 #include <math.h>
 #include <stdlib.h>
@@ -81,22 +83,25 @@ void oracle_alias_build_contract(int32_t V, int32_t K, const double *alpha, cons
     free(af);
 }
 
-/* util/OptimizedGentleAliasMethod.java:100-107 in fp32 */
-static inline int32_t alias_sample_contract(const float *ps, const int32_t *al, int32_t K, float u)
+static inline float uniform23(uint32_t w) { return ((float)(w >> 9) + 0.5f) * 0x1p-23f; }
+
+/* the alias slot floor(w1 K / 2^32) (the kernel's __umulhi): every slot is hit by floor(2^32/K) or ceil(2^32/K) words */
+static inline int32_t alias_slot(uint32_t w1, int32_t K) { return (int32_t)(((uint64_t)w1 * (uint32_t)K) >> 32); }
+
+/* util/OptimizedGentleAliasMethod.java:100-107 on two Philox words of the token (DESIGN.md 4.6): slot from w1, keep
+ * it if uniform23(w2) <= ps (fp32 compare), else its alias */
+int32_t oracle_alias_sample_contract(const float *ps, const int32_t *al, int32_t K, uint32_t w1, uint32_t w2)
 {
-    float ups = u * (float)K;
-    int32_t i = (int32_t)ups;
-    if (i > K - 1) i = K - 1;
-    if ((ups - (float)i) > ps[i]) i = al[i];
-    return i;
+    const int32_t i = alias_slot(w1, K);
+    return uniform23(w2) > ps[i] ? al[i] : i;
 }
 
-static inline float z_uniform23(uint64_t seed, uint64_t token, uint32_t sweep)
+/* the token's Philox block: word 0 -> branch / likelihood uniform, words 1 and 2 -> alias draw */
+static inline void z_words(uint64_t seed, uint64_t token, uint32_t sweep, uint32_t out[4])
 {
     uint32_t ctr[4] = {(uint32_t)token, (uint32_t)(token >> 32), sweep, (uint32_t)ORACLE_STREAM_Z << 24};
-    uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)}, out[4];
+    uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
     oracle_philox4x32_10(ctr, key, out);
-    return ((float)(out[0] >> 9) + 0.5f) * 0x1p-23f;
 }
 
 /* Sparse z-step, contract (DESIGN.md 4.6).  Per token of a document, in order:
@@ -104,7 +109,7 @@ static inline float z_uniform23(uint64_t seed, uint64_t token, uint32_t sweep)
  *   s_i = float(cnt_i) * phiT[w][nz_i] over the list in list order; cumulative sums in blocks of 256
  *   entries (8 consecutive entries per lane: lane-local prefix, Kogge-Stone over the 32 lane totals,
  *   block carries added sequentially); sum = last carry;
- *   u ~ U(0,1); tot = tn + sum; if u < tn / tot: alias draw with u' = u + (sum*u)/tn
+ *   u = uniform23(word 0); tot = tn + sum; if u < tn / tot: alias draw on words 1 and 2
  *   else: first i with u*tot - tn <= cum_i (last entry if none);
  *   add the token to its new topic (append to the list when it was 0). */
 void oracle_z_spalias_contract(int64_t D, const int64_t *doc_off, const int32_t *tokens, int32_t *z,
@@ -161,17 +166,18 @@ void oracle_z_spalias_contract(int64_t D, const int64_t *doc_off, const int32_t 
                     carry = carry + x[31];
                     sum = carry;
                 }
-                const float u = z_uniform23(seed, (uint64_t)(token_base + t), sweep);
+                uint32_t r[4];
+                z_words(seed, (uint64_t)(token_base + t), sweep, r);
+                const float u = uniform23(r[0]);
                 const float tn = type_norm[w];
                 const float tot = tn + sum;
                 int32_t nw;
                 if (!(tot > 0.0f)) {
                     /* no prior mass and no document mass for this type: uniform topic
                      * (topics/PolyaUrnSpaliasLDA.java:275-277) */
-                    nw = (int32_t)(u * (float)K);
-                    if (nw > K - 1) nw = K - 1;
+                    nw = alias_slot(r[1], K);
                 } else if (u < tn / tot || nnz == 0) {
-                    nw = alias_sample_contract(ps + (size_t)w * K, al + (size_t)w * K, K, u + (sum * u) / tn);
+                    nw = oracle_alias_sample_contract(ps + (size_t)w * K, al + (size_t)w * K, K, r[1], r[2]);
                 } else {
                     const float ul = u * tot - tn;
                     int slot = nnz - 1;
@@ -251,19 +257,18 @@ void oracle_z_spalias_faithful(int64_t D, int32_t V, const int64_t *doc_off, con
                 if (--cnt[old] == 0) { int i = back[old]; nz[i] = nz[--nnz]; back[nz[i]] = i; }
                 double sum = 0.0;
                 for (int i = 0; i < nnz; ++i) { sum += cnt[nz[i]] * ph[nz[i]]; cum[i] = sum; }
-                const double u = (double)z_uniform23(seed, (uint64_t)(token_base + t), sweep);
+                uint32_t r[4];
+                z_words(seed, (uint64_t)(token_base + t), sweep, r);
+                const double u = (double)uniform23(r[0]);
                 const double u_sigma = u * (tn[w] + sum);
                 int32_t nw;
                 if (!(tn[w] + sum > 0.0)) {
-                    nw = (int32_t)floor(u * (double)K);   /* PolyaUrnSpaliasLDA.java:275-277 */
-                    if (nw > K - 1) nw = K - 1;
+                    nw = alias_slot(r[1], K);   /* PolyaUrnSpaliasLDA.java:275-277 */
                 } else if (u < (tn[w] / (tn[w] + sum)) || nnz == 0) {
-                    double up = u + ((sum * u) / tn[w]);
-                    double ups = up * K;
-                    int i = (int)ups;
-                    if (i > K - 1) i = K - 1;
-                    if ((ups - i) > ps[(size_t)w * K + i]) i = al[(size_t)w * K + i];
-                    nw = i;
+                    /* the reference rescales u to u' = u + sum*u/tn, slot = floor(u'K), fraction against ps: given
+                     * the branch, slot and fraction are independent uniforms, here drawn from words 1 and 2 */
+                    const int i = alias_slot(r[1], K);
+                    nw = (double)uniform23(r[2]) > ps[(size_t)w * K + i] ? al[(size_t)w * K + i] : i;
                 } else {
                     double ul = u_sigma - tn[w];
                     int slot = nnz - 1;

@@ -98,6 +98,7 @@ def lib():
     sig("oracle_max_threads", C.c_int)
     sig("oracle_set_num_threads", None, C.c_int)
     sig("oracle_alias_build_contract", None, i32, i32, _f64p, _f32p, _f32p, _i32p, _f32p)
+    sig("oracle_alias_sample_contract", i32, _f32p, _i32p, i32, u32, u32)
     sig("oracle_z_spalias_contract", None, i64, _i64p, _i32p, _i32p, i32, _f32p, _f32p, _i32p, _f32p, u64, u32, i64)
     sig("oracle_z_spalias_faithful", None, i64, i32, _i64p, _i32p, _i32p, i32, _f64p, _f64p, u64, u32, i64)
     _lib = L

@@ -216,24 +216,59 @@ def test_contract_and_faithful_chains_agree_statistically(oracle, cats, scheme):
 
 # ---- sparse PCGS z-step ("spalias") ---------------------------------------------------------------
 def test_alias_tables_reproduce_the_prior(oracle):
-    """WalkerAliasTableTest / OptimizedGentleAliasMethod.main: the table must encode alpha_k*phi_kw / norm."""
-    rng = np.random.default_rng(1)
-    V, K = 40, 37
-    phi = rng.dirichlet(np.full(V, 0.05), size=K).T.astype(np.float32).copy()      # [V][K]
-    alpha = rng.random(K) + 0.01
-    ps, al, tn = oracle.alias_build_contract(phi, alpha)
-    for w in range(V):
-        p = np.zeros(K)
-        for i in range(K):
-            if al[w, i] == i:
-                p[i] += 1.0 / K
-            else:
-                p[i] += ps[w, i] / K
-                p[al[w, i]] += (1.0 - ps[w, i]) / K
-        want = alpha.astype(np.float32).astype(np.float64) * phi[w]
-        assert abs(tn[w] - want.sum()) <= 1e-6 * want.sum()
-        assert np.allclose(p, want / want.sum(), atol=2e-6)
-        assert ps[w].min() >= 0 and ps[w].max() <= 1.0 + 1e-6 and al[w].min() >= 0 and al[w].max() < K
+    """WalkerAliasTableTest / OptimizedGentleAliasMethod.main: the table must encode alpha_k*phi_kw / norm, at a small
+    K and at the K = 10 000 of the wiki-shaped workloads."""
+    V = 40
+    for K in (37, 10_000):
+        rng = np.random.default_rng(1)
+        phi = rng.dirichlet(np.full(V, 0.05), size=K).T.astype(np.float32).copy()      # [V][K]
+        alpha = rng.random(K) + 0.01
+        ps, al, tn = oracle.alias_build_contract(phi, alpha)
+        for w in range(V):
+            own = al[w] == np.arange(K)
+            keep = np.where(own, 1.0, ps[w].astype(np.float64))
+            p = keep / K
+            np.add.at(p, al[w], (1.0 - keep) / K)
+            want = alpha.astype(np.float32).astype(np.float64) * phi[w]
+            assert abs(tn[w] - want.sum()) <= 1e-6 * want.sum(), (K, w)
+            assert np.allclose(p, want / want.sum(), atol=2e-6), (K, w)
+            assert ps[w].min() >= 0 and ps[w].max() <= 1.0 + 1e-6 and al[w].min() >= 0 and al[w].max() < K, (K, w)
+
+
+@pytest.mark.parametrize("K", [1, 5, 1500, 10_000])
+def test_alias_draw_induces_the_prior_exactly(oracle, K):
+    """The prior part's draw over all its inputs, with no sampling: Philox word 1 picks slot floor(w1 K / 2^32), word 2
+    keeps it when uniform23(w2) <= ps, else the alias is taken.  Slot i is hit by exactly ceil((i+1) 2^32/K) -
+    ceil(i 2^32/K) words; (n + 1/2) 2^-23 <= ps holds for n <= ps 2^23 - 1/2.  The distribution these counts give
+    must be alpha_k phi_kw / norm.  The resolution does not depend on the prior's share of the token's mass (DESIGN.md
+    4.6).  The oracle's draw is checked at every boundary of the counting, for a flat and a skewed Phi column."""
+    rng = np.random.default_rng(K)
+    phi = np.stack([rng.gamma(1.0, size=K), rng.gamma(0.05, size=K)]).astype(np.float32)      # [V][K]
+    phi /= phi.sum(axis=1, keepdims=True)
+    alpha = np.full(K, 0.005)
+    ps, al, _ = oracle.alias_build_contract(phi, alpha)
+    i = np.arange(K, dtype=np.int64)
+    first = -((-i << 32) // K)                               # first word of slot i: ceil(i 2^32 / K)
+    hits = np.diff(np.append(first, 1 << 32))
+    assert hits.sum() == 1 << 32 and set(np.unique(hits)) <= {(1 << 32) // K, -(-(1 << 32) // K)}
+    for w in range(phi.shape[0]):
+        kept = np.clip(np.floor(ps[w].astype(np.float64) * 2.0**23 - 0.5) + 1, 0, 1 << 23)   # 23-bit values kept
+        keep = kept / 2.0**23
+        p = hits * keep
+        np.add.at(p, al[w], hits * (1.0 - keep))
+        p /= 2.0**32
+        want = np.float32(0.005) * phi[w].astype(np.float64)
+        want /= want.sum()
+        tv = 0.5 * np.abs(p - want).sum()
+        assert tv <= 1e-5, f"K = {K}, column {w}: TV {tv:.3g}"
+        draw = oracle.lib().oracle_alias_sample_contract
+        for s in {0, 1, K // 2, K - 2, K - 1} & set(range(K)):
+            lo, hi = int(first[s]), int(first[s] + hits[s] - 1)
+            for w1 in (lo, hi):
+                if kept[s] > 0:
+                    assert draw(ps[w], al[w], K, w1, (int(kept[s]) - 1) << 9) == s
+                if kept[s] < 1 << 23:
+                    assert draw(ps[w], al[w], K, w1, int(kept[s]) << 9) == al[w, s]
 
 
 def test_spalias_contract_vs_faithful_and_invariants(oracle):
